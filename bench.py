@@ -2,6 +2,7 @@
 """bench.py — throughput of the fuse-query hot path on B200 (and of the CPU reference arm).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--rows R] [--mode materialised|generated]
+                    [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[3], the README headline query):
     SELECT sum(number)/count(number), max(number), min(number) FROM system.numbers_mt(10_000_000_000)
@@ -28,17 +29,21 @@ this image) with the 8-way parallelism the reference uses.
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
+import shutil
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the tree it runs from as it found it (it may be read-only)
 
 TOTAL_ROWS = 10_000_000_000
 NUM = "(col number)"
@@ -151,6 +156,19 @@ def expected(total: int):
     return {"sum": _sum(total), "count": total, "avg": _sum(total) // total, "max": total - 1, "min": 0}
 
 
+def dump_outputs(out_dir: str, arrays: dict):
+    """--dump-outputs: each array as <out_dir>/<name>.npy in float64, so that two builds can be compared output for output."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
+def u64_hi_lo(values):
+    """u64 values as exact (high 32 bits, low 32 bits) pairs: a wrapped u64 sum does not fit float64's 53-bit mantissa."""
+    return [[v >> 32, v & 0xFFFFFFFF] for v in values]
+
+
 def common_config(total: int):
     """The part of `config` both arms print identically (the driver compares them)."""
     sql = HEADLINE_SQL if total == TOTAL_ROWS else HEADLINE_SQL.replace("10000000000", str(total))
@@ -189,6 +207,8 @@ def run_reference(args):
     value = rows * len(times) / t
     exp = expected(rows)
     assert list(res) == [exp["avg"], exp["max"], exp["min"]], (res, exp)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"result": list(res)})
     total = args.rows or TOTAL_ROWS
     sample = (f"{rows} rows of numbers_mt per step (the {total}-row workload is {total / rows:.1f}x this; rows/s is size-independent), "
               f"8 partitions on {cores} threads, 10 000-row blocks, one Arrow-style pass per aggregate")
@@ -453,6 +473,9 @@ def run_ours(args):
     exp = expected(total)
     got = {"sum": vals[0], "count": vals[1], "avg": vals[0] // vals[1], "max": vals[2], "min": vals[3]}
     assert got == exp and rows == total, f"rank {rank}: result mismatch: {got} != {exp}"
+    if args.dump_outputs and rank == 0:
+        # the query's row, the merged Aggregator-leaf states (sum, count, max, min) and the rows the last step scanned
+        dump_outputs(args.dump_outputs, {"result": [got["avg"], got["max"], got["min"]], "leaf_states_hi_lo": u64_hi_lo(vals), "rows": [rows]})
 
     # ---- the same kernels back to back without the cross-rank merge (what round 1 reported as the step) ----
     no_merge = None
@@ -976,7 +999,15 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=3)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-query-table", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if "FQ_JIT_CACHE_DIR" not in os.environ:
+        # kernels compiled at run time are cached in a directory of this run's own, not next to the library in the tree
+        jit_dir = tempfile.mkdtemp(prefix="fq_jit_")
+        atexit.register(shutil.rmtree, jit_dir, True)
+        os.environ["FQ_JIT_CACHE_DIR"] = jit_dir
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -4,6 +4,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -28,6 +30,36 @@ def test_reference_arm_prints_one_contract_line():
     assert d["e2e"] == {"value": d["value"], "unit": "rows/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert "workload" in d["config"] and "numbers_mt" in d["config"]["workload"]
     assert d["value"] > 0 and abs(d["ms_per_step"] * 1e-3 * d["value"] - 8_000_000) < 1e-3 * 8_000_000
+
+
+def test_reference_arm_dumps_its_last_result(tmp_path):
+    import numpy as np
+    r = run("--impl", "reference", "--steps", "1", "--warmup", "0", "--rows", "8000000", "--dump-outputs", str(tmp_path / "out"))
+    assert r.returncode == 0, r.stderr
+    res = np.load(tmp_path / "out" / "result.npy")
+    assert res.dtype == np.float64 and res.tolist() == [3999999, 7999999, 0]
+
+
+def test_steps_below_one_are_refused():
+    r = run("--impl", "reference", "--steps", "0", "--rows", "8000000")
+    assert r.returncode != 0 and "--steps" in r.stderr and r.stdout == ""
+
+
+@pytest.mark.gpu
+def test_timed_path_dumps_what_its_last_step_computed(tmp_path):
+    """--dump-outputs: the query's row, the merged leaf states as exact u64 halves and the row count, after exactly --steps steps."""
+    import numpy as np
+    rows = 80_000_000
+    r = run("--steps", "3", "--warmup", "1", "--rows", str(rows), "--no-query-table", "--no-cpu-baseline", "--dump-outputs", str(tmp_path / "out"))
+    assert r.returncode == 0, r.stderr[-3000:]
+    d = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][0])
+    assert d["steps"] == 3 and d["gpu_launches"] >= 3
+    out = {n: np.load(tmp_path / "out" / f"{n}.npy") for n in ("result", "leaf_states_hi_lo", "rows")}
+    assert all(a.dtype == np.float64 for a in out.values())
+    s = (rows * (rows - 1) // 2) % (1 << 64)
+    assert out["result"].tolist() == [s // rows, rows - 1, 0]
+    assert [int(h) << 32 | int(l) for h, l in out["leaf_states_hi_lo"].tolist()] == [s, rows, rows - 1, 0]
+    assert out["rows"].tolist() == [rows]
 
 
 def test_reference_arm_is_silent_on_other_ranks():
