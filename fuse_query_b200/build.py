@@ -34,7 +34,7 @@ def _run(cmd, **kw):
 
 def _sources():
     files = [os.path.join(CSRC, f) for f in ("fuse_gpu.cu", "codegen.cc", "codegen.h", "aot_pipes.txt")]
-    files += [os.path.join(CSRC, "kernels", "fq_skeleton.cuh"), os.path.join(CSRC, "kernels", "fq_sort.cuh"), os.path.join(CSRC, "tools", "aotgen.cc"),
+    files += [os.path.join(CSRC, "kernels", "fq_skeleton.cuh"), os.path.join(CSRC, "kernels", "fq_sort.cuh"), os.path.join(CSRC, "kernels", "fq_utf8.cuh"), os.path.join(CSRC, "tools", "aotgen.cc"),
               os.path.join(os.path.dirname(PKG), "include", "fuse_gpu.h"), os.path.abspath(__file__)]
     files += [os.path.join(CSRC, f) for f in HOST_SRC + HOST_HDR]
     return files

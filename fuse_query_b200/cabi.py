@@ -80,6 +80,7 @@ EXPORTS = [
     "fq_pipe_key_dtype", "fq_pipe_leaf_dtype", "fq_pipe_groupby_reserve", "fq_pipe_launch_groupby", "fq_pipe_fetch_groupby",
     "fq_pipe_export_groups", "fq_pipe_group_entry_slots", "fq_pipe_export_partials", "fq_pipe_merge_partials",
     "fq_column_set_validity_bitmap", "fq_utf8_create", "fq_utf8_free", "fq_utf8_len", "fq_utf8_compare", "fq_utf8_compare_scalar", "fq_utf8_minmax",
+    "fq_utf8_bytes", "fq_utf8_download", "fq_utf8_take", "fq_utf8_dict_encode", "fq_utf8_bounds",
     "fq_sort_indices", "fq_sort_indices_limit", "fq_column_take", "fq_column_copy", "fq_ctx_trim",
     "fq_graph_begin", "fq_graph_end", "fq_graph_launch", "fq_graph_destroy", "fq_stream_create", "fq_stream_destroy",
 ]
@@ -163,6 +164,11 @@ def lib():
         "fq_utf8_compare": (i32, [vp, i32, vp, vp, vp, vp, vp]),
         "fq_utf8_compare_scalar": (i32, [vp, i32, vp, vp, u64, vp, vp, vp]),
         "fq_utf8_minmax": (i32, [vp, i32, vp, C.POINTER(i64), vp]),
+        "fq_utf8_bytes": (u64, [vp]),
+        "fq_utf8_download": (i32, [vp, vp, vp, vp, vp]),
+        "fq_utf8_take": (i32, [vp, vp, vp, u64, vp, C.POINTER(vp), vp]),
+        "fq_utf8_dict_encode": (i32, [vp, vp, vp, C.POINTER(vp), vp]),
+        "fq_utf8_bounds": (i32, [vp, vp, vp, u64, C.POINTER(u64), C.POINTER(u64), vp]),
         "fq_sort_indices": (i32, [vp, vp, vp, i32, u64, vp, vp]),
         "fq_sort_indices_limit": (i32, [vp, vp, vp, i32, u64, u64, vp, C.POINTER(u64), vp]),
         "fq_column_take": (i32, [vp, vp, vp, u64, vp, vp, vp]),
@@ -569,6 +575,45 @@ class Utf8Array:
         row = C.c_int64()
         self.ctx.check(lib().fq_utf8_minmax(self.ctx._h, AGG[op], self._h, C.byref(row), C.c_void_p(stream)))
         return row.value
+
+    def nbytes(self) -> int:
+        return lib().fq_utf8_bytes(self._h)
+
+    def to_list(self, stream: int = 0) -> List[Optional[bytes]]:
+        """the strings as bytes (None where the array's validity says NULL)"""
+        import numpy as np
+        n = len(self)
+        offsets = np.zeros(n + 1, dtype=np.int32)
+        data = C.create_string_buffer(max(1, self.nbytes()))
+        self.ctx.check(lib().fq_utf8_download(self.ctx._h, self._h, C.c_void_p(offsets.ctypes.data), data, C.c_void_p(stream)))
+        self.ctx.synchronize(stream)
+        raw = data.raw
+        vals = [raw[offsets[i]:offsets[i + 1]] for i in range(n)]
+        if self._valid is not None:
+            ok = self._valid.to_numpy(n, stream)
+            vals = [v if f else None for v, f in zip(vals, ok)]
+        return vals
+
+    def take(self, rows: Column, n: int, valid: Optional[Column] = None, stream: int = 0) -> "Utf8Array":
+        """strings rows[0 .. n) (UInt32 column); `valid` (Boolean column) marks NULL output slots and must outlive the result"""
+        h = C.c_void_p()
+        self.ctx.check(lib().fq_utf8_take(self.ctx._h, self._h, rows._h, n, valid._h if valid is not None else None, C.byref(h), C.c_void_p(stream)))
+        return Utf8Array(self.ctx, h, valid)
+
+    def dict_encode(self, stream: int = 0):
+        """-> (codes: UInt32 Column, one slot per row, dictionary: Utf8Array of the distinct valid strings in bytewise order)"""
+        codes = self.ctx.column(U32, max(1, len(self)))
+        h = C.c_void_p()
+        self.ctx.check(lib().fq_utf8_dict_encode(self.ctx._h, self._h, codes._h, C.byref(h), C.c_void_p(stream)))
+        return codes, Utf8Array(self.ctx, h, None)
+
+    def bounds(self, value, stream: int = 0):
+        """(lower, upper) bound of `value` (str or bytes) in this array, which must be sorted"""
+        b = value.encode() if isinstance(value, str) else bytes(value)
+        lo, hi = C.c_uint64(), C.c_uint64()
+        self.ctx.check(lib().fq_utf8_bounds(self.ctx._h, self._h, C.create_string_buffer(b, max(1, len(b))), len(b), C.byref(lo), C.byref(hi),
+                                            C.c_void_p(stream)))
+        return lo.value, hi.value
 
     def free(self):
         if self._h:

@@ -196,6 +196,29 @@ PYBIND11_MODULE(_fuse_host, m) {
         auto v = a->to_arrow_bitmap();
         return py::bytes((const char *)v.data(), v.size());
       })
+      .def_static("from_utf8", [](GpuContextRef gpu, py::array_t<int32_t, py::array::c_style | py::array::forcecast> offsets, py::bytes data,
+                                  py::object valid) {
+        const std::string bytes = data;
+        const uint64_t n = offsets.size() ? (uint64_t)offsets.size() - 1 : 0;
+        if (!offsets.size()) throw FuseQueryError::internal("Utf8 offsets need len + 1 entries");
+        std::vector<unsigned char> v;
+        if (!valid.is_none()) {
+          py::array_t<uint8_t, py::array::c_style | py::array::forcecast> a = py::array::ensure(valid.attr("__ne__")(0).attr("astype")("uint8"));
+          if ((uint64_t)a.size() != n) throw FuseQueryError::internal("validity and values differ in length");
+          v.assign(a.data(), a.data() + n);
+        }
+        if (n && (uint64_t)offsets.data()[n] != bytes.size()) throw FuseQueryError::internal("Utf8 offsets do not end at the byte count");
+        return DataArray::utf8_dict(gpu, offsets.data(), bytes.data(), n, v.empty() ? nullptr : v.data());
+      }, py::arg("gpu"), py::arg("offsets"), py::arg("data"), py::arg("valid") = py::none(),
+         "Utf8 column from Arrow offsets (int32, starting at 0) + bytes (+ validity), dictionary-encoded on the device")
+      .def("dictionary", [](const DataArrayRef &a) -> py::object {
+        if (!a->dict()) return py::none();
+        const Utf8Dict &d = *a->dict();
+        std::vector<uint32_t> all(d.size);
+        for (uint64_t i = 0; i < d.size; i++) all[i] = (uint32_t)i;
+        auto rows = DataArray::from_host(a->ctx(), FQ_U32, all.data(), d.size);
+        return py::cast(DataArray::with_dict(rows, a->dict())->strings());
+      }, "the sorted dictionary of a dictionary-encoded Utf8 array (None for other arrays)")
       .def("set_validity", &DataArray::set_validity)
       .def("validity", &DataArray::validity)
       .def("null_count", &DataArray::null_count)
@@ -207,7 +230,14 @@ PYBIND11_MODULE(_fuse_host, m) {
       .def("to_numpy", &array_to_python)
       .def("to_list", [](const DataArrayRef &a) -> py::object {   // NULL slots come back as None
         py::object o = array_to_python(a);
-        if (a->is_utf8()) return o;
+        if (a->is_utf8()) {
+          if (!a->validity()) return o;
+          py::list vals = o;
+          py::list ok = array_to_python(a->validity()).attr("tolist")();
+          for (size_t i = 0; i < vals.size(); i++)
+            if (!ok[i].cast<bool>()) vals[i] = py::none();
+          return std::move(vals);
+        }
         py::list vals = o.attr("tolist")();
         if (a->validity()) {
           py::list ok = array_to_python(a->validity()).attr("tolist")();

@@ -26,6 +26,7 @@
 #include "codegen.h"
 #include "kernels/fq_skeleton.cuh"
 #include "kernels/fq_sort.cuh"
+#include "kernels/fq_utf8.cuh"
 #include "generated/skeleton_embed.h"  // static const char fq_skeleton_src[]
 
 #ifndef FQ_MAP_DEFAULT_VARIANT
@@ -2296,19 +2297,11 @@ struct fq_utf8 {
   uint64_t len = 0;
   int32_t *offsets = nullptr;   // device, len + 1
   unsigned char *data = nullptr;
+  uint64_t bytes = 0;           // offsets[len]
   const fq_column *validity = nullptr;
 };
 
 namespace {
-// bytewise order, shorter string first on a common prefix (Rust str / arrow)
-__device__ __forceinline__ int fq_utf8_cmp(const unsigned char *a, fq_u32 la, const unsigned char *b, fq_u32 lb) {
-  const fq_u32 n = la < lb ? la : lb;
-  for (fq_u32 i = 0; i < n; i++) {
-    const int d = (int)a[i] - (int)b[i];
-    if (d) return d;
-  }
-  return la < lb ? -1 : (la > lb ? 1 : 0);
-}
 __device__ __forceinline__ bool fq_cmp_holds(int op, int c) {
   switch (op) {
     case FQ_CMP_EQ: return c == 0;
@@ -2385,6 +2378,7 @@ fq_status fq_utf8_create(fq_ctx *ctx, const int32_t *offsets, const void *data, 
   if (bytes && !data) return set_err(FQ_ERR_INVALID, "Internal Error: null value buffer");
   fq_utf8 *a = new fq_utf8();
   a->len = len;
+  a->bytes = bytes;
   a->validity = validity;
   cudaError_t e = cudaMalloc(&a->offsets, sizeof(int32_t) * (len + 1));
   if (e == cudaSuccess) e = cudaMalloc(&a->data, bytes ? bytes : 1);
@@ -2462,6 +2456,198 @@ fq_status fq_utf8_minmax(fq_ctx *ctx, int32_t op, const fq_utf8 *a, int64_t *row
   CUDA_TRY(cudaStreamSynchronize(s));
   cudaFreeAsync(scratch, s);
   *row = h;
+  return FQ_OK;
+}
+
+}  // extern "C"
+
+// ---- dictionary encoding (kernels/fq_utf8.cuh) ----
+namespace {
+// device buffers of one call, given back in stream order whatever way the call ends
+struct StreamScratch {
+  cudaStream_t s;
+  std::vector<void *> bufs;
+  explicit StreamScratch(cudaStream_t st) : s(st) {}
+  ~StreamScratch() {
+    for (void *p : bufs) cudaFreeAsync(p, s);
+  }
+  template <class T>
+  cudaError_t get(T **out, uint64_t bytes) {
+    void *p = nullptr;
+    cudaError_t e = cudaMallocAsync(&p, bytes ? bytes : 1, s);
+    if (e == cudaSuccess) bufs.push_back(p);
+    *out = (T *)p;
+    return e;
+  }
+};
+
+unsigned grid_for(const fq_ctx *ctx, uint64_t n, uint64_t per_sm = 8) {
+  return (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((n + 255) / 256, (uint64_t)ctx->sm_count * per_sm));
+}
+
+// strings rows[0 .. n) of `src` (NULL where rows_valid says so) as a new array; waits for the result
+fq_status utf8_take(fq_ctx *ctx, const fq_utf8 *src, const fq_u32 *rows, uint64_t n, const fq_column *rows_valid, cudaStream_t s, fq_utf8 **out) {
+  if (n >= 0xFFFFFFFFull) return set_err(FQ_ERR_UNSUPPORTED, "Unsupported on the device path: a Utf8 array of 2^32 - 1 rows or more");
+  StreamScratch scratch(s);
+  fq_utf8 *a = new fq_utf8();
+  a->len = n;
+  a->validity = rows_valid;
+  auto fail = [&](fq_status st) { fq_utf8_free(ctx, a); return st; };
+  unsigned long long *total = nullptr;
+  fq_u32 *sums = nullptr;
+  cudaError_t e = cudaMalloc(&a->offsets, sizeof(int32_t) * (n + 1));
+  if (e == cudaSuccess) e = scratch.get(&total, 16);
+  if (e == cudaSuccess) e = scratch.get(&sums, 4 * ((n + 1 + FQ_SCAN_TILE - 1) / FQ_SCAN_TILE));
+  if (e == cudaSuccess) e = cudaMemsetAsync(total, 0, 16, s);
+  if (e != cudaSuccess) return fail(set_err(FQ_ERR_CUDA, "CUDA error: %s (Utf8 take of %" PRIu64 " rows)", cudaGetErrorString(e), n));
+  const fq_u8 *rv = rows_valid ? (const fq_u8 *)rows_valid->ptr : nullptr;
+  fq_utf8_lens<<<grid_for(ctx, n + 1), 256, 0, s>>>(src->offsets, src->len, rows, rv, n, (fq_u32 *)a->offsets, total);
+  ctx->launches++;
+  unsigned long long h[2] = {0, 0};
+  e = cudaMemcpyAsync(h, total, 16, cudaMemcpyDeviceToHost, s);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+  if (e != cudaSuccess) return fail(set_err(FQ_ERR_CUDA, "CUDA error: %s (Utf8 take of %" PRIu64 " rows)", cudaGetErrorString(e), n));
+  if (h[1]) return fail(set_err(FQ_ERR_INVALID, "Internal Error: a row index of the Utf8 take is out of range"));
+  if (h[0] > (unsigned long long)INT32_MAX)
+    return fail(set_err(FQ_ERR_UNSUPPORTED, "Unsupported on the device path: a Utf8 array of more than 2 GiB of string bytes (%llu)", h[0]));
+  if (fq_status st = sort_scan(ctx, (fq_u32 *)a->offsets, n + 1, sums, s)) return fail(st);
+  a->bytes = h[0];
+  e = cudaMalloc(&a->data, a->bytes ? a->bytes : 1);
+  if (e != cudaSuccess) return fail(set_err(FQ_ERR_CUDA, "CUDA error: %s (Utf8 take of %llu bytes)", cudaGetErrorString(e), h[0]));
+  if (n && a->bytes) {
+    fq_utf8_gather_bytes<<<grid_for(ctx, 32 * n, 16), 256, 0, s>>>(src->offsets, src->data, rows, rv, n, a->offsets, a->data);
+    ctx->launches++;
+  }
+  e = cudaGetLastError();
+  if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+  if (e != cudaSuccess) return fail(set_err(FQ_ERR_CUDA, "CUDA error: %s (Utf8 take of %" PRIu64 " rows)", cudaGetErrorString(e), n));
+  *out = a;
+  return FQ_OK;
+}
+}  // namespace
+
+extern "C" {
+
+uint64_t fq_utf8_bytes(const fq_utf8 *a) { return a ? a->bytes : 0; }
+
+fq_status fq_utf8_download(fq_ctx *ctx, const fq_utf8 *a, int32_t *offsets_host, void *data_host, void *stream) {
+  if (fq_status st = use(ctx)) return st;
+  if (!a || !offsets_host || (a->bytes && !data_host)) return set_err(FQ_ERR_INVALID, "Internal Error: null argument");
+  CUDA_TRY(cudaMemcpyAsync(offsets_host, a->offsets, sizeof(int32_t) * (a->len + 1), cudaMemcpyDeviceToHost, (cudaStream_t)stream));
+  if (a->bytes) CUDA_TRY(cudaMemcpyAsync(data_host, a->data, a->bytes, cudaMemcpyDeviceToHost, (cudaStream_t)stream));
+  return FQ_OK;
+}
+
+fq_status fq_utf8_take(fq_ctx *ctx, const fq_utf8 *src, const fq_column *rows, uint64_t n, const fq_column *rows_validity, fq_utf8 **out,
+                       void *stream) {
+  if (fq_status st = use(ctx)) return st;
+  if (!src || !rows || !out) return set_err(FQ_ERR_INVALID, "Internal Error: null argument");
+  *out = nullptr;
+  if (rows->dtype != FQ_U32 || rows->len < n) return set_err(FQ_ERR_INVALID, "Internal Error: row indexes must be a UInt32 column with at least n slots");
+  if (rows_validity && (rows_validity->dtype != FQ_BOOL || rows_validity->len < n))
+    return set_err(FQ_ERR_INVALID, "Internal Error: the validity of the row indexes must be a Boolean column with at least n slots");
+  return utf8_take(ctx, src, (const fq_u32 *)rows->ptr, n, rows_validity, (cudaStream_t)stream, out);
+}
+
+fq_status fq_utf8_dict_encode(fq_ctx *ctx, const fq_utf8 *src, fq_column *codes, fq_utf8 **dict, void *stream) {
+  if (fq_status st = use(ctx)) return st;
+  if (!src || !codes || !dict) return set_err(FQ_ERR_INVALID, "Internal Error: null argument");
+  *dict = nullptr;
+  const uint64_t n = src->len;
+  if (codes->dtype != FQ_U32 || codes->len < n) return set_err(FQ_ERR_INVALID, "Internal Error: the codes column must be UInt32 with a slot per row");
+  if (n >= 0xFFFFFFFFull) return set_err(FQ_ERR_UNSUPPORTED, "Unsupported on the device path: dictionary encoding of 2^32 - 1 rows or more");
+  if (ctx->recording) return set_err(FQ_ERR_INVALID, "Internal Error: dictionary encoding cannot be recorded into a graph (it depends on the data)");
+  cudaStream_t s = (cudaStream_t)stream;
+  const fq_u8 *valid = src->validity ? (const fq_u8 *)src->validity->ptr : nullptr;
+  // table: a power of two of at least 2 slots per row (at most 2^32, which still exceeds the row count: no retry)
+  uint64_t cap = 1024;
+  while (cap < 2 * n && cap < (1ull << 32)) cap <<= 1;
+  StreamScratch scratch(s);
+  unsigned long long *table = nullptr;
+  fq_u32 *slot_of = nullptr, *ids = nullptr, *sums = nullptr, *small = nullptr;
+  CUDA_TRY(scratch.get(&table, 8 * cap));
+  CUDA_TRY(scratch.get(&slot_of, 4 * n));
+  CUDA_TRY(scratch.get(&ids, 4 * cap));
+  CUDA_TRY(scratch.get(&sums, 4 * ((cap + FQ_SCAN_TILE - 1) / FQ_SCAN_TILE)));
+  CUDA_TRY(scratch.get(&small, 16));
+  CUDA_TRY(cudaMemsetAsync(small, 0, 16, s));
+  fq_dict_clear<<<grid_for(ctx, cap), 256, 0, s>>>(table, cap);
+  if (n) fq_dict_insert<<<grid_for(ctx, n, 16), 256, 0, s>>>(src->offsets, src->data, valid, n, table, cap - 1, slot_of);
+  fq_dict_flag<<<grid_for(ctx, cap), 256, 0, s>>>(table, cap, ids);
+  CUDA_TRY(cudaGetLastError());
+  ctx->launches += n ? 3 : 2;
+  uint32_t last[2] = {0, 0};
+  CUDA_TRY(cudaMemcpyAsync(&last[0], ids + cap - 1, 4, cudaMemcpyDeviceToHost, s));
+  if (fq_status st = sort_scan(ctx, ids, cap, sums, s)) return st;
+  CUDA_TRY(cudaMemcpyAsync(&last[1], ids + cap - 1, 4, cudaMemcpyDeviceToHost, s));
+  CUDA_TRY(cudaStreamSynchronize(s));
+  const uint64_t d = (uint64_t)last[0] + last[1];   // distinct valid strings
+  fq_u32 *rep = nullptr, *lens = nullptr, *rank = nullptr, *rows = nullptr;
+  fq_u64 *chunk = nullptr;
+  CUDA_TRY(scratch.get(&rep, 4 * d));
+  CUDA_TRY(scratch.get(&lens, 4 * d));
+  CUDA_TRY(scratch.get(&rank, 4 * d));
+  CUDA_TRY(scratch.get(&rows, 4 * d));
+  CUDA_TRY(scratch.get(&chunk, 8 * d));
+  if (d) {
+    fq_dict_compact<<<grid_for(ctx, cap), 256, 0, s>>>(table, cap, ids, src->offsets, rep, lens, small);
+    CUDA_TRY(cudaGetLastError());
+    ctx->launches++;
+    uint32_t max_len = 0;
+    CUDA_TRY(cudaMemcpyAsync(&max_len, small, 4, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaStreamSynchronize(s));
+    // bytewise order of the distinct strings: stable LSD sort by length, then by chunk K-1 down to chunk 0
+    std::lock_guard<std::mutex> sort_lock(ctx->sort_mu);
+    SortJob job{ctx, s};
+    if (fq_status st = job.acquire(d)) return st;
+    fq_column key;
+    key.dtype = FQ_U32;
+    key.len = d;
+    key.ptr = lens;
+    const fq_column *kp = &key;
+    if (fq_status st = job.sort_by_keys(&kp, nullptr, 1, d, false)) return st;
+    key.dtype = FQ_U64;
+    key.ptr = chunk;
+    for (int64_t j = ((int64_t)max_len + 7) / 8 - 1; j >= 0; j--) {
+      fq_dict_chunk<<<grid_for(ctx, d), 256, 0, s>>>(src->offsets, src->data, rep, d, (fq_u32)j, chunk);
+      CUDA_TRY(cudaGetLastError());
+      ctx->launches++;
+      if (fq_status st = job.sort_by_keys(&kp, nullptr, 1, d, true)) return st;
+    }
+    fq_dict_rank<<<grid_for(ctx, d), 256, 0, s>>>(job.idx[job.cur], d, rep, rank, rows);
+    CUDA_TRY(cudaGetLastError());
+    ctx->launches++;
+    CUDA_TRY(cudaEventRecord(ctx->sort_done, s));   // the sort scratch is free again after this point of the stream
+  }
+  if (n) {
+    fq_dict_codes<<<grid_for(ctx, n, 16), 256, 0, s>>>(valid, n, slot_of, ids, rank, (fq_u32 *)codes->ptr);
+    CUDA_TRY(cudaGetLastError());
+    ctx->launches++;
+  }
+  // the dictionary: the representative rows in sorted order (waits for the stream)
+  return utf8_take(ctx, src, rows, d, nullptr, s, dict);
+}
+
+fq_status fq_utf8_bounds(fq_ctx *ctx, const fq_utf8 *dict, const void *scalar, uint64_t scalar_len, uint64_t *lower, uint64_t *upper,
+                         void *stream) {
+  if (fq_status st = use(ctx)) return st;
+  if (!dict || !lower || !upper || (scalar_len && !scalar)) return set_err(FQ_ERR_INVALID, "Internal Error: null argument");
+  if (scalar_len > (uint64_t)INT32_MAX) return set_err(FQ_ERR_INVALID, "Internal Error: literal over 2 GiB");
+  cudaStream_t s = (cudaStream_t)stream;
+  StreamScratch scratch(s);
+  unsigned char *x = nullptr;
+  unsigned long long *out = nullptr;
+  CUDA_TRY(scratch.get(&x, scalar_len));
+  CUDA_TRY(scratch.get(&out, 16));
+  if (scalar_len) CUDA_TRY(cudaMemcpyAsync(x, scalar, scalar_len, cudaMemcpyHostToDevice, s));
+  fq_utf8_bounds_kernel<<<1, 1, 0, s>>>(dict->offsets, dict->data, dict->len, x, (fq_u32)scalar_len, out);
+  CUDA_TRY(cudaGetLastError());
+  ctx->launches++;
+  unsigned long long h[2];
+  CUDA_TRY(cudaMemcpyAsync(h, out, 16, cudaMemcpyDeviceToHost, s));
+  CUDA_TRY(cudaStreamSynchronize(s));
+  *lower = h[0];
+  *upper = h[1];
   return FQ_OK;
 }
 

@@ -408,6 +408,40 @@ PipeHandle::~PipeHandle() {
   if (pipe) fq_pipe_destroy(ctx ? ctx->raw() : nullptr, pipe);
 }
 
+Utf8Dict::~Utf8Dict() {
+  if (raw) fq_utf8_free(ctx ? ctx->raw() : nullptr, raw);
+}
+// strings rows[0 .. n) of `src` (NULL slots, per `valid`, as "") copied to the host
+static std::vector<std::string> decode_rows(const GpuContextRef &ctx, const fq_utf8 *src, const fq_column *rows, uint64_t n, const fq_column *valid) {
+  fq_utf8 *t = nullptr;
+  ctx->check(fq_utf8_take(ctx->raw(), src, rows, n, valid, &t, ctx->stream));
+  std::vector<int32_t> off(n + 1, 0);
+  std::string bytes(fq_utf8_bytes(t), '\0');
+  fq_status st = fq_utf8_download(ctx->raw(), t, off.data(), bytes.data(), ctx->stream);
+  if (st == FQ_OK) st = fq_stream_synchronize(ctx->raw(), ctx->stream);
+  fq_utf8_free(ctx->raw(), t);
+  ctx->check(st);
+  std::vector<std::string> out(n);
+  for (uint64_t i = 0; i < n; i++) out[i] = bytes.substr((size_t)off[i], (size_t)(off[i + 1] - off[i]));
+  return out;
+}
+std::string Utf8Dict::at(uint32_t code) const {
+  if (code >= size) throw FuseQueryError::internal("dictionary code " + std::to_string(code) + " out of range");
+  DataArrayRef rows = DataArray::from_host(ctx, FQ_U32, &code, 1);
+  return decode_rows(ctx, raw, rows->column(), 1, nullptr)[0];
+}
+
+std::pair<uint64_t, uint64_t> Utf8Dict::bounds(const std::string &literal) const {
+  std::lock_guard<std::mutex> lock(mu_);
+  auto it = bounds_.find(literal);
+  if (it != bounds_.end()) return it->second;
+  std::pair<uint64_t, uint64_t> b;
+  ctx->check(fq_utf8_bounds(ctx->raw(), raw, literal.data(), literal.size(), &b.first, &b.second, ctx->stream));
+  if (bounds_.size() >= 4096) bounds_.clear();   // many distinct literals: keep the memory bounded
+  bounds_[literal] = b;
+  return b;
+}
+
 DataArray::~DataArray() {
   if (col_) fq_column_free(ctx_ ? ctx_->raw() : nullptr, col_);
 }
@@ -451,7 +485,7 @@ std::vector<unsigned char> DataArray::to_arrow_bitmap() const {
   return out;
 }
 void DataArray::set_validity(DataArrayRef validity) {
-  if (is_utf8()) throw FuseQueryError::internal("validity on a Utf8 array is not supported");
+  if (is_host_utf8()) throw FuseQueryError::internal("validity on a Utf8 array is not supported");
   if (validity && (validity->data_type() != FQ_BOOL || validity->len() < len_)) throw FuseQueryError::internal("validity must be a Boolean array of the same length");
   ctx_->check(fq_column_set_validity(ctx_->raw(), col_, validity ? validity->column() : nullptr));
   validity_ = std::move(validity);
@@ -471,8 +505,39 @@ DataArrayRef DataArray::utf8(std::vector<std::string> values) {
   a->strings_ = std::move(values);
   return a;
 }
+DataArrayRef DataArray::utf8_dict(GpuContextRef ctx, const int32_t *offsets, const void *data, uint64_t len, const unsigned char *valid) {
+  DataArrayRef v = valid ? from_host(ctx, FQ_BOOL, valid, len) : nullptr;
+  fq_utf8 *src = nullptr;
+  ctx->check(fq_utf8_create(ctx->raw(), offsets, data, len, v ? v->column() : nullptr, ctx->stream, &src));
+  DataArrayRef codes = alloc(ctx, FQ_U32, len);
+  auto d = std::make_shared<Utf8Dict>();
+  d->ctx = ctx;
+  const fq_status st = fq_utf8_dict_encode(ctx->raw(), src, codes->column(), &d->raw, ctx->stream);
+  fq_utf8_free(ctx->raw(), src);
+  ctx->check(st);
+  d->size = fq_utf8_len(d->raw);
+  if (v) codes->set_validity(v);
+  return with_dict(codes, d);
+}
+DataArrayRef DataArray::with_dict(const DataArrayRef &codes, Utf8DictRef dict) {
+  if (codes->data_type() != FQ_U32 || codes->dict_) throw FuseQueryError::internal("dictionary codes must be a UInt32 array");
+  fq_column *c = nullptr;
+  codes->ctx_->check(fq_column_slice(codes->ctx_->raw(), codes->col_, 0, codes->len_, &c));
+  DataArrayRef a = device(codes->ctx_, c, codes->parent_ ? codes->parent_ : codes);   // a view: the codes stay alive
+  a->validity_ = codes->validity_;
+  a->dtype_ = FQ_UTF8;
+  a->dict_ = std::move(dict);
+  return a;
+}
+const std::vector<std::string> &DataArray::strings() const {
+  if (dict_ && !decoded_) {
+    strings_ = len_ ? decode_rows(ctx_, dict_->raw, col_, len_, validity_ ? validity_->column() : nullptr) : std::vector<std::string>{};
+    decoded_ = true;
+  }
+  return strings_;
+}
 DataArrayRef DataArray::slice(uint64_t offset, uint64_t len) {
-  if (is_utf8()) {
+  if (is_host_utf8()) {
     std::vector<std::string> v(strings_.begin() + (long)std::min<uint64_t>(offset, len_), strings_.begin() + (long)std::min<uint64_t>(offset + len, len_));
     return utf8(std::move(v));
   }
@@ -480,6 +545,8 @@ DataArrayRef DataArray::slice(uint64_t offset, uint64_t len) {
   ctx_->check(fq_column_slice(ctx_->raw(), col_, offset, len, &c));
   DataArrayRef out = device(ctx_, c, parent_ ? parent_ : shared_from_this());  // the owner of the buffer stays alive
   if (validity_) out->validity_ = validity_->slice(offset, len);   // the C ABI sliced the device validity alongside
+  out->dtype_ = dtype_;   // a dictionary array's slice shares its dictionary
+  out->dict_ = dict_;
   return out;
 }
 void DataArray::to_host(void *out) const {
@@ -491,7 +558,15 @@ void DataArray::to_host(void *out) const {
 // DataValue::try_from_array (data_value.rs:115-161)
 DataValue DataArray::value(uint64_t index) const {
   if (index >= len_) throw FuseQueryError::internal("index out of bounds: the len is " + std::to_string(len_) + " but the index is " + std::to_string(index));
-  if (is_utf8()) return DataValue::String(strings_[index]);
+  if (is_host_utf8()) return DataValue::String(strings_[index]);
+  if (dict_) {
+    unsigned char ok = 1;
+    if (validity_) {
+      ctx_->check(fq_column_download(ctx_->raw(), validity_->column(), index, &ok, 1, ctx_->stream));
+      ctx_->check(fq_stream_synchronize(ctx_->raw(), ctx_->stream));
+    }
+    return ok ? DataValue::String(strings()[index]) : DataValue::None(FQ_UTF8);
+  }
   unsigned char buf[8] = {0};
   ctx_->check(fq_column_download(ctx_->raw(), col_, index, buf, 1, ctx_->stream));
   ctx_->check(fq_stream_synchronize(ctx_->raw(), ctx_->stream));

@@ -88,8 +88,26 @@ using DataSchemaRef = std::shared_ptr<const DataSchema>;
 class GpuContext;
 using GpuContextRef = std::shared_ptr<GpuContext>;
 
-// ArrayRef (data_array.rs): a device-resident Arrow-layout column, or a host Utf8 array (partial
-// aggregate states and EXPLAIN text are the only strings on the path)
+// The sorted dictionary of a dictionary-encoded Utf8 column (fq_utf8_dict_encode): distinct valid strings in bytewise
+// order on the device, shared by the column, its slices and every result column decoded through it.
+struct Utf8Dict {
+  GpuContextRef ctx;
+  fq_utf8 *raw = nullptr;
+  uint64_t size = 0;
+  ~Utf8Dict();
+  std::string at(uint32_t code) const;   // one entry, through fq_utf8_take
+  // fq_utf8_bounds of a literal, remembered: a dictionary never changes, and every pipe of a query lowers the same literals
+  std::pair<uint64_t, uint64_t> bounds(const std::string &literal) const;
+
+ private:
+  mutable std::mutex mu_;
+  mutable std::map<std::string, std::pair<uint64_t, uint64_t>> bounds_;
+};
+using Utf8DictRef = std::shared_ptr<const Utf8Dict>;
+
+// ArrayRef (data_array.rs): a device-resident Arrow-layout column, a host Utf8 array (partial aggregate states and
+// EXPLAIN text), or a dictionary-encoded Utf8 column: UInt32 codes on the device (with the column's validity) over a
+// shared sorted dictionary, decoded lazily when its strings are asked for
 class DataArray : public std::enable_shared_from_this<DataArray> {
  public:
   ~DataArray();
@@ -104,11 +122,19 @@ class DataArray : public std::enable_shared_from_this<DataArray> {
   const std::shared_ptr<DataArray> &validity() const { return validity_; }
   uint64_t null_count() const;
   static std::shared_ptr<DataArray> utf8(std::vector<std::string> values);
+  // Arrow strings (int32 offsets[len + 1] starting at 0, the bytes, optional validity bytes 1 = valid) uploaded and
+  // dictionary-encoded on the device
+  static std::shared_ptr<DataArray> utf8_dict(GpuContextRef ctx, const int32_t *offsets, const void *data, uint64_t len,
+                                              const unsigned char *valid);
+  // a UInt32 codes array (its validity included) read as strings of `dict`
+  static std::shared_ptr<DataArray> with_dict(const std::shared_ptr<DataArray> &codes, Utf8DictRef dict);
   DataType data_type() const { return dtype_; }
   uint64_t len() const { return len_; }
   bool is_utf8() const { return dtype_ == FQ_UTF8; }
-  fq_column *column() const { return col_; }
-  const std::vector<std::string> &strings() const { return strings_; }
+  bool is_host_utf8() const { return dtype_ == FQ_UTF8 && !dict_; }
+  const Utf8DictRef &dict() const { return dict_; }
+  fq_column *column() const { return col_; }   // dictionary arrays: the codes
+  const std::vector<std::string> &strings() const;   // dictionary arrays: decoded on first use ("" in NULL slots)
   std::shared_ptr<DataArray> slice(uint64_t offset, uint64_t len);   // arrow::compute::limit == slice(0, n)
   void to_host(void *out) const;                                      // len * size bytes
   DataValue value(uint64_t index) const;                              // DataValue::try_from_array
@@ -122,7 +148,9 @@ class DataArray : public std::enable_shared_from_this<DataArray> {
   fq_column *col_ = nullptr;
   std::shared_ptr<DataArray> parent_;
   std::shared_ptr<DataArray> validity_;
-  std::vector<std::string> strings_;
+  mutable std::vector<std::string> strings_;
+  Utf8DictRef dict_;
+  mutable bool decoded_ = false;
 };
 using DataArrayRef = std::shared_ptr<DataArray>;
 

@@ -30,17 +30,91 @@ int Lowering::column_of(const DataBlock &block, const std::string &name) {
     if (!block_cols.empty() || bi != 0) throw FuseQueryError::internal("generated block column must be referenced first");
     generated = true;
   } else if (t == FQ_UTF8) {
-    throw FuseQueryError::internal("Unsupported on the device path: Utf8 column in an expression");
+    if (!block.column((size_t)bi)->dict()) throw FuseQueryError::internal("Unsupported on the device path: Utf8 column in an expression");
+    t = FQ_U32;   // a dictionary column enters the pipe as its codes
   }
   block_cols.push_back(bi);
   col_dtypes.push_back(t);
   col_nullable.push_back(!block.generated && block.column((size_t)bi)->validity() ? 1 : 0);
   return (int)block_cols.size() - 1;
 }
+Utf8DictRef dict_of(const Function &f, const DataBlock &block) {
+  const Function *g = &f;
+  while (g->kind == Function::Alias) g = g->left.get();
+  if (g->kind != Function::Variable || block.generated) return nullptr;
+  const auto &fields = block.schema()->fields;
+  for (size_t i = 0; i < fields.size() && i < block.num_columns(); i++)
+    if (fields[i].name == g->name) return block.column(i)->dict();
+  return nullptr;   // not a column of the block: lowering reports it
+
+}
+DataValue Lowering::decode_leaf(const Function &leaf, DataValue v) const {
+  auto it = leaf_dict.find(&leaf);
+  if (it == leaf_dict.end()) return v;
+  return v.some ? DataValue::String(it->second->at((uint32_t)v.u)) : DataValue::None(FQ_UTF8);
+}
+// `col op literal` over the codes of a sorted dictionary (the lowering table of fq_utf8_dict_encode in fuse_gpu.h)
+static void dict_comparison(const Utf8Dict &d, int op, const DataValue &lit, int *code_op, uint64_t *code) {
+  if (!lit.some) throw FuseQueryError::internal("DataValue to array cannot be NONE " + lit.to_string());
+  const auto [lb, ub] = d.bounds(lit.s);
+  switch (op) {
+    case FQ_CMP_EQ: *code_op = FQ_CMP_EQ; *code = lb < ub ? lb : d.size; break;
+    case FQ_CMP_LT: *code_op = FQ_CMP_LT; *code = lb; break;
+    case FQ_CMP_LTEQ: *code_op = FQ_CMP_LT; *code = ub; break;
+    case FQ_CMP_GT: *code_op = FQ_CMP_GTEQ; *code = ub; break;
+    default: *code_op = FQ_CMP_GTEQ; *code = lb; break;
+  }
+}
 int Lowering::lower(const Function &f, const DataBlock &block) {
   fq_expr_node n;
   memset(&n, 0, sizeof n);
   n.left = n.right = -1;
+  if (f.kind == Function::Arithmetic || f.kind == Function::Comparison || f.kind == Function::Logic) {
+    const Utf8DictRef ld = dict_of(*f.left, block), rd = dict_of(*f.right, block);
+    if (ld || rd) {
+      const DataSchema &sc = *block.schema();
+      const DataType lt = f.left->return_type(sc), rt = f.right->return_type(sc);
+      if (f.kind == Function::Arithmetic) numerical_coercion(arith_sym(f.op), lt, rt);   // throws "Unsupported (Utf8) + (..)"
+      if (f.kind != Function::Comparison)
+        throw FuseQueryError::internal(std::string("Unsupported on the device path: Utf8 operand of ") +
+                                       (f.kind == Function::Arithmetic ? arith_sym(f.op) : logic_sym(f.op)));
+      if (lt != FQ_UTF8 || rt != FQ_UTF8) numerical_coercion(cmp_sym(f.op), lt, rt);   // throws "Unsupported (Utf8) = (Int8)"
+      if (ld && rd && ld != rd)
+        throw FuseQueryError::internal("Unsupported on the device path: comparison of two Utf8 columns with different dictionaries");
+      if (!(ld && rd)) {
+        // column (op) literal, or literal (op) column flipped first (data_array_comparison.rs:75-85)
+        static const int flipped[] = {FQ_CMP_EQ, FQ_CMP_GT, FQ_CMP_GTEQ, FQ_CMP_LT, FQ_CMP_LTEQ};
+        const Function &col = ld ? *f.left : *f.right, &other = ld ? *f.right : *f.left;
+        const Function *lit = &other;
+        while (lit->kind == Function::Alias) lit = lit->left.get();
+        if (lit->kind != Function::Constant)
+          throw FuseQueryError::internal("Unsupported on the device path: Utf8 comparison with a computed string");
+        int code_op = 0;
+        uint64_t code = 0;
+        dict_comparison(ld ? *ld : *rd, ld ? f.op % 5 : flipped[f.op % 5], lit->value, &code_op, &code);
+        n.kind = FQ_EXPR_COMPARISON;
+        n.op = code_op;
+        n.left = lower(col, block);
+        fq_expr_node c;
+        memset(&c, 0, sizeof c);
+        c.left = c.right = -1;
+        c.kind = FQ_EXPR_CONSTANT;
+        c.dtype = FQ_U32;
+        c.value.u = code;
+        nodes.push_back(c);
+        n.right = (int)nodes.size() - 1;
+        nodes.push_back(n);
+        node_of[&f] = (int)nodes.size() - 1;
+        return (int)nodes.size() - 1;
+      }
+    }
+  }
+  if (f.kind == Function::Aggregator) {
+    if (Utf8DictRef d = dict_of(*f.left, block)) {
+      if (f.op == FQ_AGG_SUM) throw FuseQueryError::internal("Unsupported data_array_sum for data type: Utf8");
+      if (f.op != FQ_AGG_COUNT) leaf_dict[&f] = d;
+    }
+  }
   switch (f.kind) {
     case Function::Variable:
       n.kind = FQ_EXPR_FIELD;
@@ -166,8 +240,10 @@ ProjectResult run_project(GpuContextRef ctx, const DataBlock &block, const Funct
     res.limit_reached = true;
     ctx->check(fq_pipe_fetch_limit_row(ctx->raw(), pipe->pipe, &res.limit_row));
   }
-  for (size_t e = 0; e < funcs.size(); e++)
+  for (size_t e = 0; e < funcs.size(); e++) {
     if (valids[e]) res.columns[e]->set_validity(valids[e]);
+    if (Utf8DictRef d = dict_of(*funcs[e], block)) res.columns[e] = DataArray::with_dict(res.columns[e], d);   // codes out: strings again
+  }
   if (res.rows_written < cap)
     for (auto &c : res.columns) c = c->slice(0, res.rows_written);
   return res;
@@ -365,7 +441,7 @@ void Function::accumulate(GpuContextRef ctx, const DataBlock &block) {
     int32_t n = 0;
     uint64_t sel = 0;
     ctx->check(fq_pipe_fetch_aggregate(ctx->raw(), pipe->pipe, st, 4, &n, &sel));
-    part = DataValue::from_abi(st[0]);
+    part = lw.decode_leaf(*this, DataValue::from_abi(st[0]));
   }
   if (op == FQ_AGG_COUNT || op == FQ_AGG_SUM) value = data_value_arithmetic_op(FQ_AR_ADD, value, part);
   else value = data_value_aggregate_op(op, value, part);
@@ -437,12 +513,17 @@ static DataArrayRef binary_array_op(GpuContextRef ctx, Function::Kind kind, int 
 DataArrayRef data_array_arithmetic_op(GpuContextRef ctx, int op, const DataColumnarValue &l, const DataColumnarValue &r) {
   return binary_array_op(std::move(ctx), Function::Arithmetic, op, l, r);
 }
-// A Utf8 DataArray keeps its strings on the host; for a kernel it is packed into Arrow's offsets + bytes and uploaded.
+// A host Utf8 DataArray keeps its strings on the host; for a kernel it is packed into Arrow's offsets + bytes and uploaded.
+// A dictionary array is decoded on the device, with its validity.
 namespace {
 struct DeviceUtf8 {
   GpuContextRef ctx;
   fq_utf8 *raw = nullptr;
   DeviceUtf8(GpuContextRef c, const DataArray &a) : ctx(std::move(c)) {
+    if (a.dict()) {
+      ctx->check(fq_utf8_take(ctx->raw(), a.dict()->raw, a.column(), a.len(), a.validity() ? a.validity()->column() : nullptr, &raw, ctx->stream));
+      return;
+    }
     const auto &strs = a.strings();
     std::vector<int32_t> offsets(strs.size() + 1, 0);
     std::string data;
@@ -470,18 +551,23 @@ DataArrayRef data_array_comparison_op(GpuContextRef ctx, int op, const DataColum
   static const int flipped[] = {FQ_CMP_EQ, FQ_CMP_GT, FQ_CMP_GTEQ, FQ_CMP_LT, FQ_CMP_LTEQ};   // scalar (op) array = array (flipped op) scalar, :75-85
   const DataArrayRef &arr = l.is_scalar ? r.array : l.array;
   DataArrayRef out = DataArray::alloc(ctx, FQ_BOOL, arr->len());
+  // NULL slots of dictionary arrays compare to NULL
+  const bool nullable = (!l.is_scalar && l.array->validity()) || (!r.is_scalar && r.array->validity());
+  DataArrayRef out_valid = nullable ? DataArray::alloc(ctx, FQ_BOOL, arr->len()) : nullptr;
+  fq_column *ov = out_valid ? out_valid->column() : nullptr;
   DeviceUtf8 a(ctx, *arr);
   if (l.is_scalar || r.is_scalar) {
     const DataValue &sc = l.is_scalar ? l.scalar : r.scalar;
     if (!sc.some) throw FuseQueryError::internal("DataValue to array cannot be NONE " + sc.to_string());
-    ctx->check(fq_utf8_compare_scalar(ctx->raw(), l.is_scalar ? flipped[op % 5] : op, a.raw, sc.s.data(), sc.s.size(), out->column(), nullptr, ctx->stream));
+    ctx->check(fq_utf8_compare_scalar(ctx->raw(), l.is_scalar ? flipped[op % 5] : op, a.raw, sc.s.data(), sc.s.size(), out->column(), ov, ctx->stream));
   } else {
     if (l.array->len() != r.array->len())
       throw FuseQueryError::internal("Compute error: Cannot perform comparison operation on arrays of different length");
     DeviceUtf8 b(ctx, *r.array);
-    ctx->check(fq_utf8_compare(ctx->raw(), op, a.raw, b.raw, out->column(), nullptr, ctx->stream));
+    ctx->check(fq_utf8_compare(ctx->raw(), op, a.raw, b.raw, out->column(), ov, ctx->stream));
     ctx->check(fq_stream_synchronize(ctx->raw(), ctx->stream));
   }
+  if (out_valid) out->set_validity(out_valid);
   return out;
 }
 DataArrayRef data_array_logic_op(GpuContextRef ctx, int op, const DataColumnarValue &l, const DataColumnarValue &r) {

@@ -12,11 +12,17 @@ struct Lowering {
   std::vector<DataType> col_dtypes;
   std::vector<int> col_nullable;
   std::map<const Function *, int> node_of;
+  std::map<const Function *, Utf8DictRef> leaf_dict;   // min / max leaves over a dictionary column: their state is a code
   bool generated = false;
   int column_of(const DataBlock &block, const std::string &name);
   int lower(const Function &f, const DataBlock &block);
   fq_pipe_desc desc(int kind, int predicate, const std::vector<int> &roots) const;
+  // the state of Aggregator leaf `leaf` as the reference holds it: a code of a dictionary column becomes its string
+  DataValue decode_leaf(const Function &leaf, DataValue v) const;
 };
+
+// the dictionary of `f` when it is a dictionary-encoded Utf8 column of `block` (possibly under aliases), else null
+Utf8DictRef dict_of(const Function &f, const DataBlock &block);
 
 struct BoundSource {
   fq_source src;

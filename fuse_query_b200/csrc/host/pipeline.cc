@@ -435,14 +435,19 @@ SendableDataBlockStream GpuSortTransform::execute() {
   // every block of the input as one block (a sort is a pipeline breaker)
   std::vector<DataArrayRef> cols(n_cols);
   for (size_t c = 0; c < n_cols; c++) {
-    if (blocks[0].column(c)->is_utf8()) throw FuseQueryError::internal("Unsupported on the device path: ORDER BY over a block with a Utf8 column");
+    if (blocks[0].column(c)->is_host_utf8()) throw FuseQueryError::internal("Unsupported on the device path: ORDER BY over a block with a Utf8 column");
     if (blocks.size() == 1) {
       cols[c] = blocks[0].column(c);
       continue;
     }
+    // a dictionary column is concatenated as its codes: every block must carry the same dictionary
+    const Utf8DictRef dict = blocks[0].column(c)->dict();
     bool nullable = false;
-    for (const auto &b : blocks) nullable = nullable || b.column(c)->validity();
-    cols[c] = DataArray::alloc(gpu, blocks[0].column(c)->data_type(), n);
+    for (const auto &b : blocks) {
+      nullable = nullable || b.column(c)->validity();
+      if (b.column(c)->dict() != dict) throw FuseQueryError::internal("Unsupported on the device path: ORDER BY over Utf8 blocks with different dictionaries");
+    }
+    cols[c] = DataArray::alloc(gpu, dict ? (DataType)FQ_U32 : blocks[0].column(c)->data_type(), n);
     DataArrayRef valid = nullable ? DataArray::alloc(gpu, FQ_BOOL, n) : nullptr;
     uint64_t at = 0;
     for (const auto &b : blocks) {
@@ -460,6 +465,7 @@ SendableDataBlockStream GpuSortTransform::execute() {
       at += src->len();
     }
     if (valid) cols[c]->set_validity(valid);
+    if (dict) cols[c] = DataArray::with_dict(cols[c], dict);
   }
   gpu->check(fq_stream_synchronize(gpu->raw(), gpu->stream));
   DataBlock all(schema, cols);
@@ -485,10 +491,12 @@ SendableDataBlockStream GpuSortTransform::execute() {
   if (out_rows == 0) return std::make_unique<DataBlockStream>(std::vector<DataBlock>{});
   std::vector<DataArrayRef> sorted(n_cols);
   for (size_t c = 0; c < n_cols; c++) {
-    sorted[c] = DataArray::alloc(gpu, cols[c]->data_type(), out_rows);
+    const Utf8DictRef &dict = cols[c]->dict();
+    sorted[c] = DataArray::alloc(gpu, dict ? (DataType)FQ_U32 : cols[c]->data_type(), out_rows);
     DataArrayRef valid = cols[c]->validity() ? DataArray::alloc(gpu, FQ_BOOL, out_rows) : nullptr;
     gpu->check(fq_column_take(gpu->raw(), cols[c]->column(), rows->column(), out_rows, sorted[c]->column(), valid ? valid->column() : nullptr, gpu->stream));
     if (valid) sorted[c]->set_validity(valid);
+    if (dict) sorted[c] = DataArray::with_dict(sorted[c], dict);
   }
   gpu->check(fq_stream_synchronize(gpu->raw(), gpu->stream));
   return std::make_unique<DataBlockStream>(std::vector<DataBlock>{DataBlock(schema, sorted)});
@@ -632,7 +640,7 @@ SendableDataBlockStream GpuPipeTransform::execute() {
       for (const Function *l : pt.leaves) {
         int node = pt.lw.node_of.at(l);
         for (int k = 0; k < nn; k++)
-          if (nodes[k] == node) leaf_state[l] = DataValue::from_abi(st[k]);
+          if (nodes[k] == node) leaf_state[l] = pt.lw.decode_leaf(*l, DataValue::from_abi(st[k]));
       }
     }
     std::vector<std::string> rows;
@@ -721,6 +729,7 @@ SendableDataBlockStream GpuGroupByTransform::execute() {
 
   PipeRef pipe;
   Lowering lw;
+  std::vector<Utf8DictRef> key_dicts;   // GROUP BY a dictionary column: its codes are the key
   uint64_t hint = 1 << 16, n_groups = 0;
   for (;;) {   // the table is grown until the groups fit (a full re-scan: cardinality is unknown up front)
     struct OptionsGuard {
@@ -743,7 +752,10 @@ SendableDataBlockStream GpuGroupByTransform::execute() {
         const int p = pred ? lw.lower(*pred, *block) : -1;
         std::vector<int> roots, key_roots;
         for (auto &f : funcs) roots.push_back(lw.lower(*f, *block));
-        for (auto &k : keys) key_roots.push_back(lw.lower(*k, *block));
+        for (auto &k : keys) {
+          key_roots.push_back(lw.lower(*k, *block));
+          key_dicts.push_back(dict_of(*k, *block));
+        }
         fq_pipe_desc d = lw.desc(FQ_PIPE_GROUPBY, p, roots);
         d.n_keys = (int)key_roots.size();
         for (size_t k = 0; k < key_roots.size(); k++) d.keys[k] = key_roots[k];
@@ -764,7 +776,7 @@ SendableDataBlockStream GpuGroupByTransform::execute() {
 
   std::vector<DataArrayRef> out;
   if (!pipe || n_groups == 0) {   // an empty result still carries the plan's schema
-    for (const auto &f : schema_->fields) out.push_back(DataArray::alloc(gpu, f.data_type == FQ_UTF8 ? (DataType)FQ_U8 : f.data_type, 0));
+    for (const auto &f : schema_->fields) out.push_back(f.data_type == FQ_UTF8 ? DataArray::utf8({}) : DataArray::alloc(gpu, f.data_type, 0));
     return std::make_unique<DataBlockStream>(std::vector<DataBlock>{DataBlock(schema_, out)});
   }
   // export: key columns, then one column per Aggregator leaf
@@ -795,13 +807,15 @@ SendableDataBlockStream GpuGroupByTransform::execute() {
   gpu->check(fq_stream_synchronize(gpu->raw(), gpu->stream));
   for (size_t j = 0; j < keys.size(); j++) {
     if (key_valid[j]) key_arrays[j]->set_validity(key_valid[j]);
-    out.push_back(key_arrays[j]);
+    out.push_back(key_dicts[j] ? DataArray::with_dict(key_arrays[j], key_dicts[j]) : key_arrays[j]);
   }
   // the leaf block and the select expressions over it
   auto leaf_schema = std::make_shared<DataSchema>();
   std::map<const Function *, std::string> leaf_name;
   for (int k = 0; k < n_leaves; k++) {
     if (leaf_valid[k]) leaf_arrays[k]->set_validity(leaf_valid[k]);
+    for (const auto &ld : lw.leaf_dict)   // min / max of a dictionary column: codes, read as strings
+      if (lw.node_of.at(ld.first) == nodes[k]) leaf_arrays[k] = DataArray::with_dict(leaf_arrays[k], ld.second);
     leaf_schema->fields.push_back({"__leaf" + std::to_string(k), leaf_arrays[k]->data_type(), leaf_valid[k] != nullptr});
   }
   for (const Function *l : leaves) {

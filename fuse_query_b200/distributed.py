@@ -53,6 +53,9 @@ def execute_sql_distributed(ctx, sql: str, rank: int, world: int, all_gather_obj
                                + " -> ".join(p.name() for p in plans))
     if sort is not None and (sel.name() != "ProjectionPlan" or gpu is None):
         raise h.FuseQueryError("Internal Error: distributed ORDER BY needs a projection query and the rank's device context")
+    if h.DataType.Utf8 in src.schema().types():
+        # dictionary codes are local to the rank's table: rows of different ranks cannot be merged as codes
+        raise h.FuseQueryError("Internal Error: Unsupported on the device path: distributed execution over a table with a Utf8 column")
     parts = _my_partitions(list(src.partitions), rank, world)
     names = sel.schema().names()
     local_blocks = []

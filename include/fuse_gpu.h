@@ -185,6 +185,31 @@ fq_status fq_utf8_compare_scalar(fq_ctx *ctx, int32_t op, const fq_utf8 *l, cons
 /* row index of the smallest (FQ_AGG_MIN) / largest (FQ_AGG_MAX) valid string, first occurrence; -1 when there is none
  * (arrow min_string / max_string return None).  Waits for the result. */
 fq_status fq_utf8_minmax(fq_ctx *ctx, int32_t op, const fq_utf8 *a, int64_t *row, void *stream);
+/* value bytes of the array (offsets[len]) */
+uint64_t fq_utf8_bytes(const fq_utf8 *a);
+/* async copy to host memory: offsets_host receives len + 1 entries, data_host fq_utf8_bytes(a) bytes */
+fq_status fq_utf8_download(fq_ctx *ctx, const fq_utf8 *a, int32_t *offsets_host, void *data_host, void *stream);
+/* Gather by index: *out[i] = src[rows[i]] for i < n (`rows` a UInt32 column, every index < len(src)).  rows_validity (FQ_BOOL,
+ * may be NULL, borrowed: it becomes the validity of *out and must outlive it) marks output slots that are NULL; their rows are
+ * not read.  Fails, instead of truncating, when the result would exceed 2 GiB of value bytes.  Waits for the result. */
+fq_status fq_utf8_take(fq_ctx *ctx, const fq_utf8 *src, const fq_column *rows, uint64_t n, const fq_column *rows_validity, fq_utf8 **out,
+                       void *stream);
+/* Dictionary encoding (fewer than 2^32 - 1 rows).  codes (FQ_U32, at least len(src) slots) receives, for every valid row, the
+ * position of its string in *dict: the distinct valid strings of `src` in bytewise order, with no validity.  NULL rows get code
+ * 0; the caller gives `codes` the source's validity.  Because the dictionary is sorted, code order is string order, and a
+ * Utf8 column `s` with codes `c` lowers to integer work (lb / ub = fq_utf8_bounds of the literal, D = dictionary length):
+ *   s = 'x'                 c = lb when lb < ub (the literal is in the dictionary), else c = D (no row has that code)
+ *   s < 'x', s <= 'x'       c < lb, c < ub
+ *   s > 'x', s >= 'x'       c >= ub, c >= lb
+ *   'x' op s                flip the operator first (data_array_comparison.rs:75-85)
+ *   s op s2                 c op c2, when both columns hold codes of the SAME dictionary
+ *   GROUP BY s / ORDER BY s group / sort by c (NULL rows stay NULL through the codes' validity), then decode with fq_utf8_take
+ *   min(s), max(s)          min / max of c, then the dictionary entry;  count(s) is unchanged
+ * Waits for the result. */
+fq_status fq_utf8_dict_encode(fq_ctx *ctx, const fq_utf8 *src, fq_column *codes, fq_utf8 **dict, void *stream);
+/* lower = the first index of the sorted array `dict` whose string is >= the literal, upper = the first one > it.  Waits. */
+fq_status fq_utf8_bounds(fq_ctx *ctx, const fq_utf8 *dict, const void *scalar, uint64_t scalar_len, uint64_t *lower, uint64_t *upper,
+                         void *stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Source — system.numbers_mt shards.  Replaces NumbersStream::poll_next materialising 10 000-row

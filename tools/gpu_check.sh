@@ -25,6 +25,11 @@ case $what in
   topo|all)
     topo
     ;;
+  utf8)
+    # Utf8 columns: dictionary-encoding throughput and string queries vs the same queries over a UInt32 column
+    # -> profiles/r03_utf8_<rows>.json (the same JSON lines are printed as they are measured)
+    timeout 1200 python tools/bench_utf8.py "$@"; echo "bench_utf8 rc=$?"
+    ;;
   select)
     # select-kernel shapes: timings with the staged pass 2 on / off, then ncu --set full of the dense / third / 1-in-1024 selections
     FQ_SELT_STAGE2=1 timeout 600 python tools/bench_select.py > gpurun_out/bench_select_stage2.log 2>&1; echo "stage2=1 rc=$?"; cat gpurun_out/bench_select_stage2.log
