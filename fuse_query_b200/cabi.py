@@ -794,8 +794,11 @@ class Pipe:
         return n.value
 
     def run_groupby(self, source: Source, *, groups_hint: int = 1 << 16, stream: int = 0) -> int:
-        """reserve -> launch -> fetch, growing the table until the groups fit; returns the number of groups."""
-        hint = groups_hint
+        """reserve -> launch -> fetch, growing the table until the groups fit; returns the number of groups.
+
+        Every reservation after the first rehashes the keys with a new seed.  A scan has at most as many groups as rows,
+        so the table grows to room for every row and no further: two overflows at that size raise."""
+        hint, rows, full_overflows = groups_hint, source.n_rows, 0
         while True:
             self.groupby_reserve(hint)
             self.launch_groupby(source, stream=stream)
@@ -804,7 +807,11 @@ class Pipe:
             except FuseGpuError as e:
                 if e.status != ERR_CAPACITY:
                     raise
-                hint *= 8
+                if hint >= rows:
+                    full_overflows += 1
+                    if full_overflows == 2:
+                        raise FuseGpuError(ERR_CAPACITY, f"GROUP BY: two hash tables with room for all {rows} rows scanned overflowed") from e
+                hint = max(1, min(hint * 8, rows))
 
     def export_groups(self, n_groups: int, stream: int = 0):
         """-> (key columns, key validity columns or None, leaf columns, leaf validity columns or None), device-resident"""

@@ -268,6 +268,8 @@ struct fq_pipe {
   unsigned gb_reps = 1;
   bool gb_reps_dirty = false;        // freshly allocated replicas: fill them once; afterwards the fold leaves them empty
   uint64_t gb_cap = 0;
+  uint64_t gb_seed = 0;              // hash seed of the current table (fq_launch_params::gb_seed)
+  uint64_t gb_reservations = 0;
   uint32_t *gb_flags = nullptr;      // [0] overflow, [1] EMPTY-valued key seen, [2..3] group count (u64), [4..5] error bits
   uint64_t *h_gb = nullptr;          // pinned mirror of gb_flags (4 x u64)
   uint64_t *gb_identity = nullptr;   // device copy of a fresh group's state
@@ -1719,6 +1721,12 @@ std::vector<uint64_t> gb_identity(const fq::Generated &gen) {
   }
   return idn;
 }
+uint64_t splitmix64(uint64_t x) {
+  x += 0x9e3779b97f4a7c15ull;
+  x = (x ^ (x >> 30)) * 0xbf58476d1ce4e5b9ull;
+  x = (x ^ (x >> 27)) * 0x94d049bb133111ebull;
+  return x ^ (x >> 31);
+}
 fq_status gb_check(const fq_pipe *pipe) {
   if (!pipe || pipe->gen.kind != FQ_PIPE_GROUPBY) return set_err(FQ_ERR_INVALID, "Internal Error: not a GROUP BY pipe");
   return FQ_OK;
@@ -1815,6 +1823,9 @@ fq_status fq_pipe_groupby_reserve(fq_ctx *ctx, fq_pipe *pipe, uint64_t groups) {
     CUDA_TRY(cudaMalloc(&pipe->gb_identity, sizeof(uint64_t) * idn.size()));
     CUDA_TRY(cudaMemcpy(pipe->gb_identity, idn.data(), sizeof(uint64_t) * idn.size(), cudaMemcpyHostToDevice));
   }
+  // a new seed for every table after the first: keys whose hashes clustered in the last one (fq_gb_hash is a bijection)
+  // are spread again, while a pipe's first table hashes the keys themselves
+  pipe->gb_seed = pipe->gb_reservations++ ? splitmix64(pipe->gb_reservations) : 0;
   if (fq_status st = gb_clear(ctx, pipe, nullptr)) return st;
   CUDA_TRY(cudaDeviceSynchronize());
   return FQ_OK;
@@ -1851,6 +1862,7 @@ fq_status fq_pipe_launch_groupby(fq_ctx *ctx, fq_pipe *pipe, const fq_source *sr
   p.gb_rep_keys = (fq_u64 *)pipe->gb_rep_keys;
   p.gb_rep_slots = (fq_u64 *)pipe->gb_rep_slots;
   p.gb_reps = pipe->gb_reps;
+  p.gb_seed = pipe->gb_seed;
   p.result = (fq_u64 *)(pipe->gb_flags + 2);   // [0] = count (u64 at flags[2..3]), [1] = error bits (flags[4..5])
   const Kernel &k = pipe->k_groupby;
   if (!k.valid()) return set_err(FQ_ERR_INTERNAL, "Internal Error: no GROUP BY kernel was built for this pipe");
@@ -1986,6 +1998,7 @@ fq_status fq_pipe_merge_partials(fq_ctx *ctx, fq_pipe *pipe, const fq_column *en
     p.gb_slots = (fq_u64 *)pipe->gb_slots;
     p.gb_cap = pipe->gb_cap;
     p.gb_flags = (fq_u32 *)pipe->gb_flags;
+    p.gb_seed = pipe->gb_seed;
     p.gb_entries = (const fq_u64 *)entries->ptr;
     const Kernel &k = pipe->k_gbmerge;
     if (!k.valid()) return set_err(FQ_ERR_INTERNAL, "Internal Error: no GROUP BY merge kernel was built for this pipe");

@@ -598,7 +598,14 @@ DataValue DataArray::value(uint64_t index) const {
 // DataValue::to_array (data_value.rs:76-112): broadcast a scalar to `size` rows on the device
 DataArrayRef DataColumnarValue::to_array(GpuContextRef ctx, uint64_t size) const {
   if (!is_scalar) return array;
-  if (scalar.tag == FQ_UTF8) return DataArray::utf8(std::vector<std::string>(size, scalar.s));
+  if (scalar.tag == FQ_UTF8) {
+    if (scalar.some) return DataArray::utf8(std::vector<std::string>(size, scalar.s));
+    // Utf8(None) (min / max of strings that are all NULL) broadcasts to NULL rows, not to empty strings.  A host Utf8
+    // array carries no validity, so the rows are an all-NULL column encoded like a table's: an empty dictionary
+    std::vector<int32_t> offsets(size + 1, 0);
+    std::vector<unsigned char> valid(size, 0);
+    return DataArray::utf8_dict(std::move(ctx), offsets.data(), "", size, valid.data());
+  }
   require_some(scalar);
   if (scalar.tag == FQ_NULL) throw FuseQueryError::internal("Unsupported on the device path: NullArray");
   // fill through the host: broadcasts only materialise for tiny arrays on this path (merge_result().to_array(1),

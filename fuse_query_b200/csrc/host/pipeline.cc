@@ -731,7 +731,9 @@ SendableDataBlockStream GpuGroupByTransform::execute() {
   Lowering lw;
   std::vector<Utf8DictRef> key_dicts;   // GROUP BY a dictionary column: its codes are the key
   uint64_t hint = 1 << 16, n_groups = 0;
+  int full_overflows = 0;   // overflows of tables with room for every row scanned
   for (;;) {   // the table is grown until the groups fit (a full re-scan: cardinality is unknown up front)
+    uint64_t rows = 0;
     struct OptionsGuard {
       FuseQueryContextRef c;
       GpuOptions saved;
@@ -765,11 +767,19 @@ SendableDataBlockStream GpuGroupByTransform::execute() {
       BoundSource bs;
       bind_source(lw, *block, &bs);
       gpu->check(fq_pipe_launch_groupby(gpu->raw(), pipe->pipe, &bs.src, launches > 0 ? FQ_RUN_ACCUMULATE : 0, gpu->stream));
+      rows += bs.src.n_rows;
       launches++;
     }
     if (!pipe) break;   // no rows at all: no groups
     const fq_status st = fq_pipe_fetch_groupby(gpu->raw(), pipe->pipe, &n_groups);
-    if (st == FQ_ERR_CAPACITY) { hint *= 8; continue; }
+    if (st == FQ_ERR_CAPACITY) {
+      // no scan has more groups than rows: a table with room for all of them overflows only when the keys' hashes cluster,
+      // and the next reservation rehashes them with a new seed.  Two such overflows are an error, not a larger table.
+      if (hint >= rows && full_overflows++)
+        throw FuseQueryError::internal("GROUP BY: two hash tables with room for all " + std::to_string(rows) + " rows scanned overflowed");
+      hint = std::max<uint64_t>(1, std::min(hint * 8, rows));
+      continue;
+    }
     gpu->check(st);
     break;
   }

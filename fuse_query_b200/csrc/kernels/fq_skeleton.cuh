@@ -126,6 +126,7 @@ struct fq_launch_params {
   fq_u64 *gb_rep_keys;    // [gb_reps - 1][gb_cap + 1] replicas of the table: CTA b aggregates into replica b % gb_reps (0 = the
   fq_u64 *gb_rep_slots;   // table itself), the merge kernel folds them into the table and leaves them empty again
   fq_u32 gb_reps;         // >= 1
+  fq_u64 gb_seed;         // xored into every key before it is hashed for this table's slots (0 at a pipe's first reservation)
   // select / map
   void *outs[8];
   void *outs_valid[8];   // per select expression that can yield NULL: one byte per output row
@@ -1743,7 +1744,9 @@ __device__ __forceinline__ void fq_select_tma_kernel(const fq_launch_params &p) 
 // the CTA flushes its shared-memory groups into the HBM table.  Both searches keep the warp together (one probe step per
 // trip, the trip count is the warp's longest chain): the atomics that follow are issued once per warp, not once per chain
 // length.  A table that runs full raises gb_flags[0]: the host reserves
-// a bigger one and relaunches.  Algorithmic traffic: sizeof(row) read per row + the table.
+// a bigger one and relaunches.  Every reservation after a pipe's first hashes with a new seed (gb_seed): fq_gb_hash is a
+// bijection, so keys can share the low bits of their hashes, and a cluster that overflowed one table would overflow every
+// larger one under the same hash.  Algorithmic traffic: sizeof(row) read per row + the table.
 // ---------------------------------------------------------------------------------------------
 #define FQ_GB_EMPTY 0xffffffffffffffffull
 
@@ -1825,7 +1828,7 @@ template <class Q>
 __device__ __forceinline__ void fq_gb_put(const fq_launch_params &p, fq_u64 *tkeys, fq_u64 *tslots, fq_u64 *skeys, fq_u64 *sslots, fq_u32 *s_used,
                                           fq_u64 key, const fq_u64 *st, bool live, int &smem_try) {
   const fq_u32 warp = __activemask();
-  const fq_u64 h = fq_gb_hash(key);
+  const fq_u64 h = fq_gb_hash(key ^ p.gb_seed);
   const fq_u32 smask = p.gb_smem_cap - 1;
   const fq_u32 admit = p.gb_smem_cap - (p.gb_smem_cap >> FQ_GB_ADMIT_SHIFT);
   bool in_smem = false;
@@ -1932,7 +1935,7 @@ __device__ __forceinline__ void fq_groupby_kernel(const fq_launch_params &p) {
   // flush the CTA's groups into the table in HBM
   for (fq_u32 i = threadIdx.x; i < p.gb_smem_cap; i += blockDim.x) {
     const fq_u64 key = skeys[i];
-    const fq_i64 slot = fq_gb_find(p, tkeys, key, fq_gb_hash(key), key != FQ_GB_EMPTY);
+    const fq_i64 slot = fq_gb_find(p, tkeys, key, fq_gb_hash(key ^ p.gb_seed), key != FQ_GB_EMPTY);
     if (slot >= 0) Q::gb_merge(tslots + (fq_u64)slot * Q::G, sslots + (size_t)i * Q::G);
   }
   if (err) atomicOr((fq_u32 *)(p.result + 1), err);
@@ -1950,7 +1953,7 @@ __device__ __forceinline__ void fq_groupby_merge_kernel(const fq_launch_params &
     for (fq_u64 e = tid; e < p.n_rows; e += nthreads) {
       const fq_u64 *ent = p.gb_entries + e * (1 + Q::G);
       const fq_u64 key = ent[0];
-      const fq_i64 slot = fq_gb_find(p, p.gb_keys, key, fq_gb_hash(key), true);
+      const fq_i64 slot = fq_gb_find(p, p.gb_keys, key, fq_gb_hash(key ^ p.gb_seed), true);
       if (slot >= 0) Q::gb_merge(p.gb_slots + (fq_u64)slot * Q::G, ent + 1);
     }
     return;
@@ -1960,7 +1963,7 @@ __device__ __forceinline__ void fq_groupby_merge_kernel(const fq_launch_params &
     const fq_u64 key = special ? FQ_GB_EMPTY : p.gb_rep_keys[e];
     fq_u64 *from = p.gb_rep_slots + e * Q::G;
     const bool occupied = special ? from[0] != 0 : key != FQ_GB_EMPTY;   // from[0] = the group's row count
-    const fq_i64 slot = fq_gb_find(p, p.gb_keys, key, fq_gb_hash(key), occupied);
+    const fq_i64 slot = fq_gb_find(p, p.gb_keys, key, fq_gb_hash(key ^ p.gb_seed), occupied);
     if (slot >= 0) Q::gb_merge(p.gb_slots + (fq_u64)slot * Q::G, from);
     if (occupied) {
       if (!special) p.gb_rep_keys[e] = FQ_GB_EMPTY;

@@ -316,7 +316,10 @@ fq_status fq_pipe_state_device(fq_ctx *ctx, const fq_pipe *pipe, void **dev_ptr,
  * plus one bit per nullable key: at most 64 bits in all) and one 8-byte state per Aggregator leaf per group, updated with
  * atomics; every CTA pre-aggregates in a shared-memory table first, so low-cardinality keys never leave the SM.
  * fq_pipe_groupby_reserve sizes (and clears) the table; a launch that meets more groups than reserved makes
- * fq_pipe_fetch_groupby return FQ_ERR_CAPACITY (reserve more, relaunch).  FQ_RUN_ACCUMULATE keeps the table between launches.
+ * fq_pipe_fetch_groupby return FQ_ERR_CAPACITY (reserve more, relaunch).  Every reservation after a pipe's first also hashes
+ * the keys with a new seed, so keys whose hashes clustered in one table (a probe chain too long: FQ_ERR_CAPACITY with room
+ * to spare) are spread in the next.  No scan needs room for more groups than the rows it reads: an overflow at that size
+ * is worth one more reservation of the same size, not a larger one.  FQ_RUN_ACCUMULATE keeps the table between launches.
  * fq_pipe_export_groups writes the groups, in table order, to dense columns: key_cols[j] (+ key_valid[j] for nullable
  * keys, one byte per row) and one column per Aggregator leaf in fq_pipe_aggregator_nodes order (+ leaf_valid[k] for
  * leaves fq_pipe_leaf_nullable reports) — the caller evaluates arithmetic over aggregates (sum(x) / count(x)) as an
