@@ -9,6 +9,7 @@
 
 #include <cctype>
 #include <cinttypes>
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
@@ -214,8 +215,18 @@ struct Gen {
       case FQ_U8: case FQ_U16: case FQ_U32:
         return fmt("((%s)(%" PRIu64 "u))", ctype(t), v.u);
       case FQ_U64: return fmt("((fq_u64)(%" PRIu64 "ull))", v.u);
-      case FQ_F32: return fmt("((float)(%a))", (double)(float)v.f);
-      case FQ_F64: return fmt("((double)(%a))", v.f);
+      // %a prints ±inf and NaN as `inf` / `nan`, which are not CUDA identifiers: non-finite constants are written as
+      // their bit patterns, which also keeps the sign and the NaN payload
+      case FQ_F32: {
+        const float x = (float)v.f;
+        if (std::isfinite(x)) return fmt("((float)(%a))", (double)x);
+        uint32_t b;
+        memcpy(&b, &x, sizeof b);
+        return fmt("__int_as_float((int)0x%08" PRIx32 "u)", b);
+      }
+      case FQ_F64:
+        if (std::isfinite(v.f)) return fmt("((double)(%a))", v.f);
+        return fmt("__longlong_as_double((long long)0x%016" PRIx64 "ull)", v.u);
       default: return "0";
     }
   }
@@ -918,6 +929,12 @@ struct SexprParser {
     size_t b = i;
     if (i < t.size() && (t[i] == '(' || t[i] == ')')) { i++; return t.substr(b, 1); }
     while (i < t.size() && !isspace((unsigned char)t[i]) && t[i] != '(' && t[i] != ')') i++;
+    // a NaN with a payload is written as strtod reads it, `nan(0x...)`: the parenthesis belongs to the token
+    const std::string w = t.substr(b, i - b);
+    if (i < t.size() && t[i] == '(' && (w == "nan" || w == "-nan" || w == "+nan")) {
+      const size_t close = t.find(')', i);
+      if (close != std::string::npos) i = close + 1;
+    }
     return t.substr(b, i - b);
   }
   int push(fq_expr_node n) { nodes->push_back(n); return (int)nodes->size() - 1; }
