@@ -711,7 +711,8 @@ class Pipe:
         self.ctx.check(lib().fq_pipe_set_group(self.ctx._h, self._h, group._h if group is not None else None))
 
     def set_variant(self, variant: str) -> None:
-        """Kernel variant for the next launches: "tma" | "u4" | "u8" (aggregate), "tma" | "ldg" (select / projection)."""
+        """Kernel variant for the next launches: "tma" | "u4" (aggregate), "tma" | "sparse" | "dense" | "ldg" (filter +
+        projection), "tma" | "ldg" (projection); GROUP BY pipes have none."""
         self.ctx.check(lib().fq_pipe_set_variant(self.ctx._h, self._h, variant.encode()))
 
     def expr_nullable(self, i: int) -> bool:

@@ -877,7 +877,6 @@ int generate(const fq_pipe_desc &d, Generated *out, std::string *err) {
     wrappers.push_back({"_agg_u4", "extern \"C\" __global__ void __launch_bounds__(FQ_AGG_THREADS, FQ_AGG_MIN_BLOCKS) fqk_@_agg_u4(const __grid_constant__ fq_launch_params p) { fq_agg_kernel<Q_@, 4>(p); }\n"});
     if (out->tma_ok)
       wrappers.push_back({"_agg_tma", "extern \"C\" __global__ void __launch_bounds__(FQ_TMA_THREADS + 32, FQ_TMA_MIN_BLOCKS) fqk_@_agg_tma(const __grid_constant__ fq_launch_params p) { fq_agg_tma_kernel<Q_@, FQ_TMA_UNROLL, FQ_TMA_STAGES>(p); }\n"});
-    wrappers.push_back({"_agg_u8", "extern \"C\" __global__ void __launch_bounds__(FQ_AGG_THREADS, FQ_AGG_MIN_BLOCKS_U8) fqk_@_agg_u8(const __grid_constant__ fq_launch_params p) { fq_agg_kernel<Q_@, 8>(p); }\n"});
   } else if (out->has_pred) {
     wrappers.push_back({"_select", "extern \"C\" __global__ void __launch_bounds__(FQ_SEL_THREADS + 32, FQ_SEL_MIN_BLOCKS) fqk_@_select(const __grid_constant__ fq_launch_params p) { fq_select_kernel<Q_@, fq_sel_shape<Q_@::V>::U, fq_sel_shape<Q_@::V>::SEG>(p); }\n"});
     if (out->sel_tma_ok) {

@@ -29,16 +29,6 @@
 #include "kernels/fq_utf8.cuh"
 #include "generated/skeleton_embed.h"  // static const char fq_skeleton_src[]
 
-#ifndef FQ_MAP_DEFAULT_VARIANT
-#define FQ_MAP_DEFAULT_VARIANT "tma"
-#endif
-#ifndef FQ_SEL_DEFAULT_VARIANT
-#define FQ_SEL_DEFAULT_VARIANT "tma"   // "tma": pass 1 of the select kernel staged by bulk copies
-#endif
-#ifndef FQ_AGG_DEFAULT_VARIANT
-#define FQ_AGG_DEFAULT_VARIANT "tma"   // bulk-copy staged kernel when every referenced column is materialised, else u4
-#endif
-
 // ---------------------------------------------------------------------------------------------
 // precompiled kernels (generated/aot_kernels.cu)
 // ---------------------------------------------------------------------------------------------
@@ -138,7 +128,7 @@ std::mutex g_mu;
 // Launch shapes.  Defaults are the macros the precompiled kernels were built with; FQ_TUNE_* environment
 // overrides (kernel tuning experiments only) force the NVRTC path so kernel and host agree.
 struct Shapes {
-  int agg_threads = FQ_AGG_THREADS, agg_min_blocks = FQ_AGG_MIN_BLOCKS, agg_min_blocks_u8 = FQ_AGG_MIN_BLOCKS_U8;
+  int agg_threads = FQ_AGG_THREADS, agg_min_blocks = FQ_AGG_MIN_BLOCKS;
   int tma_threads = FQ_TMA_THREADS, tma_unroll = FQ_TMA_UNROLL, tma_stages = FQ_TMA_STAGES, tma_min_blocks = FQ_TMA_MIN_BLOCKS;
   int tma_stages_env = 0;   // FQ_TUNE_TMA_STAGES: ring depth override (<= FQ_TMA_STAGES)
   int sel_threads = FQ_SEL_THREADS, sel_min_blocks = FQ_SEL_MIN_BLOCKS, sel_unroll = FQ_SEL_UNROLL, sel_seg = FQ_SEL_SEG, sel_look = FQ_SEL_LOOK;
@@ -153,7 +143,6 @@ struct Shapes {
       if (e && atoi(e) > 0) { *v = atoi(e); tuned = true; }
     };
     env("FQ_TUNE_AGG_THREADS", &agg_threads); env("FQ_TUNE_AGG_MIN_BLOCKS", &agg_min_blocks);
-    env("FQ_TUNE_AGG_MIN_BLOCKS_U8", &agg_min_blocks_u8);
     env("FQ_TUNE_TMA_THREADS", &tma_threads); env("FQ_TUNE_TMA_UNROLL", &tma_unroll);
     if (getenv("FQ_TUNE_TMA_STAGES") && atoi(getenv("FQ_TUNE_TMA_STAGES")) > 0) tma_stages_env = atoi(getenv("FQ_TUNE_TMA_STAGES"));
     env("FQ_TUNE_TMA_MIN_BLOCKS", &tma_min_blocks);
@@ -169,10 +158,10 @@ struct Shapes {
     snprintf(b, sizeof b,
              "#define FQ_SELD_THREADS %d\n#define FQ_SELD_UNROLL %d\n#define FQ_SELD_SEG %d\n#define FQ_SELD_PROBE_ROWS 512\n"
              "#define FQ_SELT_THREADS %d\n#define FQ_SELT_UNROLL %d\n#define FQ_SELT_SEG %d\n#define FQ_SELT_STAGES 8\n#define FQ_SELT_LAG %d\n"
-             "#define FQ_AGG_THREADS %d\n#define FQ_AGG_MIN_BLOCKS %d\n#define FQ_AGG_MIN_BLOCKS_U8 %d\n#define FQ_TMA_THREADS %d\n"
+             "#define FQ_AGG_THREADS %d\n#define FQ_AGG_MIN_BLOCKS %d\n#define FQ_TMA_THREADS %d\n"
              "#define FQ_TMA_UNROLL %d\n#define FQ_TMA_STAGES %d\n#define FQ_TMA_MIN_BLOCKS %d\n#define FQ_SEL_THREADS %d\n"
              "#define FQ_SEL_MIN_BLOCKS %d\n#define FQ_SEL_UNROLL %d\n#define FQ_SEL_SEG %d\n#define FQ_SEL_LOOK %d\n#define FQ_MAP_THREADS %d\n#define FQ_MAP_MIN_BLOCKS %d\n#define FQ_MAP_UNROLL %d\n",
-             seld_threads, seld_unroll, seld_seg, selt_threads, selt_unroll, selt_seg, selt_lag, agg_threads, agg_min_blocks, agg_min_blocks_u8, tma_threads, tma_unroll, tma_stages, tma_min_blocks, sel_threads, sel_min_blocks, sel_unroll, sel_seg, sel_look, map_threads, map_min_blocks, map_unroll);
+             seld_threads, seld_unroll, seld_seg, selt_threads, selt_unroll, selt_seg, selt_lag, agg_threads, agg_min_blocks, tma_threads, tma_unroll, tma_stages, tma_min_blocks, sel_threads, sel_min_blocks, sel_unroll, sel_seg, sel_look, map_threads, map_min_blocks, map_unroll);
     std::string out = b;
     // FQ_TUNE_EXTRA: raw preprocessor text for A/B experiments, ';' separates lines ("#define FQ_STORE_CS 0;#define FQ_L2_HINTS 0")
     if (const char *x = getenv("FQ_TUNE_EXTRA")) {
@@ -188,18 +177,115 @@ const Shapes &shapes() {
   return s;
 }
 
+// The kernels a pipe can launch, one slot per wrapper fq::generate emits
+enum Slot { K_AGG_U4, K_AGG_TMA, K_SELECT, K_SELECT_TMA, K_SELECT_DENSE, K_SELECT_PROBE, K_MAP, K_MAP_TMA, K_GROUPBY, K_GBMERGE, K_SLOTS };
+
 struct Kernel {
+  // planned by plan_kernels
+  const char *suffix = nullptr;   // of the wrapper fqk_<tag><suffix>; null when the pipe cannot launch this slot
+  bool staged = false;            // on the bulk-copy staged path (the density probe goes with the dense build)
+  bool one_per_sm = false;        // at most one CTA per SM whatever the occupancy
+  int threads = 256;
+  unsigned smem = 0;              // dynamic shared memory per CTA
+  unsigned stages = 0;            // ring depth (fq_launch_params::stages)
+  uint64_t rows = 0;              // source rows one CTA claims at a time (chunk or segment): the unit of a persistent grid
+  // filled in by resolve_kernel
   const void *aot = nullptr;   // host stub of a precompiled kernel (cudaLaunchKernel)
   CUfunction_ jit = nullptr;   // NVRTC-built (cuLaunchKernel)
-  int threads = 256;
   int blocks_per_sm = 1;
-  unsigned smem = 0;           // dynamic shared memory per CTA
   bool valid() const { return aot || jit; }
 };
 
+// Every kernel the pipe can launch with its launch shape: the wrappers fq::generate emits for the pipe's kind, less a staged
+// one whose ring does not fit 200 KB.  Also the CTA's shared-memory table size of a GROUP BY pipe.
+void plan_kernels(const fq::Generated &gen, Kernel *k, unsigned *gb_smem_cap) {
+  const Shapes &s = shapes();
+  const int V = gen.vec;
+  auto unroll = [&](int u) { return u * V <= 32 ? u : 32 / V; };   // fq_sel{,t,d}_shape<V>::U
+  auto seg_rows = [&](int threads, int cfg_u, int cfg_seg) {        // threads x U x V x fq_sel{,t,d}_shape<V>::SEG
+    const int u = unroll(cfg_u);
+    return (uint64_t)threads * u * V * (cfg_seg * u * V <= 64 ? cfg_seg : 64 / (u * V));
+  };
+  auto plan = [&](Slot slot, const char *suffix, int threads, uint64_t rows) {
+    k[slot].suffix = suffix;
+    k[slot].threads = threads;
+    k[slot].rows = rows;
+    return &k[slot];
+  };
+  // a staged kernel: a ring of tiles of `trows` rows, `row_bytes` per row plus `bitmaps` validity bitmaps; as many tiles as
+  // fit `budget` (or the FQ_TUNE_* depth `env`), within [lo, hi]
+  auto staged = [&](Slot slot, const char *suffix, int threads, uint64_t rows, unsigned trows, int row_bytes, int bitmaps, int env,
+                    unsigned budget, unsigned lo, unsigned hi) {
+    const unsigned tile = trows * row_bytes + bitmaps * (trows / 8);
+    const unsigned stages = std::min(std::max(env > 0 ? (unsigned)env : budget / tile, lo), hi);
+    if (stages * tile > 200u * 1024u) return false;
+    Kernel *e = plan(slot, suffix, threads, rows);
+    e->staged = true;
+    e->stages = stages;
+    e->smem = stages * tile;
+    return true;
+  };
+  const unsigned tma_rows = (unsigned)s.tma_threads * s.tma_unroll * V;
+  if (gen.kind == FQ_PIPE_GROUPBY) {
+    // shared-memory table of the CTA: the largest power of two of (key + state) slots within 96 KB (two CTAs per SM)
+    const unsigned entry = 8u * (2u + (unsigned)gen.n_slots);
+    unsigned cap = 1;
+    while (cap * 2 * entry <= 96u * 1024u) cap *= 2;
+    static const int smem_env = getenv("FQ_GB_SMEM_SLOTS") ? atoi(getenv("FQ_GB_SMEM_SLOTS")) : -1;
+    if (smem_env >= 0) { cap = 1; while ((int)cap * 2 <= smem_env) cap *= 2; if (smem_env == 0) cap = 0; }
+    *gb_smem_cap = cap;
+    plan(K_GROUPBY, "_groupby", FQ_GB_THREADS, (uint64_t)FQ_GB_THREADS * FQ_GB_UNROLL * V)->smem = cap * entry;
+    plan(K_GBMERGE, "_gbmerge", 256, 0);
+  } else if (gen.kind == FQ_PIPE_AGGREGATE) {
+    plan(K_AGG_U4, "_agg_u4", s.agg_threads, (uint64_t)s.agg_threads * 4 * V);
+    // producer warp + consumers; ring of ~128 KB per CTA (measured optimum on B200)
+    if (gen.tma_ok)
+      staged(K_AGG_TMA, "_agg_tma", s.tma_threads + 32, tma_rows, tma_rows, gen.row_bytes, gen.row_bitmaps, s.tma_stages_env, 128u * 1024u, 2,
+             FQ_TMA_STAGES);
+  } else if (gen.has_pred) {
+    plan(K_SELECT, "_select", s.sel_threads + 32, seg_rows(s.sel_threads, s.sel_unroll, s.sel_seg));   // worker warps + one scan warp
+    // sparse-tuned build: consumer warps + scan warp + producer warp; pass 1 stages the predicate's columns.  ~192 KB in
+    // flight per SM measured best here (1.19 -> 1.14 ms at 1e9 rows; the aggregate kernel peaks at 128 KB)
+    // dense-tuned build: both passes staged, so a slot holds a tile of EVERY referenced column; small tiles, a ring of
+    // ~112 KB, and one CTA per SM (the look-back window covers a grid of one CTA per SM)
+    if (gen.sel_tma_ok &&
+        staged(K_SELECT_TMA, "_select_tma", s.selt_threads + 64, seg_rows(s.selt_threads, s.selt_unroll, s.selt_seg),
+               (unsigned)s.selt_threads * unroll(s.selt_unroll) * V, gen.pred_row_bytes, gen.pred_row_bitmaps, s.selt_stages_env, 192u * 1024u, 2,
+               FQ_SELT_STAGES) &&
+        staged(K_SELECT_DENSE, "_select_dense", s.seld_threads + 64, seg_rows(s.seld_threads, s.seld_unroll, s.seld_seg),
+               (unsigned)s.seld_threads * unroll(s.seld_unroll) * V, gen.row_bytes, gen.row_bitmaps, s.seld_stages, 0, 3, 16)) {
+      k[K_SELECT_DENSE].one_per_sm = true;
+      plan(K_SELECT_PROBE, "_select_probe", 128, 0)->staged = true;
+    }
+  } else {
+    plan(K_MAP, "_map", s.map_threads, (uint64_t)s.map_threads * s.map_unroll * V);
+    if (gen.tma_ok)
+      staged(K_MAP_TMA, "_map_tma", s.tma_threads + 32, tma_rows, tma_rows, gen.row_bytes, gen.row_bitmaps, s.tma_stages_env, 128u * 1024u, 2,
+             FQ_TMA_STAGES);
+  }
+}
+
+// Kernel variant a pipe's launches prefer.  tma: the staged kernel (a selection: the sparse-tuned build, and the dense-tuned
+// one when the density probe says so); sparse / dense: that staged select build alone; ldg: the LDG kernel.
+enum Variant { V_TMA, V_SPARSE, V_DENSE, V_LDG };
+// the words each kind of pipe accepts, by the variable that sets its default; a GROUP BY pipe has no variant
+const struct { const char *env, *word; Variant v; } kVariants[] = {
+    {"FQ_AGG_VARIANT", "tma", V_TMA},    {"FQ_AGG_VARIANT", "u4", V_LDG},       {"FQ_SEL_VARIANT", "tma", V_TMA},
+    {"FQ_SEL_VARIANT", "sparse", V_SPARSE}, {"FQ_SEL_VARIANT", "dense", V_DENSE}, {"FQ_SEL_VARIANT", "ldg", V_LDG},
+    {"FQ_MAP_VARIANT", "tma", V_TMA},    {"FQ_MAP_VARIANT", "ldg", V_LDG}};
+const char *variant_env(const fq::Generated &gen) {
+  return gen.kind == FQ_PIPE_GROUPBY ? nullptr : gen.kind == FQ_PIPE_AGGREGATE ? "FQ_AGG_VARIANT" : gen.has_pred ? "FQ_SEL_VARIANT" : "FQ_MAP_VARIANT";
+}
+fq_status parse_variant(const fq::Generated &gen, const char *word, Variant *out) {
+  const char *env = variant_env(gen);
+  for (const auto &w : kVariants)
+    if (env && strcmp(w.env, env) == 0 && strcmp(w.word, word) == 0) { *out = w.v; return FQ_OK; }
+  return set_err(FQ_ERR_INVALID, "Internal Error: unknown kernel variant %s", word);
+}
+
 struct Module {  // one compiled specialisation, shared by every pipe with the same tag
   std::map<std::string, Kernel> kernels;
-  std::vector<std::string> built;   // JIT: suffixes of the kernel variants in the module
+  std::vector<std::string> built;   // JIT: suffixes of the kernels in the module
   bool from_disk_cache = false;     // JIT: the cubin came from the on-disk cache instead of NVRTC
   bool precompiled = false;
   CUmodule_ mod = nullptr;
@@ -260,8 +346,7 @@ struct fq_group {
 
 struct fq_pipe {
   fq::Generated gen;
-  Kernel k_agg_u4, k_agg_u8, k_agg_tma, k_select, k_select_tma, k_select_dense, k_select_probe, k_map, k_map_tma, k_groupby, k_gbmerge;
-  unsigned seld_stages = 0;
+  Kernel k[K_SLOTS];   // plan_kernels, resolved by fq_pipe_compile
   // GROUP BY: the hash table in HBM
   uint64_t *gb_keys = nullptr, *gb_slots = nullptr;
   uint64_t *gb_rep_keys = nullptr, *gb_rep_slots = nullptr;   // gb_reps - 1 more tables of gb_cap + 1 slots (see fq_groupby_kernel)
@@ -275,11 +360,9 @@ struct fq_pipe {
   uint64_t *gb_identity = nullptr;   // device copy of a fresh group's state
   unsigned gb_smem_cap = 0;
   bool launched_groupby = false;
-  unsigned mapt_stages = 0;
-  unsigned tma_stages = 0, selt_stages = 0;
 
   int build_kind = 0;   // 0 precompiled, 1 NVRTC in this process, 2 on-disk JIT cache
-  std::string variant;  // kernel variant the launches prefer: FQ_{AGG,SEL,MAP}_VARIANT when the pipe was compiled, or fq_pipe_set_variant
+  Variant variant = V_TMA;   // FQ_{AGG,SEL,MAP}_VARIANT when the pipe was compiled, or fq_pipe_set_variant
   fq_group *group = nullptr;   // aggregate launches end with the in-kernel cross-GPU merge when set
   uint64_t *d_merged = nullptr, *h_merged = nullptr;
   bool launched_merged = false;
@@ -395,13 +478,13 @@ static void jit_cache_write(const std::string &path, const std::vector<char> &da
 
 static const char *const kNvrtcOpts[] = {"--gpu-architecture=sm_100a", "-std=c++17", "-lineinfo"};
 
-// `suffixes`: the kernel variants to build (empty = all of them)
-fq_status compile_jit(fq_ctx *ctx, const fq::Generated &gen, Module *m, const std::vector<std::string> &suffixes) {
+// builds the kernels whose suffixes m->built lists
+fq_status compile_jit(fq_ctx *ctx, const fq::Generated &gen, Module *m) {
   if (!g_nvrtc.load()) return set_err(FQ_ERR_CUDA, "NVRTC unavailable: %s", g_nvrtc.why.c_str());
   if (!g_drv.load()) return set_err(FQ_ERR_CUDA, "CUDA driver unavailable: %s", g_drv.why.c_str());
   std::string src = shapes().defines() + std::string(fq_skeleton_src) + "\n" + gen.struct_source;
   for (auto &k : gen.kernels)
-    if (suffixes.empty() || std::find(suffixes.begin(), suffixes.end(), k.first) != suffixes.end()) src += k.second;
+    if (std::find(m->built.begin(), m->built.end(), k.first) != m->built.end()) src += k.second;
   const std::string cache_dir = jit_cache_dir();
   // key = program text + everything else the cubin depends on: NVRTC's version and the compile options
   int nv_major = 0, nv_minor = 0;
@@ -442,34 +525,33 @@ fq_status compile_jit(fq_ctx *ctx, const fq::Generated &gen, Module *m, const st
   return FQ_OK;
 }
 
-// A JIT module holds only the variants it was built with: a missing one leaves `out` invalid (the launch falls back).
-fq_status resolve_kernel(Module *m, const std::string &name, int threads, Kernel *out, unsigned smem = 0) {
+// Finds a planned kernel in the pipe's module.  A JIT module holds only the kernels it was built with: a missing one stays
+// invalid (the launch falls back).
+fq_status resolve_kernel(Module *m, const std::string &tag, Kernel *k) {
+  const std::string name = "fqk_" + tag + k->suffix;
   auto it = m->kernels.find(name);
-  if (it != m->kernels.end()) { *out = it->second; return FQ_OK; }
-  if (!m->precompiled && std::find(m->built.begin(), m->built.end(), name.substr(name.find('_', 4))) == m->built.end()) return FQ_OK;
-  Kernel k;
-  k.threads = threads;
-  k.smem = smem;
+  if (it != m->kernels.end()) { *k = it->second; return FQ_OK; }
+  if (!m->precompiled && std::find(m->built.begin(), m->built.end(), k->suffix) == m->built.end()) return FQ_OK;
+  const unsigned smem = k->smem;
   if (m->precompiled) {
     for (int i = 0; i < fq_aot_count; i++)
-      if (name == fq_aot_table[i].name) k.aot = fq_aot_table[i].fn;
-    if (!k.aot) return set_err(FQ_ERR_INTERNAL, "Internal Error: precompiled kernel %s missing", name.c_str());
-    if (smem > 48 * 1024) CUDA_TRY(cudaFuncSetAttribute(k.aot, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&k.blocks_per_sm, k.aot, threads, smem));
+      if (name == fq_aot_table[i].name) k->aot = fq_aot_table[i].fn;
+    if (!k->aot) return set_err(FQ_ERR_INTERNAL, "Internal Error: precompiled kernel %s missing", name.c_str());
+    if (smem > 48 * 1024) CUDA_TRY(cudaFuncSetAttribute(k->aot, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&k->blocks_per_sm, k->aot, k->threads, smem));
   } else {
-    CUresult_ cr = g_drv.cuModuleGetFunction(&k.jit, m->mod, name.c_str());
+    CUresult_ cr = g_drv.cuModuleGetFunction(&k->jit, m->mod, name.c_str());
     if (cr) return set_err(FQ_ERR_CUDA, "cuModuleGetFunction(%s): %s", name.c_str(), g_drv.err(cr).c_str());
     if (smem > 48 * 1024) {
       if (!g_drv.cuFuncSetAttribute) return set_err(FQ_ERR_CUDA, "cuFuncSetAttribute unavailable");
-      cr = g_drv.cuFuncSetAttribute(k.jit, 8 /* CU_FUNC_ATTRIBUTE_MAX_DYNAMIC_SHARED_SIZE_BYTES */, (int)smem);
+      cr = g_drv.cuFuncSetAttribute(k->jit, 8 /* CU_FUNC_ATTRIBUTE_MAX_DYNAMIC_SHARED_SIZE_BYTES */, (int)smem);
       if (cr) return set_err(FQ_ERR_CUDA, "cuFuncSetAttribute(%s): %s", name.c_str(), g_drv.err(cr).c_str());
     }
-    cr = g_drv.cuOccupancyMaxActiveBlocksPerMultiprocessor(&k.blocks_per_sm, k.jit, threads, smem);
+    cr = g_drv.cuOccupancyMaxActiveBlocksPerMultiprocessor(&k->blocks_per_sm, k->jit, k->threads, smem);
     if (cr) return set_err(FQ_ERR_CUDA, "cuOccupancy: %s", g_drv.err(cr).c_str());
   }
-  if (k.blocks_per_sm < 1) k.blocks_per_sm = 1;
-  m->kernels[name] = k;
-  *out = k;
+  if (k->blocks_per_sm < 1 || k->one_per_sm) k->blocks_per_sm = 1;
+  m->kernels[name] = *k;
   return FQ_OK;
 }
 
@@ -483,6 +565,22 @@ fq_status launch(fq_ctx *ctx, const Kernel &k, unsigned grid, const fq_launch_pa
   }
   ctx->launches++;
   return FQ_OK;
+}
+
+// Aggregate, select and map launches: the staged kernel when the variant allows it and the source's validity bitmaps can be
+// bulk-copied, else the LDG kernel; a module that holds only one of the two (a JIT build) launches that one.
+fq_status pick_kernel(const fq_pipe *pipe, Slot staged, Slot ldg, const fq_launch_params &p, const char *what, const Kernel **out) {
+  const Kernel &ks = pipe->k[staged], &kl = pipe->k[ldg];
+  if (p.bits_unstaged && !kl.valid())
+    return set_err(FQ_ERR_INTERNAL, "Internal Error: validity bitmap off the 128-row grid needs the LDG kernel, which this pipe was not built with");
+  *out = !p.bits_unstaged && ((pipe->variant != V_LDG && ks.valid()) || !kl.valid()) ? &ks : &kl;
+  if (!(*out)->valid()) return set_err(FQ_ERR_INTERNAL, "Internal Error: no %s kernel was built for this pipe", what);
+  return FQ_OK;
+}
+
+// persistent grid: every resident CTA slot of every SM, fewer when the source has fewer units of k.rows rows
+unsigned persistent_grid(const fq_ctx *ctx, const Kernel &k, uint64_t n_rows) {
+  return (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)ctx->sm_count * k.blocks_per_sm, (n_rows + k.rows - 1) / k.rows));
 }
 
 // "the results of this launch are ready" for the fetch calls: an event on the stream, or — while a graph is being recorded
@@ -827,7 +925,12 @@ fq_status fq_pipe_compile(fq_ctx *ctx, const fq_pipe_desc *desc, fq_pipe **out) 
     return set_err(st, "%s", err.c_str());
   }
   const fq::Generated &gen = pipe->gen;
-  Module *m;
+  plan_kernels(gen, pipe->k, &pipe->gb_smem_cap);
+  // the environment is read here, once per pipe — never on the launch path
+  const char *env = variant_env(gen);
+  if (const char *word = env ? getenv(env) : nullptr) {
+    if (fq_status s2 = parse_variant(gen, word, &pipe->variant)) { delete pipe; return s2; }
+  }
   {
     std::lock_guard<std::mutex> lk(ctx->mu);
     auto it = ctx->modules.find(gen.tag);
@@ -838,120 +941,34 @@ fq_status fq_pipe_compile(fq_ctx *ctx, const fq_pipe_desc *desc, fq_pipe **out) 
         if (strncmp(fq_aot_table[i].name, probe.c_str(), probe.size()) == 0) mod.precompiled = true;
       if (getenv("FQ_FORCE_JIT") || shapes().tuned) mod.precompiled = false;
       if (!mod.precompiled) {
-        // NVRTC + ptxas cost about a second per kernel: build only the variant this pipe will launch (the staged one when
-        // its ring fits, else the LDG one; both handle ragged and unaligned sources).  FQ_JIT_ALL_VARIANTS=1 builds all.
-        std::vector<std::string> want;
-        if (!(getenv("FQ_JIT_ALL_VARIANTS") && atoi(getenv("FQ_JIT_ALL_VARIANTS")) != 0)) {
-          const bool agg = gen.kind == FQ_PIPE_AGGREGATE;
-          const int u = agg || !gen.has_pred ? shapes().tma_unroll : (shapes().selt_unroll * gen.vec <= 32 ? shapes().selt_unroll : 32 / gen.vec);
-          const unsigned trows = (unsigned)(agg || !gen.has_pred ? shapes().tma_threads : shapes().selt_threads) * u * gen.vec;
-          const unsigned tile_bytes = agg || !gen.has_pred ? trows * gen.row_bytes + gen.row_bitmaps * (trows / 8)
-                                                           : trows * gen.pred_row_bytes + gen.pred_row_bitmaps * (trows / 8);
-          const bool staged = (agg || !gen.has_pred ? gen.tma_ok : gen.sel_tma_ok) && 2u * tile_bytes <= 200u * 1024u;
-          const std::string variant_env = getenv(agg ? "FQ_AGG_VARIANT" : gen.has_pred ? "FQ_SEL_VARIANT" : "FQ_MAP_VARIANT")
-                                              ? getenv(agg ? "FQ_AGG_VARIANT" : gen.has_pred ? "FQ_SEL_VARIANT" : "FQ_MAP_VARIANT") : "tma";
-          // a validity bitmap that starts off the 128-row grid (a slice) cannot be bulk-copied: such pipes also get the LDG kernel
-          if (gen.row_bitmaps > 0 && gen.kind != FQ_PIPE_GROUPBY) want.push_back(agg ? "_agg_u4" : gen.has_pred ? "_select" : "_map");
-          if (gen.kind == FQ_PIPE_GROUPBY) { want.push_back("_groupby"); want.push_back("_gbmerge"); }
-          else if (agg) want.push_back(staged && variant_env == "tma" ? "_agg_tma" : variant_env == "u8" ? "_agg_u8" : "_agg_u4");
-          else if (gen.has_pred) {
-            if (staged && variant_env != "ldg") { want.push_back("_select_tma"); want.push_back("_select_dense"); want.push_back("_select_probe"); }
-            else want.push_back("_select");
-          }
-          else want.push_back(staged && variant_env == "tma" ? "_map_tma" : "_map");
-        }
+        // NVRTC + ptxas cost about a second per kernel: build only the path this pipe will launch (the staged one when the
+        // variant allows it and its ring fits, else the LDG one; both handle ragged and unaligned sources).  A validity bitmap
+        // that starts off the 128-row grid (a slice) cannot be bulk-copied: such pipes also get the LDG kernel.
+        // FQ_JIT_ALL_VARIANTS=1 builds every planned kernel.
+        const bool all = getenv("FQ_JIT_ALL_VARIANTS") && atoi(getenv("FQ_JIT_ALL_VARIANTS")) != 0;
+        bool staged = false;
+        for (const Kernel &k : pipe->k) staged |= k.staged && pipe->variant != V_LDG;
+        for (const Kernel &k : pipe->k)
+          if (k.suffix && (all || k.staged == staged || (!k.staged && gen.row_bitmaps > 0))) mod.built.push_back(k.suffix);
         std::lock_guard<std::mutex> lk2(g_mu);
-        if (fq_status s2 = compile_jit(ctx, gen, &mod, want)) { delete pipe; return s2; }
-        for (auto &k : gen.kernels)
-          if (want.empty() || std::find(want.begin(), want.end(), k.first) != want.end()) mod.built.push_back(k.first);
+        if (fq_status s2 = compile_jit(ctx, gen, &mod)) { delete pipe; return s2; }
       }
       it = ctx->modules.emplace(gen.tag, mod).first;
     }
-    m = &it->second;
+    Module *m = &it->second;
     pipe->precompiled = m->precompiled;
     pipe->build_kind = m->precompiled ? 0 : m->from_disk_cache ? 2 : 1;
-    fq_status s2 = FQ_OK;
-    const std::string base = "fqk_" + gen.tag;
-    if (gen.kind == FQ_PIPE_GROUPBY) {
-      // shared-memory table of the CTA: the largest power of two of (key + state) slots within 96 KB (two CTAs per SM)
-      const unsigned entry = 8u * (2u + (unsigned)gen.n_slots);
-      unsigned cap = 1;
-      while (cap * 2 * entry <= 96u * 1024u) cap *= 2;
-      static const int smem_env = getenv("FQ_GB_SMEM_SLOTS") ? atoi(getenv("FQ_GB_SMEM_SLOTS")) : -1;
-      if (smem_env >= 0) { cap = 1; while ((int)cap * 2 <= smem_env) cap *= 2; if (smem_env == 0) cap = 0; }
-      pipe->gb_smem_cap = cap;
-      s2 = resolve_kernel(m, base + "_groupby", FQ_GB_THREADS, &pipe->k_groupby, cap * entry);
-      if (!s2) s2 = resolve_kernel(m, base + "_gbmerge", 256, &pipe->k_gbmerge);
-    } else if (gen.kind == FQ_PIPE_AGGREGATE) {
-      s2 = resolve_kernel(m, base + "_agg_u4", shapes().agg_threads, &pipe->k_agg_u4);
-      if (!s2) s2 = resolve_kernel(m, base + "_agg_u8", shapes().agg_threads, &pipe->k_agg_u8);
-      if (!s2 && gen.tma_ok) {
-        // ring depth: as many tiles as fit ~128 KB per CTA (measured optimum on B200), at least 2, at most the template bound
-        const unsigned trows = (unsigned)shapes().tma_threads * shapes().tma_unroll * gen.vec;
-        const unsigned tile_bytes = trows * gen.row_bytes + gen.row_bitmaps * (trows / 8);
-        unsigned stages = shapes().tma_stages_env > 0 ? (unsigned)shapes().tma_stages_env : (128u * 1024u) / tile_bytes;
-        stages = std::min<unsigned>(std::max<unsigned>(stages, 2), FQ_TMA_STAGES);
-        if (stages * tile_bytes <= 200 * 1024) {
-          s2 = resolve_kernel(m, base + "_agg_tma", shapes().tma_threads + 32, &pipe->k_agg_tma, stages * tile_bytes);
-          pipe->tma_stages = stages;
-        }
-      }
-    } else if (gen.has_pred) {
-      s2 = resolve_kernel(m, base + "_select", shapes().sel_threads + 32, &pipe->k_select);   // worker warps + one scan warp
-      if (!s2 && gen.sel_tma_ok) {
-        // staged variant: consumer warps + scan warp + producer warp; ring of ~192 KB per CTA, at least 2 tiles
-        const int u = shapes().selt_unroll * gen.vec <= 32 ? shapes().selt_unroll : 32 / gen.vec;   // fq_selt_shape<V>::U
-        const unsigned trows_s = (unsigned)shapes().selt_threads * u * gen.vec;
-        const unsigned tile_bytes = trows_s * gen.pred_row_bytes + gen.pred_row_bitmaps * (trows_s / 8);   // pass 1 stages the predicate's columns
-        // ~192 KB in flight per SM measured best here (1.19 -> 1.14 ms at 1e9 rows; the aggregate kernel peaks at 128 KB)
-        unsigned stages = shapes().selt_stages_env > 0 ? (unsigned)shapes().selt_stages_env : (192u * 1024u) / tile_bytes;
-        stages = std::min<unsigned>(std::max<unsigned>(stages, 2), FQ_SELT_STAGES);
-        if (stages * tile_bytes <= 200 * 1024) {
-          s2 = resolve_kernel(m, base + "_select_tma", shapes().selt_threads + 64, &pipe->k_select_tma, stages * tile_bytes);
-          pipe->selt_stages = stages;
-        }
-        // the dense-tuned build: both passes staged, so a slot holds a tile of EVERY referenced column; small tiles and a
-        // ring of ~112 KB (FQ_SELT_STAGE2=0 leaves it out: dense selections then re-read kept rows from L2 with plain loads)
-        const int ud = shapes().seld_unroll * gen.vec <= 32 ? shapes().seld_unroll : 32 / gen.vec;   // fq_seld_shape<V>::U
-        const unsigned trows_d = (unsigned)shapes().seld_threads * ud * gen.vec;
-        const unsigned all_bytes = trows_d * gen.row_bytes + gen.row_bitmaps * (trows_d / 8);
-        static const bool stage2_env = !(getenv("FQ_SELT_STAGE2") && atoi(getenv("FQ_SELT_STAGE2")) == 0);
-        const unsigned dstages = std::min<unsigned>(std::max<unsigned>((unsigned)shapes().seld_stages, 3), 16);
-        if (!s2 && pipe->k_select_tma.valid() && stage2_env && dstages * all_bytes <= 200u * 1024u) {
-          s2 = resolve_kernel(m, base + "_select_dense", shapes().seld_threads + 64, &pipe->k_select_dense, dstages * all_bytes);
-          if (!s2) s2 = resolve_kernel(m, base + "_select_probe", 128, &pipe->k_select_probe);
-          pipe->seld_stages = dstages;
-        }
-      }
-    } else {
-      s2 = resolve_kernel(m, base + "_map", shapes().map_threads, &pipe->k_map);
-      if (!s2 && gen.tma_ok) {
-        const unsigned trows = (unsigned)shapes().tma_threads * shapes().tma_unroll * gen.vec;
-        const unsigned tile_bytes = trows * gen.row_bytes + gen.row_bitmaps * (trows / 8);
-        unsigned stages = shapes().tma_stages_env > 0 ? (unsigned)shapes().tma_stages_env : (128u * 1024u) / tile_bytes;
-        stages = std::min<unsigned>(std::max<unsigned>(stages, 2), FQ_TMA_STAGES);
-        if (stages * tile_bytes <= 200 * 1024) {
-          s2 = resolve_kernel(m, base + "_map_tma", shapes().tma_threads + 32, &pipe->k_map_tma, stages * tile_bytes);
-          pipe->mapt_stages = stages;
-        }
-      }
+    for (Kernel &k : pipe->k) {
+      if (!k.suffix) continue;
+      if (fq_status s2 = resolve_kernel(m, gen.tag, &k)) { delete pipe; return s2; }
     }
-    if (s2) { delete pipe; return s2; }
   }
   pipe->n_slots = FQ_STATE_HDR + gen.n_slots;
-  {
-    // the environment is read here, once per pipe — never on the launch path
-    const char *name = gen.kind == FQ_PIPE_AGGREGATE ? "FQ_AGG_VARIANT" : gen.has_pred ? "FQ_SEL_VARIANT" : "FQ_MAP_VARIANT";
-    const char *dflt = gen.kind == FQ_PIPE_AGGREGATE ? FQ_AGG_DEFAULT_VARIANT : gen.has_pred ? FQ_SEL_DEFAULT_VARIANT : FQ_MAP_DEFAULT_VARIANT;
-    const char *v = getenv(name);
-    pipe->variant = v ? v : dflt;
-    if (!v && gen.kind == FQ_PIPE_AGGREGATE && getenv("FQ_AGG_UNROLL") && atoi(getenv("FQ_AGG_UNROLL")) == 8) pipe->variant = "u8";
-  }
   cudaError_t e = cudaMalloc(&pipe->d_state, sizeof(uint64_t) * pipe->n_slots);
   if (e == cudaSuccess && gen.kind == FQ_PIPE_AGGREGATE) {
     // one partial row per CTA of the largest persistent grid any variant can launch: no allocation on the launch path
     int bps = 1;
-    for (const Kernel *k : {&pipe->k_agg_u4, &pipe->k_agg_u8, &pipe->k_agg_tma})
+    for (const Kernel *k : {&pipe->k[K_AGG_U4], &pipe->k[K_AGG_TMA]})
       if (k->valid()) bps = std::max(bps, k->blocks_per_sm);
     pipe->partials_cap = ctx->sm_count * bps;
     e = cudaMalloc(&pipe->d_partials, sizeof(uint64_t) * pipe->n_slots * pipe->partials_cap);
@@ -997,12 +1014,7 @@ void fq_pipe_destroy(fq_ctx *ctx, fq_pipe *pipe) {
 
 fq_status fq_pipe_set_variant(fq_ctx *, fq_pipe *pipe, const char *variant) {
   if (!pipe || !variant) return set_err(FQ_ERR_INVALID, "Internal Error: null argument");
-  const std::string v = variant;
-  const bool ok = pipe->gen.kind == FQ_PIPE_AGGREGATE ? (v == "tma" || v == "u4" || v == "u8")
-                                                       : (v == "tma" || v == "ldg" || v == "sparse" || v == "dense");
-  if (!ok) return set_err(FQ_ERR_INVALID, "Internal Error: unknown kernel variant %s", variant);
-  pipe->variant = v;
-  return FQ_OK;
+  return parse_variant(pipe->gen, variant, &pipe->variant);
 }
 int32_t fq_pipe_is_precompiled(const fq_pipe *pipe) { return pipe && pipe->precompiled; }
 int32_t fq_pipe_build_kind(const fq_pipe *pipe) { return pipe ? pipe->build_kind : 0; }
@@ -1040,28 +1052,15 @@ fq_status fq_pipe_launch_aggregate(fq_ctx *ctx, fq_pipe *pipe, const fq_source *
   fq_launch_params p;
   memset(&p, 0, sizeof p);
   if (fq_status st = bind_source(pipe, src, &p)) return st;
-  // kernel variant: chosen when the pipe was compiled (FQ_AGG_VARIANT) or by fq_pipe_set_variant
-  const std::string &variant = pipe->variant;
-  // the preferred variant when the module holds it, else whichever it was built with
-  if (p.bits_unstaged && !pipe->k_agg_u4.valid() && !pipe->k_agg_u8.valid())
-    return set_err(FQ_ERR_INTERNAL, "Internal Error: validity bitmap off the 128-row grid needs the LDG kernel, which this pipe was not built with");
-  const bool use_tma = !p.bits_unstaged && ((variant == "tma" && pipe->k_agg_tma.valid()) || (!pipe->k_agg_u4.valid() && !pipe->k_agg_u8.valid()));
-  const bool want_u8 = (variant == "u8" && pipe->k_agg_u8.valid()) || (!use_tma && !pipe->k_agg_u4.valid());
-  const Kernel &k = use_tma ? pipe->k_agg_tma : want_u8 ? pipe->k_agg_u8 : pipe->k_agg_u4;
-  if (!k.valid()) return set_err(FQ_ERR_INTERNAL, "Internal Error: no aggregate kernel was built for this pipe");
-  const int unroll = use_tma ? shapes().tma_unroll : want_u8 ? 8 : 4;
-  // persistent grid: every resident CTA slot of every SM, fewer when the shard has fewer chunks
-  const uint64_t chunk_rows = (uint64_t)(use_tma ? k.threads - 32 : k.threads) * unroll * pipe->gen.vec;
-  const uint64_t chunks = (src->n_rows + chunk_rows - 1) / chunk_rows;
-  static const int bps_env = getenv("FQ_AGG_BLOCKS_PER_SM") ? atoi(getenv("FQ_AGG_BLOCKS_PER_SM")) : 0;
-  const int bps = bps_env > 0 ? std::min(bps_env, k.blocks_per_sm) : k.blocks_per_sm;
-  unsigned grid = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)ctx->sm_count * bps, chunks));
+  const Kernel *k;
+  if (fq_status st = pick_kernel(pipe, K_AGG_TMA, K_AGG_U4, p, "aggregate", &k)) return st;
+  const unsigned grid = persistent_grid(ctx, *k, src->n_rows);
   if ((int)grid > pipe->partials_cap) return set_err(FQ_ERR_INTERNAL, "Internal Error: grid of %u CTAs exceeds the pipe's %d partial rows", grid, pipe->partials_cap);
   p.partials = (fq_u64 *)pipe->d_partials;
   p.state = (fq_u64 *)pipe->d_state;
   p.ticket = (fq_u32 *)(pipe->d_ctl + 4);
   p.accumulate = (flags & FQ_RUN_ACCUMULATE) ? 1u : 0u;
-  p.stages = pipe->tma_stages;
+  p.stages = pipe->k[K_AGG_TMA].stages;   // the staged kernel's ring (the LDG kernel does not read it)
   if (fq_group *g = pipe->group) {
     if (ctx->recording) return set_err(FQ_ERR_INVALID, "Internal Error: a pipe with a group attached cannot be recorded into a graph (the merge epoch advances per launch)");
     if (!g->connected) return set_err(FQ_ERR_INVALID, "Internal Error: the pipe's group is not connected to its peers");
@@ -1083,7 +1082,7 @@ fq_status fq_pipe_launch_aggregate(fq_ctx *ctx, fq_pipe *pipe, const fq_source *
   // the kernel's last CTA writes state (and merged state) straight into the pinned host mirrors: nothing is queued behind it
   p.host_state = (fq_u64 *)pipe->h_state;
   p.host_merged = pipe->group ? (fq_u64 *)pipe->h_merged : nullptr;
-  if (fq_status st = launch(ctx, k, grid, p, stream)) return st;
+  if (fq_status st = launch(ctx, *k, grid, p, stream)) return st;
   pipe->launched_merged = pipe->group != nullptr;
   if (fq_status st = mark_done(ctx, pipe->ev, (cudaStream_t)stream)) return st;
   pipe->launched = true;
@@ -1487,29 +1486,16 @@ fq_status fq_pipe_launch_project(fq_ctx *ctx, fq_pipe *pipe, const fq_source *sr
   if (src->n_rows == 0) {
     pipe->skipped = true;
   } else if (pipe->gen.has_pred) {
-    // kernel variant: FQ_SEL_VARIANT = tma (default: pass 1 staged by bulk copies; needs every referenced column materialised) | ldg
-    // kernel variant: FQ_SEL_VARIANT / fq_pipe_set_variant = tma (default: staged by bulk copies; the dense-tuned build when a
-    // density probe says so) | sparse | dense (force one staged build) | ldg (worker-warp loads; generated sources)
-    const std::string &variant = pipe->variant;
-    const bool staged_ok = pipe->k_select_tma.valid();
-    if (p.bits_unstaged && !pipe->k_select.valid())
-      return set_err(FQ_ERR_INTERNAL, "Internal Error: validity bitmap off the 128-row grid needs the LDG kernel, which this pipe was not built with");
-    const bool use_tma = !p.bits_unstaged && ((variant != "ldg" && staged_ok) || !pipe->k_select.valid());
-    const int vec = pipe->gen.vec;
-    auto seg_rows = [&](int threads, int cfg_u, int cfg_seg) {
-      const int u = cfg_u * vec <= 32 ? cfg_u : 32 / vec;
-      const int seg = cfg_seg * u * vec <= 64 ? cfg_seg : 64 / (u * vec);
-      return (uint64_t)threads * u * vec * seg;
-    };
-    const uint64_t rows_sparse = use_tma ? seg_rows(shapes().selt_threads, shapes().selt_unroll, shapes().selt_seg)
-                                         : seg_rows(pipe->k_select.threads - 32, shapes().sel_unroll, shapes().sel_seg);
-    const uint64_t rows_dense = seg_rows(shapes().seld_threads, shapes().seld_unroll, shapes().seld_seg);
+    const Kernel *k;
+    if (fq_status st = pick_kernel(pipe, K_SELECT_TMA, K_SELECT, p, "select", &k)) return st;
+    const Kernel &kd = pipe->k[K_SELECT_DENSE];
     // the dense-tuned build pays off when a good part of the rows is written: outputs of at least 1/16 of a large source
-    const bool dense_ok = use_tma && pipe->k_select_dense.valid() && pipe->k_select_probe.valid() && !p.unaligned;
-    const bool force_dense = dense_ok && variant == "dense";
-    const bool probe = dense_ok && variant == "tma" && src->n_rows >= (4u << 20) && cap >= src->n_rows / 16 && p.stop_after == 0;
-    const uint64_t segs_sparse = (src->n_rows + rows_sparse - 1) / rows_sparse, segs_dense = (src->n_rows + rows_dense - 1) / rows_dense;
-    const uint64_t segs_max = (probe || force_dense) ? std::max(segs_sparse, segs_dense) : segs_sparse;
+    const bool dense_ok = k->staged && kd.valid() && pipe->k[K_SELECT_PROBE].valid() && !p.unaligned;
+    const bool force_dense = dense_ok && pipe->variant == V_DENSE;
+    const bool probe = dense_ok && pipe->variant == V_TMA && src->n_rows >= (4u << 20) && cap >= src->n_rows / 16 && p.stop_after == 0;
+    const uint64_t segs_sparse = (src->n_rows + k->rows - 1) / k->rows;
+    const uint64_t segs_dense = (probe || force_dense) ? (src->n_rows + kd.rows - 1) / kd.rows : 0;
+    const uint64_t segs_max = std::max(segs_sparse, segs_dense);
     if (segs_max > pipe->tiles_cap) {
       cudaFree(pipe->d_tiles);
       pipe->d_tiles = nullptr;
@@ -1518,32 +1504,26 @@ fq_status fq_pipe_launch_project(fq_ctx *ctx, fq_pipe *pipe, const fq_source *sr
     }
     p.tile_status = (fq_u64 *)pipe->d_tiles;
     CUDA_TRY(cudaMemsetAsync(pipe->d_tiles, 0, sizeof(uint64_t) * segs_max, (cudaStream_t)stream));
-    static const int sel_bps_env = getenv("FQ_SEL_BLOCKS_PER_SM") ? atoi(getenv("FQ_SEL_BLOCKS_PER_SM")) : 0;
     fq_u32 *probe_words = (fq_u32 *)(pipe->d_ctl + 6);   // [0] sampled, [1] kept, [2] mode, [3] CTA ticket
     if (probe) {
       fq_launch_params pp = p;
       pp.probe = probe_words;
-      if (fq_status st = launch(ctx, pipe->k_select_probe, (unsigned)ctx->sm_count, pp, stream)) return st;
+      if (fq_status st = launch(ctx, pipe->k[K_SELECT_PROBE], (unsigned)ctx->sm_count, pp, stream)) return st;
       p.sel_mode = probe_words + 2;
     }
     if (!force_dense) {   // the sparse-tuned build (or the LDG kernel)
-      const Kernel &k = use_tma ? pipe->k_select_tma : pipe->k_select;
-      if (!k.valid()) return set_err(FQ_ERR_INTERNAL, "Internal Error: no select kernel was built for this pipe");
       fq_launch_params ps = p;
-      ps.stages = pipe->selt_stages;
+      ps.stages = pipe->k[K_SELECT_TMA].stages;
       ps.stages2 = 0;
       ps.n_tiles = segs_sparse;
-      const int sel_bps = (sel_bps_env > 0 && !use_tma) ? std::min(sel_bps_env, k.blocks_per_sm) : k.blocks_per_sm;
-      const unsigned grid = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)ctx->sm_count * sel_bps, ps.n_tiles));
-      if (fq_status st = launch(ctx, k, grid, ps, stream)) return st;
+      if (fq_status st = launch(ctx, *k, persistent_grid(ctx, *k, src->n_rows), ps, stream)) return st;
     }
     if (probe || force_dense) {   // the dense-tuned build: returns at once when the probe chose the other one
       fq_launch_params pd = p;
-      pd.stages = pipe->seld_stages;
+      pd.stages = kd.stages;
       pd.stages2 = 1;
       pd.n_tiles = segs_dense;
-      const unsigned grid = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)ctx->sm_count, pd.n_tiles));
-      if (fq_status st = launch(ctx, pipe->k_select_dense, grid, pd, stream)) return st;
+      if (fq_status st = launch(ctx, kd, persistent_grid(ctx, kd, src->n_rows), pd, stream)) return st;
     }
     pipe->project_has_pred_launch = true;
   } else {
@@ -1555,18 +1535,10 @@ fq_status fq_pipe_launch_project(fq_ctx *ctx, fq_pipe *pipe, const fq_source *sr
       const uint64_t blocks = ((uint64_t)limit + FQ_REF_BLOCK_ROWS - 1) / FQ_REF_BLOCK_ROWS;
       p.n_rows = std::min<uint64_t>(p.n_rows, std::max<uint64_t>(blocks, 1) * FQ_REF_BLOCK_ROWS);
     }
-    // FQ_MAP_VARIANT = tma (default: reads staged by bulk copies; needs every referenced column materialised) | ldg
-    const std::string &variant = pipe->variant;
-    if (p.bits_unstaged && !pipe->k_map.valid())
-      return set_err(FQ_ERR_INTERNAL, "Internal Error: validity bitmap off the 128-row grid needs the LDG kernel, which this pipe was not built with");
-    const bool use_tma = !p.bits_unstaged && ((variant == "tma" && pipe->k_map_tma.valid()) || !pipe->k_map.valid());
-    const Kernel &k = use_tma ? pipe->k_map_tma : pipe->k_map;
-    if (!k.valid()) return set_err(FQ_ERR_INTERNAL, "Internal Error: no projection kernel was built for this pipe");
-    p.stages = pipe->mapt_stages;
-    const uint64_t chunk_rows = (uint64_t)(use_tma ? shapes().tma_threads * shapes().tma_unroll : k.threads * shapes().map_unroll) * pipe->gen.vec;
-    const uint64_t chunks = (p.n_rows + chunk_rows - 1) / chunk_rows;
-    unsigned grid = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)ctx->sm_count * k.blocks_per_sm, chunks));
-    if (fq_status st = launch(ctx, k, grid, p, stream)) return st;
+    const Kernel *k;
+    if (fq_status st = pick_kernel(pipe, K_MAP_TMA, K_MAP, p, "projection", &k)) return st;
+    p.stages = pipe->k[K_MAP_TMA].stages;
+    if (fq_status st = launch(ctx, *k, persistent_grid(ctx, *k, p.n_rows), p, stream)) return st;
   }
   CUDA_TRY(cudaMemcpyAsync(pipe->h_result, pipe->d_ctl, 48, cudaMemcpyDeviceToHost, (cudaStream_t)stream));
   if (fq_status st = mark_done(ctx, pipe->ev, (cudaStream_t)stream)) return st;
@@ -1864,17 +1836,15 @@ fq_status fq_pipe_launch_groupby(fq_ctx *ctx, fq_pipe *pipe, const fq_source *sr
   p.gb_reps = pipe->gb_reps;
   p.gb_seed = pipe->gb_seed;
   p.result = (fq_u64 *)(pipe->gb_flags + 2);   // [0] = count (u64 at flags[2..3]), [1] = error bits (flags[4..5])
-  const Kernel &k = pipe->k_groupby;
+  const Kernel &k = pipe->k[K_GROUPBY];
   if (!k.valid()) return set_err(FQ_ERR_INTERNAL, "Internal Error: no GROUP BY kernel was built for this pipe");
   if (src->n_rows > 0) {
-    const uint64_t chunk_rows = (uint64_t)k.threads * FQ_GB_UNROLL * pipe->gen.vec;
-    const uint64_t chunks = (src->n_rows + chunk_rows - 1) / chunk_rows;
-    const unsigned grid = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)ctx->sm_count * k.blocks_per_sm, chunks));
+    const unsigned grid = persistent_grid(ctx, k, src->n_rows);
     if (grid < p.gb_reps) p.gb_reps = 1;   // a small scan: every CTA on the table itself, nothing to fold
     if (fq_status st = launch(ctx, k, grid, p, stream)) return st;
     if (p.gb_reps > 1) {
       // fold the replicas into the table (and leave them empty): the merge kernel without an entry list
-      const Kernel &km = pipe->k_gbmerge;
+      const Kernel &km = pipe->k[K_GBMERGE];
       if (!km.valid()) return set_err(FQ_ERR_INTERNAL, "Internal Error: no GROUP BY merge kernel was built for this pipe");
       fq_launch_params q = p;
       q.n_rows = (pipe->gb_cap + 1) * (uint64_t)(pipe->gb_reps - 1);
@@ -2000,7 +1970,7 @@ fq_status fq_pipe_merge_partials(fq_ctx *ctx, fq_pipe *pipe, const fq_column *en
     p.gb_flags = (fq_u32 *)pipe->gb_flags;
     p.gb_seed = pipe->gb_seed;
     p.gb_entries = (const fq_u64 *)entries->ptr;
-    const Kernel &k = pipe->k_gbmerge;
+    const Kernel &k = pipe->k[K_GBMERGE];
     if (!k.valid()) return set_err(FQ_ERR_INTERNAL, "Internal Error: no GROUP BY merge kernel was built for this pipe");
     const unsigned grid = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((n_entries + 255) / 256, (uint64_t)ctx->sm_count * 8));
     if (fq_status st = launch(ctx, k, grid, p, stream)) return st;

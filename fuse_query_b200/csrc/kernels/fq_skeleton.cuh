@@ -37,7 +37,6 @@ typedef signed char fq_i8;
 #ifndef FQ_AGG_THREADS
 #define FQ_AGG_THREADS 256
 #define FQ_AGG_MIN_BLOCKS 4
-#define FQ_AGG_MIN_BLOCKS_U8 2
 #define FQ_TMA_THREADS 256   // consumer threads (+32 for the producer warp)
 #define FQ_TMA_UNROLL 8      // tile = 256 * 8 vector groups = 32 KB of a UInt64 column per bulk copy
 #define FQ_TMA_STAGES 8      // upper bound of the ring; the host picks stages so that ~128 KB are in flight per SM

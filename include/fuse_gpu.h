@@ -259,9 +259,10 @@ typedef struct fq_pipe fq_pipe;
 
 fq_status fq_pipe_compile(fq_ctx *ctx, const fq_pipe_desc *desc, fq_pipe **out);
 void fq_pipe_destroy(fq_ctx *ctx, fq_pipe *pipe);
-/* Kernel variant the pipe's launches prefer: aggregate pipes "tma" (bulk-copy staged, default) | "u4" | "u8" (LDG.128 x 4 / x 8),
- * select and projection pipes "tma" | "ldg".  The default comes from FQ_AGG_VARIANT / FQ_SEL_VARIANT / FQ_MAP_VARIANT, read once
- * when the pipe is compiled (never on the launch path).  A variant the pipe's module does not hold falls back to one it does. */
+/* Kernel variant the pipe's launches prefer: aggregate pipes "tma" (bulk-copy staged, default) | "u4" (LDG.128 x 4), filter +
+ * projection pipes "tma" | "sparse" | "dense" | "ldg", projection pipes "tma" | "ldg"; GROUP BY pipes have none.  The default
+ * comes from FQ_AGG_VARIANT / FQ_SEL_VARIANT / FQ_MAP_VARIANT, read once when the pipe is compiled (never on the launch path);
+ * another word is FQ_ERR_INVALID, there and here.  A variant the pipe's module does not hold falls back to one it does. */
 fq_status fq_pipe_set_variant(fq_ctx *ctx, fq_pipe *pipe, const char *variant);
 /* 1 if the kernel came from the library's precompiled table, 0 if NVRTC built it */
 int32_t fq_pipe_is_precompiled(const fq_pipe *pipe);

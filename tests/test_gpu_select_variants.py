@@ -27,7 +27,7 @@ def all_jit_variants():
 @pytest.fixture(params=["ldg", "tma", "dense"])
 def variant(request):
     old = os.environ.get("FQ_SEL_VARIANT")
-    os.environ["FQ_SEL_VARIANT"] = request.param     # read by the library at every launch
+    os.environ["FQ_SEL_VARIANT"] = request.param     # read by the library when a pipe is compiled
     yield request.param
     if old is None:
         os.environ.pop("FQ_SEL_VARIANT", None)

@@ -31,9 +31,8 @@ case $what in
     timeout 1200 python tools/bench_utf8.py "$@"; echo "bench_utf8 rc=$?"
     ;;
   select)
-    # select-kernel shapes: timings with the staged pass 2 on / off, then ncu --set full of the dense / third / 1-in-1024 selections
-    FQ_SELT_STAGE2=1 timeout 600 python tools/bench_select.py > gpurun_out/bench_select_stage2.log 2>&1; echo "stage2=1 rc=$?"; cat gpurun_out/bench_select_stage2.log
-    FQ_SELT_STAGE2=0 timeout 600 python tools/bench_select.py > gpurun_out/bench_select_nostage2.log 2>&1; echo "stage2=0 rc=$?"; cat gpurun_out/bench_select_nostage2.log
+    # select-kernel shapes: timings with the dense build available (tma) / never launched (sparse), then ncu --set full of the dense / third / 1-in-1024 selections
+    for v in tma sparse; do FQ_SEL_VARIANT=$v timeout 600 python tools/bench_select.py 2>&1; echo "$v rc=$?"; done
     for c in all third 1024; do
       timeout 600 ncu --set full --clock-control none --import-source on -k regex:select --launch-skip 2 --launch-count 1 -o gpurun_out/ncu_select_$c -f python tools/prof_select.py 1000000000 $c > gpurun_out/ncu_select_$c.log 2>&1; echo "ncu $c rc=$?"
     done
