@@ -20,7 +20,8 @@ DTYPE_NAMES = ["Null", "Boolean", "Int8", "Int16", "Int32", "Int64", "UInt8", "U
 DTYPE_SIZE = {BOOL: 1, I8: 1, I16: 2, I32: 4, I64: 8, U8: 1, U16: 2, U32: 4, U64: 8, F32: 4, F64: 8}
 
 OK, ERR_INTERNAL, ERR_PLAN, ERR_DIVIDE_BY_ZERO, ERR_UNSUPPORTED, ERR_CUDA, ERR_INVALID, ERR_CAPACITY = range(8)
-EXPR_ALIAS, EXPR_CONSTANT, EXPR_FIELD, EXPR_ARITHMETIC, EXPR_COMPARISON, EXPR_LOGIC, EXPR_AGGREGATOR = range(7)
+EXPR_ALIAS, EXPR_CONSTANT, EXPR_FIELD, EXPR_ARITHMETIC, EXPR_COMPARISON, EXPR_LOGIC, EXPR_AGGREGATOR, EXPR_LOOKUP = range(8)
+MAX_LOOKUPS = 4
 PIPE_PROJECT, PIPE_AGGREGATE, PIPE_GROUPBY = 0, 1, 2
 RUN_ACCUMULATE, RUN_LIMIT_EARLY_EXIT, RUN_BLOCK_STATS = 1, 2, 4
 STATE_HEADER_SLOTS = 6   # FQ_STATE_HEADER_SLOTS
@@ -80,7 +81,7 @@ EXPORTS = [
     "fq_pipe_key_dtype", "fq_pipe_leaf_dtype", "fq_pipe_groupby_reserve", "fq_pipe_launch_groupby", "fq_pipe_fetch_groupby",
     "fq_pipe_export_groups", "fq_pipe_group_entry_slots", "fq_pipe_export_partials", "fq_pipe_merge_partials",
     "fq_column_set_validity_bitmap", "fq_utf8_create", "fq_utf8_free", "fq_utf8_len", "fq_utf8_compare", "fq_utf8_compare_scalar", "fq_utf8_minmax",
-    "fq_utf8_bytes", "fq_utf8_download", "fq_utf8_take", "fq_utf8_dict_encode", "fq_utf8_bounds",
+    "fq_utf8_bytes", "fq_utf8_download", "fq_utf8_take", "fq_utf8_dict_encode", "fq_utf8_bounds", "fq_utf8_like", "fq_pipe_set_lookup",
     "fq_sort_indices", "fq_sort_indices_limit", "fq_column_take", "fq_column_copy", "fq_ctx_trim",
     "fq_graph_begin", "fq_graph_end", "fq_graph_launch", "fq_graph_destroy", "fq_stream_create", "fq_stream_destroy",
 ]
@@ -169,6 +170,8 @@ def lib():
         "fq_utf8_take": (i32, [vp, vp, vp, u64, vp, C.POINTER(vp), vp]),
         "fq_utf8_dict_encode": (i32, [vp, vp, vp, C.POINTER(vp), vp]),
         "fq_utf8_bounds": (i32, [vp, vp, vp, u64, C.POINTER(u64), C.POINTER(u64), vp]),
+        "fq_utf8_like": (i32, [vp, vp, vp, u64, i32, vp, vp]),
+        "fq_pipe_set_lookup": (i32, [vp, vp, i32, vp, u64]),
         "fq_sort_indices": (i32, [vp, vp, vp, i32, u64, vp, vp]),
         "fq_sort_indices_limit": (i32, [vp, vp, vp, i32, u64, u64, vp, C.POINTER(u64), vp]),
         "fq_column_take": (i32, [vp, vp, vp, u64, vp, vp, vp]),
@@ -244,6 +247,10 @@ class ExprBuilder:
             i += 1
             child, i = self._parse(t, i)
             node = self._push(kind=EXPR_ALIAS, left=child)
+        elif head == "lookup":   # (lookup <slot> <index expression>)
+            slot = int(t[i])
+            child, i = self._parse(t, i + 1)
+            node = self._push(kind=EXPR_LOOKUP, op=slot, left=child)
         elif head.lower() in AGG:
             child, i = self._parse(t, i)
             node = self._push(kind=EXPR_AGGREGATOR, op=AGG[head.lower()], left=child)
@@ -615,6 +622,17 @@ class Utf8Array:
                                             C.c_void_p(stream)))
         return lo.value, hi.value
 
+    def like(self, pattern, negate: bool = False, stream: int = 0) -> Column:
+        """fq_utf8_like: a UInt8 column of ceil(len / 8) bytes, bit i = string i LIKE `pattern` (str or bytes), negated by
+        `negate`; NULL rows and the padding bits get 0.  An empty array gets one zero byte (a column is never empty)."""
+        import numpy as np
+        b = pattern.encode() if isinstance(pattern, str) else bytes(pattern)
+        n = len(self)
+        bits = self.ctx.column(U8, (n + 7) // 8) if n else self.ctx.from_numpy(np.zeros(1, dtype=np.uint8))
+        self.ctx.check(lib().fq_utf8_like(self.ctx._h, self._h, C.create_string_buffer(b, max(1, len(b))), len(b), int(negate), bits._h,
+                                          C.c_void_p(stream)))
+        return bits
+
     def free(self):
         if self._h:
             lib().fq_utf8_free(self.ctx._h, self._h)
@@ -709,6 +727,11 @@ class Pipe:
     def set_group(self, group: Optional["Group"]) -> None:
         """Aggregate launches end with the in-kernel merge across the group's ranks (fetch_merged reads it)."""
         self.ctx.check(lib().fq_pipe_set_group(self.ctx._h, self._h, group._h if group is not None else None))
+
+    def set_lookup(self, slot: int, bits: Column, n_bits: int) -> None:
+        """Binds bit table `slot` of the pipe's (lookup <slot> ...) nodes: a UInt8 column, LSB-first, read by later launches
+        (keep it alive as long as they run)."""
+        self.ctx.check(lib().fq_pipe_set_lookup(self.ctx._h, self._h, slot, bits._h, n_bits))
 
     def set_variant(self, variant: str) -> None:
         """Kernel variant for the next launches: "tma" | "u4" (aggregate), "tma" | "sparse" | "dense" | "ldg" (filter +

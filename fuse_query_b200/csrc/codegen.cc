@@ -84,6 +84,7 @@ struct Gen {
   int status = FQ_OK;
   bool const_div0 = false;
   int quiet_depth = 0;
+  unsigned lookup_slots = 0;   // bit k: some FQ_EXPR_LOOKUP node reads table k
 
   // columns referenced below node i (any depth)
   void cols_below(int i, std::set<int> *out, int depth = 0) const {
@@ -199,6 +200,18 @@ struct Gen {
         ty[i] = FQ_BOOL;
         return true;
       }
+      case FQ_EXPR_LOOKUP: {
+        if (n->op < 0 || n->op >= FQ_MAX_LOOKUPS)
+          return fail(FQ_ERR_INVALID, fmt("Internal Error: lookup slot %d out of range [0, %d)", n->op, FQ_MAX_LOOKUPS));
+        if (!infer(n->left, depth + 1)) return false;
+        const fq_dtype t = ty[n->left];
+        if (t < FQ_U8 || t > FQ_U64)
+          return fail(FQ_ERR_INVALID, fmt("Internal Error: a lookup takes an unsigned integer index, not %s", dtype_name(t)));
+        if (scalar[n->left]) return fail(FQ_ERR_INVALID, "Internal Error: a lookup of a constant index");
+        lookup_slots |= 1u << n->op;
+        ty[i] = FQ_BOOL;
+        return true;
+      }
       default:
         return fail(FQ_ERR_INVALID, fmt("Internal Error: unknown expression node kind %d", n->kind));
     }
@@ -284,6 +297,12 @@ struct Gen {
           val[i] = val[n.left];
           ok[i] = ok[n.left];
           return;
+        case FQ_EXPR_LOOKUP:   // the row functions receive the launch parameters, which hold the bound tables
+          node(n.left);
+          body += ind + fmt("const bool n%d = fq_lookup(p.lookup[%d], p.lookup_bits[%d], (fq_u64)(", i, n.op, n.op) + val[n.left] + "));\n";
+          val[i] = fmt("n%d", i);
+          ok[i] = ok[n.left];
+          return;
         default: break;
       }
       node(n.left);
@@ -337,7 +356,7 @@ struct Gen {
     const fq_expr_node &n = d.nodes[i];
     switch (n.kind) {
       case FQ_EXPR_AGGREGATOR: out.insert(i); break;
-      case FQ_EXPR_ALIAS: collect_aggs(n.left, out); break;
+      case FQ_EXPR_ALIAS: case FQ_EXPR_LOOKUP: collect_aggs(n.left, out); break;
       case FQ_EXPR_ARITHMETIC: case FQ_EXPR_COMPARISON: case FQ_EXPR_LOGIC:
         collect_aggs(n.left, out);
         collect_aggs(n.right, out);
@@ -503,6 +522,7 @@ int generate(const fq_pipe_desc &d, Generated *out, std::string *err) {
   s += "  struct Rows {";
   for (int c : g.used_cols) s += fmt(" %s c%d[V];", ctype(g.col_dtype(c)), c);
   for (int c : null_cols) s += fmt(" bool k%d[V];", c);
+  out->lookup_slots = g.lookup_slots;
   s += " };\n";
   s += "  __device__ static __forceinline__ void load(Rows &r, const fq_launch_params &p, fq_u64 g) {\n";
   for (int c : g.used_cols) {
@@ -658,7 +678,7 @@ int generate(const fq_pipe_desc &d, Generated *out, std::string *err) {
     s += "  }\n";
   }
   // WHERE: a NULL predicate keeps nothing
-  s += "  __device__ static __forceinline__ bool pred(const Rows &r, int v, fq_u32 &err) {\n";
+  s += "  __device__ static __forceinline__ bool pred(const fq_launch_params &p, const Rows &r, int v, fq_u32 &err) {\n";
   if (out->has_pred) {
     Gen::Emitter e(g, "    ");
     e.node(d.predicate);
@@ -673,8 +693,8 @@ int generate(const fq_pipe_desc &d, Generated *out, std::string *err) {
     auto is_f = [&](int k) { return is_float(out->agg_dtypes[k]); };
     auto is_s = [&](int k) { return is_signed_int(out->agg_dtypes[k]); };
     s += fmt("  static constexpr int G = %d;\n", 1 + n_slots);
-    s += "  __device__ static __forceinline__ bool gb_row(const Rows &r, int v, fq_u32 &err, fq_u64 &key, fq_u64 (&val)[NSLOTS > 0 ? NSLOTS : 1], fq_u32 &vmask) {\n";
-    if (out->has_pred) s += "    if (!pred(r, v, err)) return false;\n";
+    s += "  __device__ static __forceinline__ bool gb_row(const fq_launch_params &p, const Rows &r, int v, fq_u32 &err, fq_u64 &key, fq_u64 (&val)[NSLOTS > 0 ? NSLOTS : 1], fq_u32 &vmask) {\n";
+    if (out->has_pred) s += "    if (!pred(p, r, v, err)) return false;\n";
     {
       Gen::Emitter e(g, "    ");
       std::string st = "    key = 0ull;\n    vmask = 0u;\n";
@@ -779,8 +799,8 @@ int generate(const fq_pipe_desc &d, Generated *out, std::string *err) {
     for (int k = 0; k < n; k++)
       if (leaf_counted[k]) s += fmt("    a.c%d = 0;\n", k);
     s += "  }\n";
-    s += "  __device__ static __forceinline__ bool consume(Acc &a, const Rows &r, int v, fq_u64 &nsel, fq_u32 &err) {\n";
-    if (out->has_pred) s += "    if (!pred(r, v, err)) return false;\n    nsel += 1;\n";
+    s += "  __device__ static __forceinline__ bool consume(const fq_launch_params &p, Acc &a, const Rows &r, int v, fq_u64 &nsel, fq_u32 &err) {\n";
+    if (out->has_pred) s += "    if (!pred(p, r, v, err)) return false;\n    nsel += 1;\n";
     {
       Gen::Emitter e(g, "    ");
       std::string upd;
@@ -963,6 +983,12 @@ struct SexprParser {
     } else if (h == "alias") {
       tok();
       n.kind = FQ_EXPR_ALIAS;
+      n.left = parse();
+      if (n.left < 0) return -1;
+      done = true;
+    } else if (h == "lookup") {   // (lookup <slot> <index expression>)
+      n.kind = FQ_EXPR_LOOKUP;
+      n.op = (int)strtol(tok().c_str(), nullptr, 10);
       n.left = parse();
       if (n.left < 0) return -1;
       done = true;

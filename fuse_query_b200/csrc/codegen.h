@@ -42,6 +42,7 @@ struct Generated {
   bool sel_tma_ok = false;              // ... and the predicate reads at least one column: the staged select kernel exists
   bool track_blocks = false;            // aggregate pipe with a predicate and a Sum leaf: reference-block tracking compiled in
   bool const_divide_by_zero = false;    // a literal zero divisor is evaluated for every scanned row
+  unsigned lookup_slots = 0;            // bit k: an FQ_EXPR_LOOKUP node reads table k, which every launch needs bound
 };
 
 // Returns FQ_OK or an fq_status; `err` receives the FuseQueryError-style message.
@@ -53,7 +54,7 @@ const char *dtype_name(fq_dtype t);   // arrow DataType Debug
 size_t dtype_size(fq_dtype t);
 
 // Tiny s-expression reader used by the build-time AOT generator and the C++ tests:
-//   (col number) (u64 1) (+ a b) (sum a) (alias c1 a) ...   `cols` maps names to column indexes.
+//   (col number) (u64 1) (+ a b) (sum a) (alias c1 a) (lookup 0 a) ...   `cols` maps names to column indexes.
 int parse_sexpr(const std::string &text, const std::vector<std::string> &cols, std::vector<fq_expr_node> *nodes,
                 int *root, std::string *err);
 

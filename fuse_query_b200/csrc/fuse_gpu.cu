@@ -379,7 +379,12 @@ struct fq_pipe {
   uint64_t capacity_eff = 0;
   bool skipped = false;     // project launch over zero rows
   bool project_has_pred_launch = false;
+  // bit tables of the pipe's FQ_EXPR_LOOKUP nodes (fq_pipe_set_lookup), borrowed
+  const fq_u8 *lookup[FQ_MAX_LOOKUPS] = {nullptr, nullptr, nullptr, nullptr};
+  uint64_t lookup_bits[FQ_MAX_LOOKUPS] = {0, 0, 0, 0};
+  unsigned lookup_bound = 0;   // bit k: slot k is bound
 };
+static_assert(sizeof(((fq_launch_params *)nullptr)->lookup) / sizeof(void *) == FQ_MAX_LOOKUPS, "fq_launch_params holds FQ_MAX_LOOKUPS tables");
 
 namespace {
 
@@ -601,6 +606,12 @@ fq_status bind_source(const fq_pipe *pipe, const fq_source *src, fq_launch_param
     return set_err(FQ_ERR_INVALID, "Internal Error: pipe was compiled for a %s source", pipe->gen.generated_source ? "generated" : "materialised");
   p->n_rows = src->n_rows;
   p->numbers_begin = src->numbers_begin;
+  for (int k = 0; k < FQ_MAX_LOOKUPS; k++) {
+    if (!(pipe->gen.lookup_slots & (1u << k))) continue;
+    if (!(pipe->lookup_bound & (1u << k))) return set_err(FQ_ERR_INVALID, "Internal Error: lookup slot %d of the pipe is not bound (fq_pipe_set_lookup)", k);
+    p->lookup[k] = pipe->lookup[k];
+    p->lookup_bits[k] = pipe->lookup_bits[k];
+  }
   for (int c : pipe->gen.used_cols) {
     if (pipe->gen.generated_source && c == 0) continue;
     if (c >= src->n_cols || !src->cols || !src->cols[c]) return set_err(FQ_ERR_INVALID, "Internal Error: source lacks column %d", c);
@@ -1015,6 +1026,16 @@ void fq_pipe_destroy(fq_ctx *ctx, fq_pipe *pipe) {
 fq_status fq_pipe_set_variant(fq_ctx *, fq_pipe *pipe, const char *variant) {
   if (!pipe || !variant) return set_err(FQ_ERR_INVALID, "Internal Error: null argument");
   return parse_variant(pipe->gen, variant, &pipe->variant);
+}
+fq_status fq_pipe_set_lookup(fq_ctx *, fq_pipe *pipe, int32_t slot, const fq_column *bits, uint64_t n_bits) {
+  if (!pipe || !bits) return set_err(FQ_ERR_INVALID, "Internal Error: null argument");
+  if (slot < 0 || slot >= FQ_MAX_LOOKUPS) return set_err(FQ_ERR_INVALID, "Internal Error: lookup slot %d out of range [0, %d)", slot, FQ_MAX_LOOKUPS);
+  if (bits->dtype != FQ_U8 || bits->len < (n_bits + 7) / 8)
+    return set_err(FQ_ERR_INVALID, "Internal Error: a lookup table of %" PRIu64 " bits is a UInt8 column of at least %" PRIu64 " bytes", n_bits, (n_bits + 7) / 8);
+  pipe->lookup[slot] = (const fq_u8 *)bits->ptr;
+  pipe->lookup_bits[slot] = n_bits;
+  pipe->lookup_bound |= 1u << slot;
+  return FQ_OK;
 }
 int32_t fq_pipe_is_precompiled(const fq_pipe *pipe) { return pipe && pipe->precompiled; }
 int32_t fq_pipe_build_kind(const fq_pipe *pipe) { return pipe ? pipe->build_kind : 0; }
@@ -2609,6 +2630,32 @@ fq_status fq_utf8_dict_encode(fq_ctx *ctx, const fq_utf8 *src, fq_column *codes,
   }
   // the dictionary: the representative rows in sorted order (waits for the stream)
   return utf8_take(ctx, src, rows, d, nullptr, s, dict);
+}
+
+fq_status fq_utf8_like(fq_ctx *ctx, const fq_utf8 *a, const void *pattern, uint64_t pattern_len, int32_t negate, fq_column *bits,
+                       void *stream) {
+  if (fq_status st = use(ctx)) return st;
+  if (!a || !bits || (pattern_len && !pattern)) return set_err(FQ_ERR_INVALID, "Internal Error: null argument");
+  if (bits->dtype != FQ_U8 || bits->len < (a->len + 7) / 8)
+    return set_err(FQ_ERR_INVALID, "Internal Error: LIKE bits of %" PRIu64 " rows need a UInt8 column of at least %" PRIu64 " bytes", a->len, (a->len + 7) / 8);
+  if (pattern_len > (uint64_t)INT32_MAX) return set_err(FQ_ERR_INVALID, "Internal Error: LIKE pattern over 2 GiB");
+  // a `\` escapes the byte after it: the pattern ends in an unpaired one when the run of `\` at its end is odd
+  const unsigned char *pat = (const unsigned char *)pattern;
+  uint64_t run = 0;
+  while (run < pattern_len && pat[pattern_len - 1 - run] == '\\') run++;
+  if (run & 1) return set_err(FQ_ERR_INVALID, "Internal Error: LIKE pattern ends with the escape character \\");
+  if (a->len == 0) return FQ_OK;
+  cudaStream_t s = (cudaStream_t)stream;
+  StreamScratch scratch(s);
+  unsigned char *dev = nullptr;
+  CUDA_TRY(scratch.get(&dev, pattern_len));
+  if (pattern_len) CUDA_TRY(cudaMemcpyAsync(dev, pattern, pattern_len, cudaMemcpyHostToDevice, s));
+  fq_utf8_like_kernel<<<grid_for(ctx, a->len, 16), 256, 0, s>>>(a->offsets, a->data, a->validity ? (const fq_u8 *)a->validity->ptr : nullptr, a->len,
+                                                                dev, (fq_u32)pattern_len, negate ? 1 : 0, (fq_u8 *)bits->ptr);
+  CUDA_TRY(cudaGetLastError());
+  ctx->launches++;
+  CUDA_TRY(cudaStreamSynchronize(s));   // `pattern` may go away after the call
+  return FQ_OK;
 }
 
 fq_status fq_utf8_bounds(fq_ctx *ctx, const fq_utf8 *dict, const void *scalar, uint64_t scalar_len, uint64_t *lower, uint64_t *upper,

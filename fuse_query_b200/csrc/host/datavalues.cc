@@ -1,4 +1,5 @@
 // datavalues.cc — host mirror of src/datavalues: DataValue, coercion, scalar merges, device arrays.
+#include <algorithm>
 #include <cinttypes>
 #include <cmath>
 #include <cstdio>
@@ -440,6 +441,25 @@ std::pair<uint64_t, uint64_t> Utf8Dict::bounds(const std::string &literal) const
   if (bounds_.size() >= 4096) bounds_.clear();   // many distinct literals: keep the memory bounded
   bounds_[literal] = b;
   return b;
+}
+DataArrayRef Utf8Dict::like(const std::string &pattern, bool negate) const {
+  std::lock_guard<std::mutex> lock(mu_);
+  const auto key = std::make_pair(pattern, negate);
+  auto it = like_.find(key);
+  if (it != like_.end()) return it->second;
+  const uint64_t bytes = std::max<uint64_t>(1, (size + 7) / 8);
+  // fq_utf8_like writes ceil(size / 8) bytes: the table of an empty dictionary is one zero byte, so that no byte of it is left unset
+  static const unsigned char zero = 0;
+  DataArrayRef bits = size ? DataArray::alloc(ctx, FQ_U8, bytes) : DataArray::from_host(ctx, FQ_U8, &zero, 1);
+  ctx->check(fq_utf8_like(ctx->raw(), raw, pattern.data(), pattern.size(), negate ? 1 : 0, bits->column(), ctx->stream));
+  // many distinct patterns: keep the memory bounded (pipes that still read a table share its ownership)
+  if (like_.size() >= 4096 || like_bytes_ + bytes > (256ull << 20)) {
+    like_.clear();
+    like_bytes_ = 0;
+  }
+  like_[key] = bits;
+  like_bytes_ += bytes;
+  return bits;
 }
 
 DataArray::~DataArray() {

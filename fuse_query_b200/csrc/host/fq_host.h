@@ -87,6 +87,7 @@ using DataSchemaRef = std::shared_ptr<const DataSchema>;
 
 class GpuContext;
 using GpuContextRef = std::shared_ptr<GpuContext>;
+class DataArray;
 
 // The sorted dictionary of a dictionary-encoded Utf8 column (fq_utf8_dict_encode): distinct valid strings in bytewise
 // order on the device, shared by the column, its slices and every result column decoded through it.
@@ -98,10 +99,15 @@ struct Utf8Dict {
   std::string at(uint32_t code) const;   // one entry, through fq_utf8_take
   // fq_utf8_bounds of a literal, remembered: a dictionary never changes, and every pipe of a query lowers the same literals
   std::pair<uint64_t, uint64_t> bounds(const std::string &literal) const;
+  // bit `code` = entry `code` LIKE `pattern` (NOT LIKE when `negate`): a UInt8 column of ceil(size / 8) bytes (at least one)
+  // from fq_utf8_like, remembered like the bounds.  Pipes read it through an FQ_EXPR_LOOKUP node.
+  std::shared_ptr<DataArray> like(const std::string &pattern, bool negate) const;
 
  private:
   mutable std::mutex mu_;
   mutable std::map<std::string, std::pair<uint64_t, uint64_t>> bounds_;
+  mutable std::map<std::pair<std::string, bool>, std::shared_ptr<DataArray>> like_;
+  mutable uint64_t like_bytes_ = 0;
 };
 using Utf8DictRef = std::shared_ptr<const Utf8Dict>;
 
@@ -199,6 +205,7 @@ DataValue data_array_aggregate_op(GpuContextRef ctx, int op, const DataArrayRef 
 struct PipeHandle {
   GpuContextRef ctx;
   fq_pipe *pipe = nullptr;
+  std::vector<DataArrayRef> lookups;   // bit tables bound with fq_pipe_set_lookup: the pipe borrows them
   ~PipeHandle();
 };
 using PipeRef = std::shared_ptr<PipeHandle>;
@@ -249,9 +256,9 @@ using FunctionRef = std::shared_ptr<Function>;
 
 class Function {
  public:
-  enum Kind { Alias, Constant, Variable, Arithmetic, Comparison, Logic, Aggregator };
+  enum Kind { Alias, Constant, Variable, Arithmetic, Comparison, Logic, Aggregator, Like };
   Kind kind;
-  int op = 0;               // FQ_AR_* / FQ_CMP_* / FQ_LG_* / FQ_AGG_*
+  int op = 0;               // FQ_AR_* / FQ_CMP_* / FQ_LG_* / FQ_AGG_*; Like: 1 = NOT LIKE
   size_t depth = 0;
   std::string name;         // field name / alias
   DataValue value;          // constant value; aggregator state (starts Null, function_aggregator.rs:30)
@@ -265,6 +272,8 @@ class Function {
   static FunctionRef ComparisonFunction(int op, const std::vector<FunctionRef> &args);   // function_comparison.rs:25-37
   static FunctionRef LogicFunction(int op, const std::vector<FunctionRef> &args);        // function_logic.rs:25-33
   static FunctionRef AggregatorFunction(int op, const std::vector<FunctionRef> &args);   // function_aggregator.rs:25-36
+  // `s LIKE 'pattern'` / `s NOT LIKE 'pattern'` (no counterpart in the reference): Boolean, NULL where s is
+  static FunctionRef LikeFunction(bool negate, const std::vector<FunctionRef> &args);
   // ScalarFunctionFactory::get, function_factory.rs:17-39
   static FunctionRef factory_get(const std::string &name, const std::vector<FunctionRef> &args);
 

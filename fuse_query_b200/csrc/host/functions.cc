@@ -15,6 +15,7 @@ namespace fuse {
 static const char *arith_sym(int op) { static const char *s[] = {"+", "-", "*", "/"}; return s[op & 3]; }
 static const char *cmp_sym(int op) { static const char *s[] = {"=", "<", "<=", ">", ">="}; return s[op % 5]; }
 static const char *logic_sym(int op) { return op == FQ_LG_AND ? "and" : "or"; }
+static const char *like_sym(int op) { return op ? "NOT LIKE" : "LIKE"; }
 
 // ---------------------------------------------------------------------------------------------
 // lowering: Function tree + block -> fq_pipe_desc
@@ -65,7 +66,42 @@ static void dict_comparison(const Utf8Dict &d, int op, const DataValue &lit, int
     default: *code_op = FQ_CMP_GTEQ; *code = lb; break;
   }
 }
+// `s [NOT] LIKE 'pattern'` over a dictionary column: the pattern is matched once per dictionary entry (Utf8Dict::like), and
+// the pipe reads the bit of each row's code through a lookup slot, so its generated source does not depend on the pattern
+static const Function &like_pattern(const Function &f) {
+  const Function *pat = f.right.get();
+  while (pat->kind == Function::Alias) pat = pat->left.get();
+  return *pat;
+}
+// what LIKE accepts: a Utf8 operand and a string literal pattern (checked when the plan is typed and when it is lowered)
+static void check_like(const Function &f, const DataSchema &s) {
+  const DataType lt = f.left->return_type(s), rt = f.right->return_type(s);
+  if (lt != FQ_UTF8)
+    throw FuseQueryError::internal(std::string("Unsupported (") + data_type_name(lt) + ") " + like_sym(f.op) + " (" + data_type_name(rt) + ")");
+  const Function &pat = like_pattern(f);
+  if (pat.kind != Function::Constant || pat.value.tag != FQ_UTF8 || !pat.value.some)
+    throw FuseQueryError::internal("Unsupported on the device path: LIKE with a pattern that is not a string literal");
+}
+static int lower_like(Lowering &lw, const Function &f, const DataBlock &block) {
+  check_like(f, *block.schema());
+  const Utf8DictRef d = dict_of(*f.left, block);
+  if (!d) throw FuseQueryError::internal("Unsupported on the device path: LIKE over a Utf8 value that is not a dictionary-encoded column");
+  if (lw.lookups.size() == (size_t)FQ_MAX_LOOKUPS)
+    throw FuseQueryError::internal("Unsupported on the device path: more than " + std::to_string(FQ_MAX_LOOKUPS) + " LIKE predicates in one pipe");
+  const int slot = (int)lw.lookups.size();
+  lw.lookups.push_back({d->like(like_pattern(f).value.s, f.op != 0), d->size});
+  fq_expr_node n;
+  memset(&n, 0, sizeof n);
+  n.right = -1;
+  n.kind = FQ_EXPR_LOOKUP;
+  n.op = slot;
+  n.left = lw.lower(*f.left, block);
+  lw.nodes.push_back(n);
+  lw.node_of[&f] = (int)lw.nodes.size() - 1;
+  return (int)lw.nodes.size() - 1;
+}
 int Lowering::lower(const Function &f, const DataBlock &block) {
+  if (f.kind == Function::Like) return lower_like(*this, f, block);
   fq_expr_node n;
   memset(&n, 0, sizeof n);
   n.left = n.right = -1;
@@ -178,10 +214,14 @@ void bind_source(const Lowering &lw, const DataBlock &block, BoundSource *b) {
   b->src.numbers_begin = block.numbers_begin;
 }
 
-PipeRef compile_pipe(GpuContextRef ctx, const fq_pipe_desc &d) {
+PipeRef compile_pipe(GpuContextRef ctx, const Lowering &lw, const fq_pipe_desc &d) {
   auto h = std::make_shared<PipeHandle>();
   h->ctx = ctx;
   ctx->check(fq_pipe_compile(ctx->raw(), &d, &h->pipe));
+  for (size_t k = 0; k < lw.lookups.size(); k++) {
+    ctx->check(fq_pipe_set_lookup(ctx->raw(), h->pipe, (int32_t)k, lw.lookups[k].first->column(), lw.lookups[k].second));
+    h->lookups.push_back(lw.lookups[k].first);
+  }
   return h;
 }
 
@@ -209,7 +249,7 @@ ProjectResult run_project(GpuContextRef ctx, const DataBlock &block, const Funct
   std::vector<int> roots;
   for (const Function *f : funcs) roots.push_back(lw.lower(*f, block));
   fq_pipe_desc d = lw.desc(FQ_PIPE_PROJECT, pred, roots);
-  PipeRef pipe = compile_pipe(ctx, d);
+  PipeRef pipe = compile_pipe(ctx, lw, d);
   const uint64_t rows = block.rows();
   uint64_t cap = rows;
   if (limit >= 0 && (uint64_t)limit < cap) cap = (uint64_t)limit;
@@ -289,6 +329,11 @@ FunctionRef Function::LogicFunction(int op, const std::vector<FunctionRef> &args
   f->op = op;
   return binary(f, args);
 }
+FunctionRef Function::LikeFunction(bool negate, const std::vector<FunctionRef> &args) {
+  auto f = FunctionRef(new Function(Like));
+  f->op = negate ? 1 : 0;
+  return binary(f, args);
+}
 FunctionRef Function::AggregatorFunction(int op, const std::vector<FunctionRef> &args) {
   if (args.empty()) throw FuseQueryError::internal("index out of bounds: the len is 0 but the index is 0");
   auto f = FunctionRef(new Function(Aggregator));
@@ -312,6 +357,8 @@ FunctionRef Function::factory_get(const std::string &name, const std::vector<Fun
   if (n == ">=") return ComparisonFunction(FQ_CMP_GTEQ, args);
   if (n == "and") return LogicFunction(FQ_LG_AND, args);
   if (n == "or") return LogicFunction(FQ_LG_OR, args);
+  if (n == "like") return LikeFunction(false, args);
+  if (n == "not like") return LikeFunction(true, args);
   if (n == "count") return AggregatorFunction(FQ_AGG_COUNT, args);
   if (n == "min") return AggregatorFunction(FQ_AGG_MIN, args);
   if (n == "max") return AggregatorFunction(FQ_AGG_MAX, args);
@@ -340,6 +387,7 @@ DataType Function::return_type(const DataSchema &s) const {
     case Variable: return s.field_with_name(name).data_type;
     case Arithmetic: return numerical_coercion(arith_sym(op), left->return_type(s), right->return_type(s));  // function_arithmetic.rs:36-42
     case Comparison: case Logic: return FQ_BOOL;
+    case Like: check_like(*this, s); return FQ_BOOL;
     default: return op == FQ_AGG_COUNT ? (DataType)FQ_U64 : left->return_type(s);  // function_aggregator.rs:38-43
   }
 }
@@ -348,6 +396,7 @@ bool Function::nullable(const DataSchema &s) const {
     case Alias: return left->nullable(s);
     case Constant: return value.is_null();
     case Variable: return s.field_with_name(name).nullable;
+    case Like: return left->nullable(s);
     default: return false;
   }
 }
@@ -359,6 +408,7 @@ std::string Function::to_string() const {
     case Arithmetic: return left->to_string() + " " + arith_sym(op) + " " + right->to_string();
     case Comparison: return left->to_string() + " " + cmp_sym(op) + " " + right->to_string();
     case Logic: return left->to_string() + " " + logic_sym(op) + " " + right->to_string();
+    case Like: return left->to_string() + " " + like_sym(op) + " " + right->to_string();
     default: return std::string(agg[op & 3]) + "(" + left->to_string() + ")";
   }
 }
@@ -408,6 +458,7 @@ DataColumnarValue Function::eval(GpuContextRef ctx, const DataBlock &block) {
 
 static const char *unsupported_agg_name(const Function &f) {
   if (f.kind == Function::Variable) return "field";
+  if (f.kind == Function::Like) return like_sym(f.op);
   return f.kind == Function::Comparison ? cmp_sym(f.op) : logic_sym(f.op);
 }
 
@@ -415,7 +466,7 @@ void Function::accumulate(GpuContextRef ctx, const DataBlock &block) {
   switch (kind) {
     case Alias: left->accumulate(ctx, block); return;
     case Constant: case Variable: return;
-    case Arithmetic: case Comparison: case Logic:
+    case Arithmetic: case Comparison: case Logic: case Like:
       left->accumulate(ctx, block);
       right->accumulate(ctx, block);
       return;
@@ -433,7 +484,7 @@ void Function::accumulate(GpuContextRef ctx, const DataBlock &block) {
     if (block.generated) lw.column_of(block, block.schema()->fields[0].name);
     int root = lw.lower(*this, block);
     fq_pipe_desc d = lw.desc(FQ_PIPE_AGGREGATE, -1, {root});
-    PipeRef pipe = compile_pipe(ctx, d);
+    PipeRef pipe = compile_pipe(ctx, lw, d);
     BoundSource bs;
     bind_source(lw, block, &bs);
     ctx->check(fq_pipe_launch_aggregate(ctx->raw(), pipe->pipe, &bs.src, 0, ctx->stream));

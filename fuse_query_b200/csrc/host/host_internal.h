@@ -13,6 +13,7 @@ struct Lowering {
   std::vector<int> col_nullable;
   std::map<const Function *, int> node_of;
   std::map<const Function *, Utf8DictRef> leaf_dict;   // min / max leaves over a dictionary column: their state is a code
+  std::vector<std::pair<DataArrayRef, uint64_t>> lookups;   // slot k of the pipe's LOOKUP nodes: bit table, bits (one per LIKE)
   bool generated = false;
   int column_of(const DataBlock &block, const std::string &name);
   int lower(const Function &f, const DataBlock &block);
@@ -29,7 +30,8 @@ struct BoundSource {
   std::vector<const fq_column *> cols;
 };
 void bind_source(const Lowering &lw, const DataBlock &block, BoundSource *b);
-PipeRef compile_pipe(GpuContextRef ctx, const fq_pipe_desc &d);
+// compiles the pipe `d` lowered by `lw` and binds its lookup tables
+PipeRef compile_pipe(GpuContextRef ctx, const Lowering &lw, const fq_pipe_desc &d);
 
 struct ProjectResult {
   std::vector<DataArrayRef> columns;

@@ -553,6 +553,7 @@ static void collect_states(const Function &f, const std::map<const Function *, D
     case Function::Variable: throw FuseQueryError::internal("Unsupported aggregate operation for function field");
     case Function::Comparison:
       throw FuseQueryError::internal(std::string("Unsupported aggregate operation for function ") + (const char *[]){"=", "<", "<=", ">", ">="}[f.op % 5]);
+    case Function::Like: throw FuseQueryError::internal(std::string("Unsupported aggregate operation for function ") + (f.op ? "NOT LIKE" : "LIKE"));
     default: throw FuseQueryError::internal(std::string("Unsupported aggregate operation for function ") + (f.op == FQ_LG_AND ? "and" : "or"));
   }
 }
@@ -610,7 +611,7 @@ SendableDataBlockStream GpuPipeTransform::execute() {
           std::vector<int> roots;
           for (const Function *f : pt.funcs) roots.push_back(pt.lw.lower(*f, *block));
           fq_pipe_desc d = pt.lw.desc(FQ_PIPE_AGGREGATE, p, roots);
-          pt.pipe = compile_pipe(gpu, d);
+          pt.pipe = compile_pipe(gpu, pt.lw, d);
         }
         BoundSource bs;
         bind_source(pt.lw, *block, &bs);
@@ -713,6 +714,7 @@ static FunctionRef over_leaves(const Function &f, const std::map<const Function 
     case Function::Variable: throw FuseQueryError::internal("Unsupported aggregate operation for function field");
     case Function::Comparison:
       throw FuseQueryError::internal(std::string("Unsupported aggregate operation for function ") + (const char *[]){"=", "<", "<=", ">", ">="}[f.op % 5]);
+    case Function::Like: throw FuseQueryError::internal(std::string("Unsupported aggregate operation for function ") + (f.op ? "NOT LIKE" : "LIKE"));
     default: throw FuseQueryError::internal(std::string("Unsupported aggregate operation for function ") + (f.op == FQ_LG_AND ? "and" : "or"));
   }
 }
@@ -761,7 +763,7 @@ SendableDataBlockStream GpuGroupByTransform::execute() {
         fq_pipe_desc d = lw.desc(FQ_PIPE_GROUPBY, p, roots);
         d.n_keys = (int)key_roots.size();
         for (size_t k = 0; k < key_roots.size(); k++) d.keys[k] = key_roots[k];
-        pipe = compile_pipe(gpu, d);
+        pipe = compile_pipe(gpu, lw, d);
       }
       if (launches == 0) gpu->check(fq_pipe_groupby_reserve(gpu->raw(), pipe->pipe, hint));
       BoundSource bs;

@@ -346,14 +346,23 @@ struct SqlParser {
     return false;
   }
 
-  // precedence climbing as sqlparser: OR(5) < AND(10) < comparisons(20) < + -(30) < * / %(40)
+  bool next_is_kw(const char *kw) const {
+    if (t[p].k == Tok::End || t[p + 1].k != Tok::Word) return false;
+    std::string w = t[p + 1].text;
+    std::transform(w.begin(), w.end(), w.begin(), ::toupper);
+    return w == kw;
+  }
+
+  // precedence climbing as sqlparser: OR(5) < AND(10) < comparisons, LIKE, NOT LIKE(20) < + -(30) < * / %(40)
   ExpressionPlan expr(int min_prec = 0) {
     ExpressionPlan lhs = prefix();
     for (;;) {
-      int prec = 0;
+      int prec = 0, width = 1;
       std::string op;
       if (is_kw("OR")) { prec = 5; op = "OR"; }
       else if (is_kw("AND")) { prec = 10; op = "AND"; }
+      else if (is_kw("LIKE")) { prec = 20; op = "LIKE"; }
+      else if (is_kw("NOT") && next_is_kw("LIKE")) { prec = 20; op = "NOT LIKE"; width = 2; }
       else if (peek().k == Tok::Sym) {
         const std::string &s = peek().text;
         if (s == "=" || s == "<" || s == ">" || s == "<=" || s == ">=" || s == "<>" || s == "!=") { prec = 20; op = s == "!=" ? "<>" : s; }
@@ -361,7 +370,7 @@ struct SqlParser {
         else if (s == "*" || s == "/" || s == "%") { prec = 40; op = s; }
       }
       if (prec == 0 || prec <= min_prec) return lhs;
-      p++;
+      p += width;
       ExpressionPlan rhs = expr(prec);
       lhs = ExpressionPlan::binary(std::move(lhs), op, std::move(rhs));   // op: format!("{}", op), plan_parser.rs:241-247
     }

@@ -91,6 +91,10 @@ struct fq_launch_params {
                               // compiled for one or the other), or null when the column is NOT NULL
   fq_u64 cols_valid_bit0[8];  // bitmap validity: bit of row 0 of the source
   fq_u64 numbers_begin;  // generated mode: column 0 = numbers_begin + row
+  // bit tables of the pipe's FQ_EXPR_LOOKUP nodes (FQ_MAX_LOOKUPS slots): LSB-first bitmaps, read a byte at a time so that a
+  // table needs no alignment and no padding past its last byte; the row functions (pred, consume, gb_row, emit) receive them here
+  const fq_u8 *lookup[4];
+  fq_u64 lookup_bits[4];
   // aggregate
   fq_u64 *partials;      // [gridDim.x][FQ_STATE_HDR + Q::NSLOTS]
   fq_u64 *state;         // [FQ_STATE_HDR + Q::NSLOTS] running state of the pipe
@@ -191,6 +195,11 @@ template <int V> __device__ __forceinline__ void fq_load_bits(bool (&dst)[V], co
       for (int v = 0; v < 8; v++) dst[8 * b + v] = (w >> v) & 1u;
     }
   }
+}
+
+// FQ_EXPR_LOOKUP: bit c of a bit table of n bits, false at or beyond n (the table of an empty dictionary has no bits)
+__device__ __forceinline__ bool fq_lookup(const fq_u8 *table, fq_u64 n, fq_u64 c) {
+  return c < n && ((__ldg(table + (c >> 3)) >> (c & 7)) & 1u);
 }
 
 // one value (scalar tails, ragged last tile)
@@ -667,7 +676,7 @@ __device__ __forceinline__ void fq_agg_kernel(const fq_launch_params &p) {
     for (int u = 0; u < UNROLL; u++) {
       fq_u32 kept = 0;
 #pragma unroll
-      for (int v = 0; v < V; v++) kept |= (Q::consume(acc, rows[u], v, nsel, err) ? 1u : 0u) << v;
+      for (int v = 0; v < V; v++) kept |= (Q::consume(p, acc, rows[u], v, nsel, err) ? 1u : 0u) << v;
       if constexpr (Q::TRACK_BLOCKS) {
         if (p.block_hit) fq_mark_blocks_warp<V>(p, (g0 + (fq_u64)u * blockDim.x) * V, kept);
       }
@@ -681,7 +690,7 @@ __device__ __forceinline__ void fq_agg_kernel(const fq_launch_params &p) {
     Q::load(r, p, g);
     fq_u32 kept = 0;
 #pragma unroll
-    for (int v = 0; v < V; v++) kept |= (Q::consume(acc, r, v, nsel, err) ? 1u : 0u) << v;
+    for (int v = 0; v < V; v++) kept |= (Q::consume(p, acc, r, v, nsel, err) ? 1u : 0u) << v;
     if constexpr (Q::TRACK_BLOCKS) {
       if (p.block_hit) fq_mark_blocks_lane<V>(p, g * V, kept);
     }
@@ -689,7 +698,7 @@ __device__ __forceinline__ void fq_agg_kernel(const fq_launch_params &p) {
   for (fq_u64 row = nvec * V + tid; row < p.n_rows; row += nthreads) {
     typename Q::Rows r;
     Q::load1(r, p, row);
-    const bool kept = Q::consume(acc, r, 0, nsel, err);
+    const bool kept = Q::consume(p, acc, r, 0, nsel, err);
     if constexpr (Q::TRACK_BLOCKS) {
       if (p.block_hit && kept) fq_mark_one(p.block_hit, row / FQ_REF_BLOCK_ROWS);
     }
@@ -838,7 +847,7 @@ __device__ __forceinline__ void fq_agg_tma_kernel(const fq_launch_params &p) {
       for (int u = 0; u < U; u++) {
         fq_u32 kept = 0;
 #pragma unroll
-        for (int v = 0; v < V; v++) kept |= (Q::consume(acc, rows[u], v, nsel, err) ? 1u : 0u) << v;
+        for (int v = 0; v < V; v++) kept |= (Q::consume(p, acc, rows[u], v, nsel, err) ? 1u : 0u) << v;
         if constexpr (Q::TRACK_BLOCKS) {
           if (p.block_hit) fq_mark_blocks_warp<V>(p, (t * tile_groups + (fq_u64)u * cthreads + threadIdx.x) * V, kept);
         }
@@ -855,7 +864,7 @@ __device__ __forceinline__ void fq_agg_tma_kernel(const fq_launch_params &p) {
       Q::load(r, p, g);
       fq_u32 kept = 0;
 #pragma unroll
-      for (int v = 0; v < V; v++) kept |= (Q::consume(acc, r, v, nsel, err) ? 1u : 0u) << v;
+      for (int v = 0; v < V; v++) kept |= (Q::consume(p, acc, r, v, nsel, err) ? 1u : 0u) << v;
       if constexpr (Q::TRACK_BLOCKS) {
         if (p.block_hit) fq_mark_blocks_lane<V>(p, g * V, kept);
       }
@@ -863,7 +872,7 @@ __device__ __forceinline__ void fq_agg_tma_kernel(const fq_launch_params &p) {
     for (fq_u64 row = nvec * V + ctid; row < p.n_rows; row += cn) {
       typename Q::Rows r;
       Q::load1(r, p, row);
-      const bool kept = Q::consume(acc, r, 0, nsel, err);
+      const bool kept = Q::consume(p, acc, r, 0, nsel, err);
       if constexpr (Q::TRACK_BLOCKS) {
         if (p.block_hit && kept) fq_mark_one(p.block_hit, row / FQ_REF_BLOCK_ROWS);
       }
@@ -948,7 +957,7 @@ __device__ __forceinline__ fq_u32 fq_tile_pred(const fq_launch_params &p, fq_u64
 #pragma unroll
     for (int u = 0; u < U; u++)
 #pragma unroll
-      for (int v = 0; v < V; v++) keep |= (Q::pred(rows[u], v, err) ? 1u : 0u) << (u * V + v);
+      for (int v = 0; v < V; v++) keep |= (Q::pred(p, rows[u], v, err) ? 1u : 0u) << (u * V + v);
   } else if (tile * tile_groups * V < p.n_rows) {
     const fq_u64 g0 = tile * tile_groups + (fq_u64)warp * 32 * U + lane;
 #pragma unroll
@@ -956,7 +965,7 @@ __device__ __forceinline__ fq_u32 fq_tile_pred(const fq_launch_params &p, fq_u64
       const fq_u64 row0 = (g0 + 32ull * u) * V;
 #pragma unroll
       for (int v = 0; v < V; v++)
-        if (row0 + v < p.n_rows) keep |= (Q::pred(rows[u], v, err) ? 1u : 0u) << (u * V + v);
+        if (row0 + v < p.n_rows) keep |= (Q::pred(p, rows[u], v, err) ? 1u : 0u) << (u * V + v);
     }
   }
   return keep;
@@ -1464,7 +1473,7 @@ __device__ __forceinline__ void fq_select_probe_kernel(const fq_launch_params &p
       typename Q::Rows r;
       Q::load_pred(r, p, g0 + g);
 #pragma unroll
-      for (int v = 0; v < V; v++) kept += Q::pred(r, v, err) ? 1u : 0u;
+      for (int v = 0; v < V; v++) kept += Q::pred(p, r, v, err) ? 1u : 0u;
       sampled += V;
     }
   }
@@ -1672,7 +1681,7 @@ __device__ __forceinline__ void fq_select_tma_kernel(const fq_launch_params &p) 
 #pragma unroll
           for (int u = 0; u < U; u++)
 #pragma unroll
-            for (int v = 0; v < V; v++) keep |= (Q::pred(rows[u], v, err) ? 1u : 0u) << (u * V + v);
+            for (int v = 0; v < V; v++) keep |= (Q::pred(p, rows[u], v, err) ? 1u : 0u) << (u * V + v);
           __syncwarp();
           if (lane == 0) fq_mbar_arrive(fq_smem_addr(&s_bars[STAGES + slot]));
           if (++slot == stages) { slot = 0; round++; }
@@ -1873,7 +1882,7 @@ __device__ __forceinline__ void fq_gb_row(const fq_launch_params &p, fq_u64 *tke
                                           const typename Q::Rows &r, int v, fq_u32 &err, int &smem_try) {
   fq_u64 key = 0, val[Q::NSLOTS > 0 ? Q::NSLOTS : 1] = {};
   fq_u32 vmask = 0;
-  const bool live = Q::gb_row(r, v, err, key, val, vmask);
+  const bool live = Q::gb_row(p, r, v, err, key, val, vmask);
   fq_u64 st[Q::G];
   Q::gb_one(st, val, vmask);
   fq_gb_put<Q>(p, tkeys, tslots, skeys, sslots, s_used, key, st, live, smem_try);

@@ -13,6 +13,8 @@
 //   4. fq_dict_rank + fq_dict_codes: rank[id] = position in sorted order, codes[row] = rank[id of the row's slot].
 // fq_utf8_lens / fq_utf8_gather_bytes gather strings by row index (the sorted dictionary from the representative rows, and
 // result columns from codes); fq_utf8_bounds_kernel finds a literal's (lower, upper) bound in a sorted dictionary.
+// fq_utf8_like_kernel matches a LIKE pattern against every string of an array (over a dictionary: once per distinct string)
+// and writes one bit per row, which pipes read through an FQ_EXPR_LOOKUP node.
 #pragma once
 
 #define FQ_DICT_EMPTY 0xFFFFFFFFFFFFFFFFull   // hash32 = row = 0xFFFFFFFF cannot occur: rows are fewer than 2^32 - 1
@@ -165,6 +167,68 @@ __global__ void __launch_bounds__(256) fq_utf8_gather_bytes(const int *off, cons
     const unsigned char *s = data + off[rows[i]];
     unsigned char *d = out + out_off[i];
     for (fq_u32 b = lane; b < len; b += 32) d[b] = s[b];
+  }
+}
+
+// SQL LIKE, bytewise and case-sensitive: `%` = any run of characters (newlines included), `_` = one UTF-8 code point,
+// `\` makes the next pattern byte literal (the caller refuses a pattern that ends in an unpaired `\`).  Greedy matching that
+// keeps one backtrack point, the last `%` seen: when the text after it fails, that `%` swallows one more code point and the
+// rest of the pattern is tried again.  No recursion, O(len * plen) steps at worst.  Plain code, no intrinsics: the tests
+// compile this very function for the host.
+__device__ __forceinline__ bool fq_like_match(const unsigned char *s, fq_u32 len, const unsigned char *p, fq_u32 plen) {
+  fq_u32 i = 0, j = 0;
+  fq_u32 star_j = 0xFFFFFFFFu, star_i = 0;   // pattern position after the last `%`, text position it was resumed from
+  while (i < len) {
+    if (j < plen) {
+      const unsigned char c = p[j];
+      if (c == '%') {
+        star_j = ++j;
+        star_i = i;
+        continue;
+      }
+      if (c == '_') {   // one code point: the lead byte and its continuation bytes
+        i++;
+        while (i < len && (s[i] & 0xC0) == 0x80) i++;
+        j++;
+        continue;
+      }
+      const bool esc = c == '\\' && j + 1 < plen;
+      if (s[i] == (esc ? p[j + 1] : c)) {
+        i++;
+        j += esc ? 2 : 1;
+        continue;
+      }
+    }
+    if (star_j == 0xFFFFFFFFu) return false;
+    star_i++;   // the last `%` takes one more code point
+    while (star_i < len && (s[star_i] & 0xC0) == 0x80) star_i++;
+    i = star_i;
+    j = star_j;
+  }
+  while (j < plen && p[j] == '%') j++;
+  return j == plen;
+}
+
+// bit i of `bits` (LSB-first) = string i LIKE the pattern, xor `negate`; NULL rows and the padding of the last byte get 0.
+// One thread per string, one 32-bit word per warp from a ballot: no atomics.  The word is stored byte by byte where the
+// column is not 4-byte aligned or ends inside it (the column holds ceil(n / 8) bytes).
+__global__ void __launch_bounds__(256) fq_utf8_like_kernel(const int *off, const unsigned char *data, const fq_u8 *valid, fq_u64 n,
+                                                           const unsigned char *pat, fq_u32 plen, int negate, fq_u8 *bits) {
+  const unsigned lane = threadIdx.x & 31;
+  const fq_u64 n_words = (n + 31) / 32, n_bytes = (n + 7) / 8;
+  const bool aligned = ((unsigned long long)bits & 3) == 0;
+  for (fq_u64 w = ((fq_u64)blockIdx.x * blockDim.x + threadIdx.x) >> 5; w < n_words; w += ((fq_u64)gridDim.x * blockDim.x) >> 5) {
+    const fq_u64 i = w * 32 + lane;
+    bool hit = false;
+    if (i < n && (!valid || valid[i])) hit = fq_like_match(data + off[i], (fq_u32)(off[i + 1] - off[i]), pat, plen) != (negate != 0);
+    const fq_u32 word = __ballot_sync(0xffffffffu, hit);
+    if (lane == 0) {
+      if (aligned && 4 * w + 4 <= n_bytes) {
+        reinterpret_cast<fq_u32 *>(bits)[w] = word;
+      } else {
+        for (fq_u64 b = 4 * w; b < 4 * w + 4 && b < n_bytes; b++) bits[b] = (fq_u8)(word >> (8 * (b - 4 * w)));
+      }
+    }
   }
 }
 

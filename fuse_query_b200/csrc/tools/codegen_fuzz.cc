@@ -31,8 +31,9 @@ int main(int argc, char **argv) {
     std::vector<fq_expr_node> nodes((size_t)n);
     for (int i = 0; i < n; i++) {
       fq_expr_node &x = nodes[(size_t)i];
-      x.kind = wild ? pick(-1, 8) : pick(FQ_EXPR_ALIAS, FQ_EXPR_AGGREGATOR);
+      x.kind = wild ? pick(-1, 9) : pick(FQ_EXPR_ALIAS, FQ_EXPR_LOOKUP);
       x.op = wild ? pick(-1, 9) : pick(0, 4);
+      if (x.kind == FQ_EXPR_LOOKUP && !wild) x.op = pick(0, 4) ? pick(0, FQ_MAX_LOOKUPS - 1) : pick(-2, FQ_MAX_LOOKUPS + 2);   // slots, a few out of range
       // children mostly point backwards (a DAG), sometimes anywhere (cycles, self references, out of range)
       x.left = pick(0, 9) ? (i ? pick(0, i - 1) : -1) : pick(-3, n + 2);
       x.right = pick(0, 9) ? (i ? pick(0, i - 1) : -1) : pick(-3, n + 2);

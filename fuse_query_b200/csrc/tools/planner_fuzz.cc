@@ -21,18 +21,18 @@ int main(int argc, char **argv) {
       "select", "from", "where", "limit", "group", "by", "as", "and", "or", "not", "explain", "system", ".", "numbers_mt", "number",
       "(", ")", ",", "*", "+", "-", "/", "%", "=", "<", ">", "<=", ">=", "<>", "!=", "1", "0", "10000", "1.5", "'a'", "sum", "count",
       "max", "min", "avg", "x", "t", ";", "having", "order", "asc", "desc", "join", "union", "-1", "1e10", "99999999999999999999", "\"q\"", "`b`",
-      "'", "''", "\\", "/*", "--", "\t", "\n", "0x10", "1.", ".5", "e", "1e", "select(", "))", "((", "system.numbers_mt(10)"};
+      "'", "''", "\\", "/*", "--", "\t", "\n", "0x10", "1.", ".5", "e", "1e", "select(", "))", "((", "system.numbers_mt(10)", "like", "'%a_'", "'\\'"};
   auto pick = [&](size_t n) { return (size_t)(rng() % n); };
   // a grammar-shaped generator beside the token soup, so that the optimizer, EXPLAIN and the pipeline builder see plans too
   std::function<std::string(int)> expr = [&](int depth) -> std::string {
     static const char *leaf[] = {"number", "1", "0", "2.5", "'s'", "x", "c1", "10000"};
-    static const char *ops[] = {"+", "-", "*", "/", "=", "<", ">", "<=", ">=", "and", "or", "%", "<>"};
+    static const char *ops[] = {"+", "-", "*", "/", "=", "<", ">", "<=", ">=", "and", "or", "%", "<>", "like", "not like"};
     static const char *fns[] = {"sum", "count", "max", "min", "avg", "nosuch"};
     if (depth <= 0 || pick(3) == 0) return leaf[pick(8)];
     switch (pick(4)) {
       case 0: return "(" + expr(depth - 1) + ")";
       case 1: return std::string(fns[pick(6)]) + "(" + expr(depth - 1) + ")";
-      default: return expr(depth - 1) + " " + ops[pick(13)] + " " + expr(depth - 1);
+      default: return expr(depth - 1) + " " + ops[pick(15)] + " " + expr(depth - 1);
     }
   };
   std::function<std::string(int)> query = [&](int nest) -> std::string {

@@ -69,7 +69,10 @@ enum {
   FQ_EXPR_ARITHMETIC = 3, /* function_arithmetic.rs: op in FQ_AR_* */
   FQ_EXPR_COMPARISON = 4, /* function_comparison.rs: op in FQ_CMP_* */
   FQ_EXPR_LOGIC = 5,      /* function_logic.rs: op in FQ_LG_* */
-  FQ_EXPR_AGGREGATOR = 6  /* function_aggregator.rs: op in FQ_AGG_*, argument in `left` */
+  FQ_EXPR_AGGREGATOR = 6, /* function_aggregator.rs: op in FQ_AGG_*, argument in `left` */
+  FQ_EXPR_LOOKUP = 7      /* Boolean: bit `left` of the bit table bound to slot `op` (fq_pipe_set_lookup); `left` is an unsigned
+                             integer expression (normally a dictionary codes column) and not a constant, op in
+                             [0, FQ_MAX_LOOKUPS); a value at or beyond the table's bit count gives false; NULL where `left` is */
 };
 
 typedef union fq_scalar_bits {
@@ -80,7 +83,7 @@ typedef union fq_scalar_bits {
 
 typedef struct fq_expr_node {
   int32_t kind;   /* FQ_EXPR_* */
-  int32_t op;     /* operator for ARITHMETIC / COMPARISON / LOGIC / AGGREGATOR */
+  int32_t op;     /* operator for ARITHMETIC / COMPARISON / LOGIC / AGGREGATOR, slot for LOOKUP */
   int32_t left;   /* child index or -1 */
   int32_t right;  /* child index or -1 */
   int32_t column; /* FIELD: index into the pipe's input columns */
@@ -210,6 +213,17 @@ fq_status fq_utf8_dict_encode(fq_ctx *ctx, const fq_utf8 *src, fq_column *codes,
 /* lower = the first index of the sorted array `dict` whose string is >= the literal, upper = the first one > it.  Waits. */
 fq_status fq_utf8_bounds(fq_ctx *ctx, const fq_utf8 *dict, const void *scalar, uint64_t scalar_len, uint64_t *lower, uint64_t *upper,
                          void *stream);
+/* SQL LIKE against one pattern: bit i of `bits` (an FQ_U8 column of at least ceil(len(a) / 8) bytes, LSB-first like Arrow's
+ * bitmaps) = a[i] LIKE pattern, negated when `negate` is set (NOT LIKE); NULL rows get bit 0 in both cases, the caller keeps
+ * a's validity.  `%` matches any run of characters (newlines included), `_` one character (one UTF-8 code point), `\` makes
+ * the next pattern character literal (`\%`, `\_`, `\\`); there is no ESCAPE clause.  Matching is bytewise and case-sensitive,
+ * the equality fq_utf8_compare uses.  A pattern that ends in an unpaired `\` is FQ_ERR_INVALID.  Waits for the result.
+ * Over a dictionary the pattern is matched once per distinct string, and a Utf8 column `s` with codes `c` lowers to
+ *   s LIKE 'p'              (lookup k c)  with slot k bound to fq_utf8_like(dict, 'p', 0)   (FQ_EXPR_LOOKUP)
+ *   s NOT LIKE 'p'          (lookup k c)  with slot k bound to fq_utf8_like(dict, 'p', 1)
+ * so the pipe's generated source depends on the slot, not on the pattern: one compiled pipe serves every pattern. */
+fq_status fq_utf8_like(fq_ctx *ctx, const fq_utf8 *a, const void *pattern, uint64_t pattern_len, int32_t negate, fq_column *bits,
+                       void *stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Source — system.numbers_mt shards.  Replaces NumbersStream::poll_next materialising 10 000-row
@@ -235,6 +249,8 @@ typedef struct fq_source {
 #define FQ_MAX_COLS 8
 #define FQ_MAX_EXPRS 8
 #define FQ_MAX_KEYS 4
+/* bit tables one pipe reads through FQ_EXPR_LOOKUP nodes */
+#define FQ_MAX_LOOKUPS 4
 
 enum { FQ_PIPE_PROJECT = 0, FQ_PIPE_AGGREGATE = 1, FQ_PIPE_GROUPBY = 2 };
 
@@ -264,6 +280,10 @@ void fq_pipe_destroy(fq_ctx *ctx, fq_pipe *pipe);
  * comes from FQ_AGG_VARIANT / FQ_SEL_VARIANT / FQ_MAP_VARIANT, read once when the pipe is compiled (never on the launch path);
  * another word is FQ_ERR_INVALID, there and here.  A variant the pipe's module does not hold falls back to one it does. */
 fq_status fq_pipe_set_variant(fq_ctx *ctx, fq_pipe *pipe, const char *variant);
+/* Binds bit table `slot` of the pipe's FQ_EXPR_LOOKUP nodes: `bits` is an FQ_U8 column holding at least ceil(n_bits / 8) bytes,
+ * LSB-first (fq_utf8_like writes one).  Borrowed: it must outlive the launches that follow, which read it; binding the slot
+ * again replaces it for later launches.  A launch of a pipe with an unbound slot is FQ_ERR_INVALID. */
+fq_status fq_pipe_set_lookup(fq_ctx *ctx, fq_pipe *pipe, int32_t slot, const fq_column *bits, uint64_t n_bits);
 /* 1 if the kernel came from the library's precompiled table, 0 if NVRTC built it */
 int32_t fq_pipe_is_precompiled(const fq_pipe *pipe);
 /* where the pipe's kernels came from: 0 = the library's precompiled table, 1 = built by NVRTC in this process,
@@ -429,7 +449,8 @@ fq_status fq_column_take(fq_ctx *ctx, const fq_column *src, const fq_column *row
  *   for every execution: fq_graph_launch(ctx, g, stream);  fq_pipe_fetch_*(...) as after a direct launch.
  * Sources, output columns, limits and flags are frozen as recorded.  Between begin and end nothing runs; only launches
  * on `stream` belong to the recording, one recording at a time per context.  A pipe with a group attached is refused
- * (its merge carries an epoch that advances with every execution). */
+ * (its merge carries an epoch that advances with every execution).  Lookup tables (fq_pipe_set_lookup) are frozen too: a
+ * replay reads the tables that were bound when the launch was recorded, whatever is bound to the pipe since. */
 typedef struct fq_graph fq_graph;
 fq_status fq_graph_begin(fq_ctx *ctx, void *stream);
 fq_status fq_graph_end(fq_ctx *ctx, void *stream, fq_graph **out);

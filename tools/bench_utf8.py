@@ -1,8 +1,9 @@
 """Utf8 columns on the device: dictionary-encoding throughput, string queries against the same queries over a plain UInt32
-column holding the codes, and pyarrow on the host CPU as a baseline.  Writes <out>/r03_utf8_<rows>.json with the GPU's
-name and power limit.
+column holding the codes, LIKE queries against `s = '...'` on the same column, fq_utf8_like over dictionaries, and pyarrow
+on the host CPU as a baseline.  Writes <out>/r03_utf8_<rows>.json (or r04_like_<rows>.json for --sections like) with the
+GPU's name and power limit.
 
-    python tools/bench_utf8.py [--rows 100000000] [--out profiles]
+    python tools/bench_utf8.py [--rows 100000000] [--out profiles] [--sections encode,queries,like]
 """
 import argparse
 import ctypes as C
@@ -123,6 +124,61 @@ def query_cases(rows, distinct, rng, reps):
     return {"rows": rows, "distinct": distinct, "queries": out, "pyarrow_host_seconds": base}
 
 
+def alternate(fctx, qa, qb, reps):
+    """median seconds of two queries, run in turn so that drift on a shared host hits both alike"""
+    ta, tb = [], []
+    for _ in range(2):   # warm-up both (module loads, the pattern's bit table)
+        h.execute_sql(fctx, qa), h.execute_sql(fctx, qb)
+    for _ in range(reps):
+        t0 = time.perf_counter(); h.execute_sql(fctx, qa); ta.append(time.perf_counter() - t0)
+        t0 = time.perf_counter(); h.execute_sql(fctx, qb); tb.append(time.perf_counter() - t0)
+    return float(np.median(ta)), float(np.median(tb)), [round(t, 6) for t in ta], [round(t, 6) for t in tb]
+
+
+def like_cases(rows, distinct, rng, reps):
+    """LIKE and NOT LIKE over the Utf8 column s of the query table, each beside `s = '...'` over the same column; the matching
+    kernel alone over sorted dictionaries of 10^4, 10^6 and 10^8 distinct 16-byte strings; pyarrow match_like on the host"""
+    import pyarrow as pa
+    import pyarrow.compute as pc
+    values = rng.integers(0, distinct, rows)
+    offsets, data = strings(values, 16)
+    x = rng.integers(0, 1000, rows).astype(np.uint64)
+    gpu = h.GpuContext.create(0)
+    fctx = h.FuseQueryContext.create_ctx(8, gpu)
+    s = h.DataArray.from_utf8(gpu, offsets, data.tobytes(), None)
+    schema = h.DataSchema([h.DataField("s", h.DataType.Utf8, False), h.DataField("x", h.DataType.UInt64, False)])
+    ds = fctx.datasource()
+    ds.add_database("b")
+    ds.add_table("b", h.MemoryTable("b", "t", schema, [s, h.DataArray.from_numpy(gpu, x)]))
+    lit = f"{distinct // 2:016d}"
+    eq = f"select count(x) from b.t where s = '{lit}'"
+    queries = {"prefix": "select count(x) from b.t where s like '00000000000042%'",
+               "infix": "select count(x) from b.t where s like '%42%'",
+               "not_like": "select count(x) from b.t where s not like '%42%'"}
+    out = {}
+    for name, q in queries.items():
+        tl, te, al, ae = alternate(fctx, q, eq, reps)
+        out[name] = {"like_sql": q, "eq_sql": eq, "like_seconds": tl, "eq_seconds": te, "like_over_eq": tl / te, "like_all": al, "eq_all": ae,
+                     "rows": rows, "result": h.execute_sql(fctx, q)[0].column(0).to_list()[0]}
+    arr = pa.Array.from_buffers(pa.string(), rows, [None, pa.py_buffer(offsets), pa.py_buffer(data)])
+    base = {}
+    for name, pat in (("prefix", "00000000000042%"), ("infix", "%42%")):
+        t0 = time.perf_counter(); pc.sum(pc.match_like(arr, pat)).as_py(); base[name] = time.perf_counter() - t0
+    kernel = []
+    ctx = cabi.Context(0)
+    for d in (10**4, 10**6, 10**8):
+        offs, dat = strings(np.arange(d), 16)   # zero-padded decimals: already in bytewise order, a dictionary as fq_utf8_dict_encode leaves it
+        dictionary = device_utf8(ctx, offs, dat)
+        for pat in ("%42%", "00000000000042%"):
+            sec, all_t = median_time(lambda: dictionary.like(pat).free(), reps)
+            kernel.append({"distinct": d, "pattern": pat, "seconds": sec, "all_seconds": all_t, "strings_per_s": d / sec,
+                           "bytes_read": d * (16 + 4), "GBps": d * 20 / sec / 1e9})
+            print(json.dumps(kernel[-1]), flush=True)
+        dictionary.free()
+    ctx.close()
+    return {"rows": rows, "distinct": distinct, "queries": out, "fq_utf8_like": kernel, "pyarrow_match_like_host_seconds": base}
+
+
 def device_info():
     import torch
     info = {"gpu": torch.cuda.get_device_name(0)}
@@ -141,10 +197,22 @@ def main():
     ap.add_argument("--prefix-rows", type=int, default=20_000_000, help="rows of the 100-byte case (int32 offsets: at most 2 GiB of bytes)")
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--out", default="profiles")
+    ap.add_argument("--sections", default="encode,queries", help="comma-separated: encode, queries, like")
     a = ap.parse_args()
+    sections = a.sections.split(",")
     rng = np.random.default_rng(2026)
-    ctx = cabi.Context(0)
     res = {"device": device_info(), "encode": [], "note": "seconds are host wall time around calls that end with a device synchronise"}
+    if "like" in sections:
+        res["like"] = like_cases(a.rows, 10**4, rng, max(a.reps, 5))
+        print(json.dumps(res["like"]["queries"]), flush=True)
+    if sections == ["like"]:
+        os.makedirs(a.out, exist_ok=True)
+        path = os.path.join(a.out, f"r04_like_{a.rows}.json")
+        with open(path, "w") as f:
+            json.dump(res, f, indent=1)
+        print("wrote", path)
+        return
+    ctx = cabi.Context(0)
     for distinct in (10, 10**4, 10**6, a.rows):
         res["encode"].append(encode_case(ctx, a.rows, distinct, 16, b"", rng, a.reps))
         print(json.dumps(res["encode"][-1]), flush=True)
