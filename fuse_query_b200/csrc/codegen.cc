@@ -440,10 +440,11 @@ int generate(const fq_pipe_desc &d, Generated *out, std::string *err) {
       out->key_shift.push_back(ki.shift);
       out->key_bits.push_back(ki.bits);
     }
-    if (shift > 64) {
-      *err = fmt("Unsupported on the device path: GROUP BY keys of %d bits (values plus one bit per nullable key) do not pack into 64", shift);
+    if (shift > 128) {
+      *err = fmt("Unsupported on the device path: GROUP BY keys of %d bits (values plus one bit per nullable key) do not pack into 64 or 128", shift);
       return FQ_ERR_UNSUPPORTED;
     }
+    out->key_words = shift > 64 ? 2 : 1;
   }
 
   std::set<int> aggs;
@@ -692,12 +693,14 @@ int generate(const fq_pipe_desc &d, Generated *out, std::string *err) {
     const int n = n_leaves;
     auto is_f = [&](int k) { return is_float(out->agg_dtypes[k]); };
     auto is_s = [&](int k) { return is_signed_int(out->agg_dtypes[k]); };
+    const bool wide = out->key_words == 2;
     s += fmt("  static constexpr int G = %d;\n", 1 + n_slots);
-    s += "  __device__ static __forceinline__ bool gb_row(const fq_launch_params &p, const Rows &r, int v, fq_u32 &err, fq_u64 &key, fq_u64 (&val)[NSLOTS > 0 ? NSLOTS : 1], fq_u32 &vmask) {\n";
+    s += wide ? "  using Key = fq_gb_key2;\n" : "  using Key = fq_u64;\n";
+    s += "  __device__ static __forceinline__ bool gb_row(const fq_launch_params &p, const Rows &r, int v, fq_u32 &err, Key &key, fq_u64 (&val)[NSLOTS > 0 ? NSLOTS : 1], fq_u32 &vmask) {\n";
     if (out->has_pred) s += "    if (!pred(p, r, v, err)) return false;\n";
     {
       Gen::Emitter e(g, "    ");
-      std::string st = "    key = 0ull;\n    vmask = 0u;\n";
+      std::string st = wide ? "    key.lo = 0ull;\n    key.hi = 0ull;\n    vmask = 0u;\n" : "    key = 0ull;\n    vmask = 0u;\n";
       for (const KeyInfo &ki : keys) {
         e.node(ki.node);
         std::string bits;
@@ -708,8 +711,21 @@ int generate(const fq_pipe_desc &d, Generated *out, std::string *err) {
           case FQ_BOOL: bits = "(fq_u64)((" + x + ") ? 1u : 0u)"; break;
           default: bits = fmt("(fq_u64)(fq_traits<%s>::unsigned_t)(", ctype(ki.t)) + x + ")";
         }
-        if (ki.nullable) st += fmt("    key |= (%s) ? (%s << %d) : (1ull << %d);\n", e.ok[ki.node].c_str(), bits.c_str(), ki.shift, ki.shift + ki.bits);
-        else st += fmt("    key |= %s << %d;\n", bits.c_str(), ki.shift);
+        if (!wide) {
+          if (ki.nullable) st += fmt("    key |= (%s) ? (%s << %d) : (1ull << %d);\n", e.ok[ki.node].c_str(), bits.c_str(), ki.shift, ki.shift + ki.bits);
+          else st += fmt("    key |= %s << %d;\n", bits.c_str(), ki.shift);
+          continue;
+        }
+        // two words: the field's value bits at [shift, shift + bits), which may straddle lo / hi, then its null flag
+        const std::string b = ki.nullable ? fmt("((%s) ? %s : 0ull)", e.ok[ki.node].c_str(), bits.c_str()) : bits;
+        st += "    {\n      const fq_u64 b = " + b + ";\n";
+        if (ki.shift < 64) st += fmt("      key.lo |= b << %d;\n", ki.shift);
+        if (ki.shift + ki.bits > 64) st += ki.shift < 64 ? fmt("      key.hi |= b >> %d;\n", 64 - ki.shift) : fmt("      key.hi |= b << %d;\n", ki.shift - 64);
+        if (ki.nullable) {
+          const int f = ki.shift + ki.bits;
+          st += fmt("      key.%s |= (%s) ? 0ull : (1ull << %d);\n", f < 64 ? "lo" : "hi", e.ok[ki.node].c_str(), f < 64 ? f : f - 64);
+        }
+        st += "    }\n";
       }
       for (int k = 0; k < n; k++) {
         const fq_expr_node &an = d.nodes[out->agg_nodes[k]];

@@ -35,9 +35,11 @@ struct Generated {
   std::vector<fq_dtype> expr_dtypes;    // Function::return_type
   std::vector<int> expr_nullable;       // projection pipes: can select expression i yield NULL?
   std::vector<fq_dtype> node_dtypes;    // per node, FQ_NULL when not reachable
-  // GROUP BY pipes: how the key expressions pack into the 64-bit table key, lowest bits first
+  // GROUP BY pipes: how the key expressions pack into the table key of key_words 64-bit words (lo, then hi), lowest bits
+  // first; a field may straddle the two words
   std::vector<fq_dtype> key_dtypes;
   std::vector<int> key_nullable, key_shift, key_bits;   // per key: can it be NULL, first bit, value bits (the null flag sits above them)
+  int key_words = 1;                    // 1: keys of up to 64 bits (Q::Key = fq_u64), 2: 65..128 bits (Q::Key = fq_gb_key2)
   bool tma_ok = false;                  // every referenced column is materialised: the bulk-copy staged kernel exists
   bool sel_tma_ok = false;              // ... and the predicate reads at least one column: the staged select kernel exists
   bool track_blocks = false;            // aggregate pipe with a predicate and a Sum leaf: reference-block tracking compiled in

@@ -227,8 +227,8 @@ void plan_kernels(const fq::Generated &gen, Kernel *k, unsigned *gb_smem_cap) {
   };
   const unsigned tma_rows = (unsigned)s.tma_threads * s.tma_unroll * V;
   if (gen.kind == FQ_PIPE_GROUPBY) {
-    // shared-memory table of the CTA: the largest power of two of (key + state) slots within 96 KB (two CTAs per SM)
-    const unsigned entry = 8u * (2u + (unsigned)gen.n_slots);
+    // shared-memory table of the CTA: the largest power of two of (key words + state) slots within 96 KB (two CTAs per SM)
+    const unsigned entry = 8u * ((unsigned)gen.key_words + 1u + (unsigned)gen.n_slots);
     unsigned cap = 1;
     while (cap * 2 * entry <= 96u * 1024u) cap *= 2;
     static const int smem_env = getenv("FQ_GB_SMEM_SLOTS") ? atoi(getenv("FQ_GB_SMEM_SLOTS")) : -1;
@@ -1594,18 +1594,24 @@ fq_status fq_pipe_fetch_limit_row(fq_ctx *ctx, fq_pipe *pipe, uint64_t *row) {
 // GROUP BY pipes (hash aggregation)
 // =============================================================================================
 namespace {
-__global__ void __launch_bounds__(256) fq_gb_fill(fq_u64 *keys, fq_u64 *slots, fq_u64 n_entries, int G, const fq_u64 *identity) {
+// The host-compiled kernels below serve every GROUP BY pipe: `kw` is its key width in 64-bit words (Generated::key_words),
+// and key i of a table is words [i * kw, i * kw + kw) of its key array.
+__global__ void __launch_bounds__(256) fq_gb_fill(fq_u64 *keys, int kw, fq_u64 *slots, fq_u64 n_entries, int G, const fq_u64 *identity) {
   const fq_u64 tid = (fq_u64)blockIdx.x * blockDim.x + threadIdx.x, nthreads = (fq_u64)gridDim.x * blockDim.x;
-  for (fq_u64 i = tid; i < n_entries; i += nthreads) keys[i] = FQ_GB_EMPTY;
+  for (fq_u64 i = tid; i < n_entries * (fq_u64)kw; i += nthreads) keys[i] = FQ_GB_EMPTY;
   for (fq_u64 i = tid; i < n_entries * (fq_u64)G; i += nthreads) slots[i] = identity[i % (fq_u64)G];
 }
-__device__ __forceinline__ bool fq_gb_occupied(const fq_u64 *keys, fq_u64 cap, const fq_u32 *flags, fq_u64 i) {
-  return i < cap ? keys[i] != FQ_GB_EMPTY : (i == cap && flags[1] != 0);
+// the words of key i: hi = 0 for one-word keys
+__device__ __forceinline__ fq_gb_key2 fq_gb_key_at(const fq_u64 *keys, int kw, fq_u64 i) {
+  return {keys[i * kw], kw == 2 ? keys[i * kw + 1] : 0ull};
 }
-__global__ void __launch_bounds__(256) fq_gb_count(const fq_u64 *keys, fq_u64 cap, fq_u32 *flags) {
+__device__ __forceinline__ bool fq_gb_occupied(const fq_u64 *keys, int kw, fq_u64 cap, const fq_u32 *flags, fq_u64 i) {
+  return i < cap ? keys[i * kw] != FQ_GB_EMPTY || (kw == 2 && keys[i * kw + 1] != FQ_GB_EMPTY) : (i == cap && flags[1] != 0);
+}
+__global__ void __launch_bounds__(256) fq_gb_count(const fq_u64 *keys, int kw, fq_u64 cap, fq_u32 *flags) {
   const fq_u64 tid = (fq_u64)blockIdx.x * blockDim.x + threadIdx.x, nthreads = (fq_u64)gridDim.x * blockDim.x;
   fq_u64 n = 0;
-  for (fq_u64 i = tid; i <= cap; i += nthreads) n += fq_gb_occupied(keys, cap, flags, i) ? 1 : 0;
+  for (fq_u64 i = tid; i <= cap; i += nthreads) n += fq_gb_occupied(keys, kw, cap, flags, i) ? 1 : 0;
   for (int m = 16; m > 0; m >>= 1) n += __shfl_xor_sync(0xffffffffu, n, m);
   if ((threadIdx.x & 31) == 0 && n) atomicAdd((unsigned long long *)(flags + 2), (unsigned long long)n);
 }
@@ -1613,7 +1619,7 @@ struct fq_gb_export_params {
   const fq_u64 *keys, *slots;
   fq_u64 cap;
   const fq_u32 *flags;
-  int G, n_keys, n_leaves;
+  int kw, G, n_keys, n_leaves;
   int key_shift[FQ_MAX_KEYS], key_bits[FQ_MAX_KEYS], key_nullable[FQ_MAX_KEYS];
   void *key_out[FQ_MAX_KEYS], *key_valid[FQ_MAX_KEYS];
   int leaf_op[16], leaf_dtype[16], leaf_count_slot[16];
@@ -1635,7 +1641,7 @@ __global__ void __launch_bounds__(256) fq_gb_export(const __grid_constant__ fq_g
   const fq_u64 rounds = (a.cap + 1 + nthreads - 1) / nthreads;
   for (fq_u64 k = 0; k < rounds; k++) {
     const fq_u64 i = k * nthreads + tid;
-    const bool occ = i <= a.cap && fq_gb_occupied(a.keys, a.cap, a.flags, i);
+    const bool occ = i <= a.cap && fq_gb_occupied(a.keys, a.kw, a.cap, a.flags, i);
     const fq_u32 m = __ballot_sync(0xffffffffu, occ);
     if (!m) continue;
     fq_u64 base = 0;
@@ -1644,11 +1650,14 @@ __global__ void __launch_bounds__(256) fq_gb_export(const __grid_constant__ fq_g
     if (!occ) continue;
     const fq_u64 pos = base + __popc(m & ((1u << lane) - 1u));
     if (pos >= a.capacity) continue;
-    const fq_u64 key = i < a.cap ? a.keys[i] : FQ_GB_EMPTY;
+    const fq_gb_key2 key = i < a.cap ? fq_gb_key_at(a.keys, a.kw, i) : fq_gb_key2{FQ_GB_EMPTY, FQ_GB_EMPTY};
     for (int j = 0; j < a.n_keys; j++) {
-      const fq_u64 bits = a.key_bits[j] >= 64 ? key : ((key >> a.key_shift[j]) & ((1ull << a.key_bits[j]) - 1ull));
-      fq_store_low(a.key_out[j], pos, a.key_bits[j] / 8, bits);
-      if (a.key_nullable[j]) ((fq_u8 *)a.key_valid[j])[pos] = (fq_u8)(((key >> (a.key_shift[j] + a.key_bits[j])) & 1ull) ? 0 : 1);
+      // the field's value bits at [s, s + w), possibly across lo / hi, and its null flag at bit s + w
+      const int s = a.key_shift[j], w = a.key_bits[j], f = s + w;
+      fq_u64 bits = s >= 64 ? key.hi >> (s - 64) : s == 0 ? key.lo : (key.lo >> s) | (key.hi << (64 - s));
+      if (w < 64) bits &= (1ull << w) - 1ull;
+      fq_store_low(a.key_out[j], pos, w / 8, bits);
+      if (a.key_nullable[j]) ((fq_u8 *)a.key_valid[j])[pos] = (fq_u8)((((f >= 64 ? key.hi >> (f - 64) : key.lo >> f)) & 1ull) ? 0 : 1);
     }
     const fq_u64 *st = a.slots + i * (fq_u64)a.G;
     for (int l = 0; l < a.n_leaves; l++) {
@@ -1666,7 +1675,7 @@ __global__ void __launch_bounds__(256) fq_gb_export(const __grid_constant__ fq_g
   }
 }
 // partial groups ordered by owner rank: pass 0 counts (cursor[d] += ...), pass 1 writes entries at cursor positions
-__global__ void __launch_bounds__(256) fq_gb_partials(const fq_u64 *keys, const fq_u64 *slots, fq_u64 cap, const fq_u32 *flags, int G, int world,
+__global__ void __launch_bounds__(256) fq_gb_partials(const fq_u64 *keys, int kw, const fq_u64 *slots, fq_u64 cap, const fq_u32 *flags, int G, int world,
                                                       unsigned long long *cursor, fq_u64 *entries, int pass) {
   __shared__ fq_u32 cnt[8], base_lo[8];
   __shared__ unsigned long long base[8];
@@ -1677,18 +1686,21 @@ __global__ void __launch_bounds__(256) fq_gb_partials(const fq_u64 *keys, const 
     const fq_u64 i = (k * gridDim.x + blockIdx.x) * blockDim.x + threadIdx.x;
     if (threadIdx.x < 8) cnt[threadIdx.x] = 0;
     __syncthreads();
-    const bool occ = i <= cap && fq_gb_occupied(keys, cap, flags, i);
-    const fq_u64 key = occ && i < cap ? keys[i] : FQ_GB_EMPTY;
-    const int dest = (int)((fq_gb_hash(key) >> 40) % (fq_u64)world);
+    const bool occ = i <= cap && fq_gb_occupied(keys, kw, cap, flags, i);
+    const fq_gb_key2 key = occ && i < cap ? fq_gb_key_at(keys, kw, i) : fq_gb_key2{FQ_GB_EMPTY, kw == 2 ? FQ_GB_EMPTY : 0ull};
+    // the owner rank: the unseeded hash the pipe's first table uses, so every rank agrees whatever its own table's seed
+    const fq_u64 h = kw == 2 ? fq_gb_seeded(key, 0) : fq_gb_hash(key.lo);
+    const int dest = (int)((h >> 40) % (fq_u64)world);
     fq_u32 r = 0;
     if (occ) r = atomicAdd(&cnt[dest], 1u);
     __syncthreads();
     if ((int)threadIdx.x < world && cnt[threadIdx.x]) base[threadIdx.x] = atomicAdd(cursor + threadIdx.x, (unsigned long long)cnt[threadIdx.x]);
     __syncthreads();
     if (occ && pass == 1) {
-      fq_u64 *e = entries + (base[dest] + r) * (fq_u64)(1 + G);
-      e[0] = key;
-      for (int s = 0; s < G; s++) e[1 + s] = slots[i * (fq_u64)G + s];
+      fq_u64 *e = entries + (base[dest] + r) * (fq_u64)(kw + G);
+      e[0] = key.lo;
+      if (kw == 2) e[1] = key.hi;
+      for (int s = 0; s < G; s++) e[kw + s] = slots[i * (fq_u64)G + s];
     }
     __syncthreads();
   }
@@ -1729,13 +1741,14 @@ fq_status gb_clear(fq_ctx *ctx, fq_pipe *pipe, cudaStream_t s) {
   const int G = 1 + pipe->gen.n_slots;
   CUDA_TRY(cudaMemsetAsync(pipe->gb_flags, 0, 64, s));
   const unsigned grid = (unsigned)std::min<uint64_t>((pipe->gb_cap + 256) / 256, (uint64_t)ctx->sm_count * 8);
-  fq_gb_fill<<<grid, 256, 0, s>>>((fq_u64 *)pipe->gb_keys, (fq_u64 *)pipe->gb_slots, pipe->gb_cap + 1, G, (const fq_u64 *)pipe->gb_identity);
+  const int kw = pipe->gen.key_words;
+  fq_gb_fill<<<grid, 256, 0, s>>>((fq_u64 *)pipe->gb_keys, kw, (fq_u64 *)pipe->gb_slots, pipe->gb_cap + 1, G, (const fq_u64 *)pipe->gb_identity);
   CUDA_TRY(cudaGetLastError());
   ctx->launches++;
   if (pipe->gb_reps > 1 && pipe->gb_reps_dirty) {
     const uint64_t n = (pipe->gb_cap + 1) * (pipe->gb_reps - 1);
     const unsigned g2 = (unsigned)std::min<uint64_t>((n + 255) / 256, (uint64_t)ctx->sm_count * 8);
-    fq_gb_fill<<<g2, 256, 0, s>>>((fq_u64 *)pipe->gb_rep_keys, (fq_u64 *)pipe->gb_rep_slots, n, G, (const fq_u64 *)pipe->gb_identity);
+    fq_gb_fill<<<g2, 256, 0, s>>>((fq_u64 *)pipe->gb_rep_keys, kw, (fq_u64 *)pipe->gb_rep_slots, n, G, (const fq_u64 *)pipe->gb_identity);
     CUDA_TRY(cudaGetLastError());
     ctx->launches++;
     pipe->gb_reps_dirty = false;
@@ -1764,7 +1777,7 @@ fq_status fq_pipe_leaf_dtype(fq_ctx *, const fq_pipe *pipe, int32_t k, fq_dtype 
 fq_status fq_pipe_group_entry_slots(fq_ctx *, const fq_pipe *pipe, int32_t *slots) {
   if (fq_status st = gb_check(pipe)) return st;
   if (!slots) return set_err(FQ_ERR_INVALID, "Internal Error: null argument");
-  *slots = 2 + pipe->gen.n_slots;
+  *slots = pipe->gen.key_words + 1 + pipe->gen.n_slots;
   return FQ_OK;
 }
 
@@ -1773,7 +1786,7 @@ fq_status fq_pipe_groupby_reserve(fq_ctx *ctx, fq_pipe *pipe, uint64_t groups) {
   if (fq_status st = gb_check(pipe)) return st;
   uint64_t cap = 1024;
   while (cap < groups * 2 && cap < (1ull << 40)) cap *= 2;   // load factor <= 1/2
-  const int G = 1 + pipe->gen.n_slots;
+  const int G = 1 + pipe->gen.n_slots, kw = pipe->gen.key_words;
   // Replicas of a small table (CTA b aggregates into replica b % reps, folded into the table after the scan): as many as
   // fit FQ_GB_REPLICA_BYTES (default 32 MB, a quarter of L2), at most 32.  A table beyond that budget has enough slots that
   // the CTAs rarely meet on one line and stays single.
@@ -1782,7 +1795,7 @@ fq_status fq_pipe_groupby_reserve(fq_ctx *ctx, fq_pipe *pipe, uint64_t groups) {
   if (const char *e = getenv("FQ_GB_REPLICA_BYTES")) budget = strtoull(e, nullptr, 10);
   if (const char *e = getenv("FQ_GB_REPLICAS")) max_reps = (unsigned)std::max(1, atoi(e));
   unsigned reps = 1;
-  while (reps * 2 <= max_reps && (uint64_t)(reps * 2) * (cap + 1) * 8 * (1 + G) <= budget) reps *= 2;
+  while (reps * 2 <= max_reps && (uint64_t)(reps * 2) * (cap + 1) * 8 * (kw + G) <= budget) reps *= 2;
   if (cap != pipe->gb_cap || reps != pipe->gb_reps) {
     cudaFree(pipe->gb_keys);
     cudaFree(pipe->gb_slots);
@@ -1791,9 +1804,9 @@ fq_status fq_pipe_groupby_reserve(fq_ctx *ctx, fq_pipe *pipe, uint64_t groups) {
     pipe->gb_keys = pipe->gb_slots = pipe->gb_rep_keys = pipe->gb_rep_slots = nullptr;
     pipe->gb_cap = 0;
     pipe->gb_reps = 1;
-    cudaError_t e = cudaMalloc(&pipe->gb_keys, sizeof(uint64_t) * (cap + 1));
+    cudaError_t e = cudaMalloc(&pipe->gb_keys, sizeof(uint64_t) * kw * (cap + 1));
     if (e == cudaSuccess) e = cudaMalloc(&pipe->gb_slots, sizeof(uint64_t) * (cap + 1) * G);
-    if (e == cudaSuccess && reps > 1) e = cudaMalloc(&pipe->gb_rep_keys, sizeof(uint64_t) * (cap + 1) * (reps - 1));
+    if (e == cudaSuccess && reps > 1) e = cudaMalloc(&pipe->gb_rep_keys, sizeof(uint64_t) * kw * (cap + 1) * (reps - 1));
     if (e == cudaSuccess && reps > 1) e = cudaMalloc(&pipe->gb_rep_slots, sizeof(uint64_t) * (cap + 1) * G * (reps - 1));
     if (e != cudaSuccess) {
       cudaFree(pipe->gb_keys);
@@ -1828,7 +1841,7 @@ static fq_status gb_after_launch(fq_ctx *ctx, fq_pipe *pipe, cudaStream_t s) {
   // count the groups, mirror {overflow, count, error bits} to the host
   CUDA_TRY(cudaMemsetAsync(pipe->gb_flags + 2, 0, 8, s));
   const unsigned grid = (unsigned)std::min<uint64_t>((pipe->gb_cap + 256) / 256, (uint64_t)ctx->sm_count * 8);
-  fq_gb_count<<<grid, 256, 0, s>>>((const fq_u64 *)pipe->gb_keys, pipe->gb_cap, (fq_u32 *)pipe->gb_flags);
+  fq_gb_count<<<grid, 256, 0, s>>>((const fq_u64 *)pipe->gb_keys, pipe->gen.key_words, pipe->gb_cap, (fq_u32 *)pipe->gb_flags);
   CUDA_TRY(cudaGetLastError());
   ctx->launches++;
   CUDA_TRY(cudaMemcpyAsync(pipe->h_gb, pipe->gb_flags, 32, cudaMemcpyDeviceToHost, s));
@@ -1900,6 +1913,7 @@ fq_status fq_pipe_export_groups(fq_ctx *ctx, fq_pipe *pipe, fq_column *const *ke
   a.slots = (const fq_u64 *)pipe->gb_slots;
   a.cap = pipe->gb_cap;
   a.flags = (const fq_u32 *)pipe->gb_flags;
+  a.kw = gen.key_words;
   a.G = 1 + gen.n_slots;
   a.n_keys = (int)gen.key_dtypes.size();
   a.n_leaves = (int)gen.agg_nodes.size();
@@ -1948,18 +1962,18 @@ fq_status fq_pipe_export_partials(fq_ctx *ctx, fq_pipe *pipe, int32_t world, fq_
   if (!pipe->launched_groupby) return set_err(FQ_ERR_INVALID, "Internal Error: no GROUP BY launch to export");
   CUDA_TRY(cudaEventSynchronize(pipe->ev));
   const uint64_t n_groups = pipe->h_gb[1];
-  const int G = 1 + pipe->gen.n_slots;
-  if (!entries || entries->dtype != FQ_U64 || entries->len < n_groups * (uint64_t)(1 + G))
-    return set_err(FQ_ERR_INVALID, "Internal Error: the entries column must be UInt64 with groups x %d rows", 1 + G);
+  const int G = 1 + pipe->gen.n_slots, kw = pipe->gen.key_words;
+  if (!entries || entries->dtype != FQ_U64 || entries->len < n_groups * (uint64_t)(kw + G))
+    return set_err(FQ_ERR_INVALID, "Internal Error: the entries column must be UInt64 with groups x %d rows", kw + G);
   cudaStream_t s = (cudaStream_t)stream;
   unsigned long long *cursor = nullptr;
   CUDA_TRY(cudaMalloc(&cursor, 16 * sizeof(unsigned long long)));
   CUDA_TRY(cudaMemsetAsync(cursor, 0, 16 * sizeof(unsigned long long), s));
   const unsigned grid = (unsigned)std::min<uint64_t>((pipe->gb_cap + 256) / 256, (uint64_t)ctx->sm_count * 8);
-  fq_gb_partials<<<grid, 256, 0, s>>>((const fq_u64 *)pipe->gb_keys, (const fq_u64 *)pipe->gb_slots, pipe->gb_cap, (const fq_u32 *)pipe->gb_flags, G,
+  fq_gb_partials<<<grid, 256, 0, s>>>((const fq_u64 *)pipe->gb_keys, kw, (const fq_u64 *)pipe->gb_slots, pipe->gb_cap, (const fq_u32 *)pipe->gb_flags, G,
                                       world, cursor, nullptr, 0);
   fq_gb_prefix<<<1, 1, 0, s>>>(cursor, cursor + 8, world);
-  fq_gb_partials<<<grid, 256, 0, s>>>((const fq_u64 *)pipe->gb_keys, (const fq_u64 *)pipe->gb_slots, pipe->gb_cap, (const fq_u32 *)pipe->gb_flags, G,
+  fq_gb_partials<<<grid, 256, 0, s>>>((const fq_u64 *)pipe->gb_keys, kw, (const fq_u64 *)pipe->gb_slots, pipe->gb_cap, (const fq_u32 *)pipe->gb_flags, G,
                                       world, cursor, (fq_u64 *)entries->ptr, 1);
   CUDA_TRY(cudaGetLastError());
   ctx->launches += 3;
@@ -1975,9 +1989,9 @@ fq_status fq_pipe_merge_partials(fq_ctx *ctx, fq_pipe *pipe, const fq_column *en
   if (fq_status st = use(ctx)) return st;
   if (fq_status st = gb_check(pipe)) return st;
   if (!pipe->gb_cap) return set_err(FQ_ERR_INVALID, "Internal Error: fq_pipe_groupby_reserve was not called");
-  const int G = 1 + pipe->gen.n_slots;
-  if (n_entries && (!entries || entries->dtype != FQ_U64 || entries->len < n_entries * (uint64_t)(1 + G)))
-    return set_err(FQ_ERR_INVALID, "Internal Error: the entries column must be UInt64 with entries x %d rows", 1 + G);
+  const int G = 1 + pipe->gen.n_slots, kw = pipe->gen.key_words;
+  if (n_entries && (!entries || entries->dtype != FQ_U64 || entries->len < n_entries * (uint64_t)(kw + G)))
+    return set_err(FQ_ERR_INVALID, "Internal Error: the entries column must be UInt64 with entries x %d rows", kw + G);
   if (!(flags & FQ_RUN_ACCUMULATE) && pipe->launched_groupby) {
     if (fq_status st = gb_clear(ctx, pipe, (cudaStream_t)stream)) return st;
   }

@@ -120,12 +120,12 @@ struct fq_launch_params {
   fq_u64 *host_merged;     // behind the launch: a 10^7-row query is launch-latency bound and the copy cost as much as the kernel)
   fq_u32 group_rank, group_world, group_row_slots;
   // group by: open-addressing table in HBM, gb_cap (a power of two) slots + 1 for the key that equals the EMPTY mark
-  fq_u64 *gb_keys;        // [gb_cap + 1] packed keys, FQ_GB_EMPTY = free
+  fq_u64 *gb_keys;        // [gb_cap + 1] packed keys (Q::Key: one or two words), every word FQ_GB_EMPTY = free
   fq_u64 *gb_slots;       // [gb_cap + 1][Q::G] group states
   fq_u64 gb_cap;
   fq_u32 *gb_flags;       // [0] != 0: the table overflowed (results void), [1] != 0: the EMPTY-valued key occurred
   fq_u32 gb_smem_cap;     // slots of the CTA's shared-memory table (a power of two, 0 = none)
-  const fq_u64 *gb_entries;  // merge kernel: n_rows partial entries of 1 + Q::G slots each (packed key, state)
+  const fq_u64 *gb_entries;  // merge kernel: n_rows partial entries of KW + Q::G slots each (packed key's KW words, state)
   fq_u64 *gb_rep_keys;    // [gb_reps - 1][gb_cap + 1] replicas of the table: CTA b aggregates into replica b % gb_reps (0 = the
   fq_u64 *gb_rep_slots;   // table itself), the merge kernel folds them into the table and leaves them empty again
   fq_u32 gb_reps;         // >= 1
@@ -1744,8 +1744,9 @@ __device__ __forceinline__ void fq_select_tma_kernel(const fq_launch_params &p) 
 //
 // The reference plans GROUP BY but never executes it (pipeline_builder.rs:50-65 uses only aggr_expr); this is the
 // operator AggregatePlan{group_expr, aggr_expr} describes, with the aggregate protocol of function_aggregator.rs:57-100
-// applied per group.  Generated code (codegen.cc) supplies, per row, the 64-bit packed key and the encoded value of every
-// Aggregator leaf (Q::gb_row), and the atomics that fold a row / a partial state into a group's Q::G slots.
+// applied per group.  Generated code (codegen.cc) supplies, per row, the packed key (Q::Key: fq_u64 for keys of up to 64
+// bits, fq_gb_key2 for 65..128) and the encoded value of every Aggregator leaf (Q::gb_row), and the atomics that fold a row /
+// a partial state into a group's Q::G slots.
 // Two levels of open-addressing tables: every CTA aggregates into a table in shared memory first (gb_smem_cap slots, new
 // keys admitted until it is 3/4 full) — with few distinct keys nothing but the final flush leaves the SM; a row whose key
 // is not admitted there goes straight to the table in HBM (atomicCAS on the key, then atomics on the state).  At the end
@@ -1774,15 +1775,65 @@ __device__ __forceinline__ fq_u64 fq_gb_hash(fq_u64 k) {
   k ^= k >> 33;
   return k;
 }
+// hash of a 128-bit key under `seed`.  fq_gb_hash is a bijection, so two distinct keys with the same lo never collide, and
+// two with different lo collide only for particular seeds: the reseeded table after an overflow spreads a cluster again.
+// (A form such as hash(lo ^ hash(hi)) ^ seed would keep every collision under every seed.)
+__device__ __forceinline__ fq_u64 fq_gb_hash2(fq_u64 lo, fq_u64 hi, fq_u64 seed) {
+  return fq_gb_hash(hi ^ fq_gb_hash(lo ^ seed));
+}
+
+// The table key: one 8-byte word, or two for keys of 65..128 bits.  Either is claimed by ONE compare-and-swap (sm_100a has
+// a native 16-byte CAS in shared and global memory), so a slot goes from EMPTY to its key in one step and never changes
+// again.  The overloads below are the only code that knows the width; the fq_u64 ones are the expressions of the 64-bit
+// table, so its kernels compile as before.
+struct __align__(16) fq_gb_key2 {
+  fq_u64 lo, hi;
+};
+template <class K> __device__ __forceinline__ K fq_gb_empty();
+template <> __device__ __forceinline__ fq_u64 fq_gb_empty<fq_u64>() { return FQ_GB_EMPTY; }
+template <> __device__ __forceinline__ fq_gb_key2 fq_gb_empty<fq_gb_key2>() { return {FQ_GB_EMPTY, FQ_GB_EMPTY}; }
+__device__ __forceinline__ bool fq_gb_eq(fq_u64 a, fq_u64 b) { return a == b; }
+__device__ __forceinline__ bool fq_gb_eq(const fq_gb_key2 &a, const fq_gb_key2 &b) { return a.lo == b.lo && a.hi == b.hi; }
+__device__ __forceinline__ bool fq_gb_is_empty(fq_u64 k) { return k == FQ_GB_EMPTY; }
+__device__ __forceinline__ bool fq_gb_is_empty(const fq_gb_key2 &k) { return k.lo == FQ_GB_EMPTY && k.hi == FQ_GB_EMPTY; }
+__device__ __forceinline__ fq_u64 fq_gb_seeded(fq_u64 k, fq_u64 seed) { return fq_gb_hash(k ^ seed); }
+__device__ __forceinline__ fq_u64 fq_gb_seeded(const fq_gb_key2 &k, fq_u64 seed) { return fq_gb_hash2(k.lo, k.hi, seed); }
+// a key stored as words (a partial entry: the key's words, then the group state)
+__device__ __forceinline__ void fq_gb_from_words(fq_u64 &k, const fq_u64 *w) { k = w[0]; }
+__device__ __forceinline__ void fq_gb_from_words(fq_gb_key2 &k, const fq_u64 *w) {
+  k.lo = w[0];
+  k.hi = w[1];
+}
+// The look before the CAS.  A 16-byte look is two 8-byte loads and is NOT taken to be single-copy atomic: it can mix one
+// half of EMPTY (~0) with one half of a key being written, the looking lane's own key included, and skipping that as
+// "another key" would insert the key twice.  Slots only go from EMPTY to a key, so a look whose halves are both not ~0 is
+// the whole key and is trusted.  Any other look, a fully EMPTY one included, is "unsure": the lane CASes (EMPTY -> its
+// key) and decides on the value the CAS returns.  That costs one extra CAS only for real keys with an all-ones half.
+__device__ __forceinline__ fq_u64 fq_gb_look(const fq_u64 *k) { return fq_ld_volatile(k); }
+__device__ __forceinline__ fq_gb_key2 fq_gb_look(const fq_gb_key2 *k) { return {fq_ld_volatile(&k->lo), fq_ld_volatile(&k->hi)}; }
+__device__ __forceinline__ fq_u64 fq_gb_look_s(const fq_u64 *k) { return *(volatile fq_u64 *)k; }
+__device__ __forceinline__ fq_gb_key2 fq_gb_look_s(const fq_gb_key2 *k) {
+  const volatile fq_u64 *w = (const volatile fq_u64 *)k;
+  return {w[0], w[1]};
+}
+__device__ __forceinline__ bool fq_gb_unsure(fq_u64 k) { return k == FQ_GB_EMPTY; }
+__device__ __forceinline__ bool fq_gb_unsure(const fq_gb_key2 &k) { return k.lo == FQ_GB_EMPTY || k.hi == FQ_GB_EMPTY; }
+// EMPTY -> key in one atomic; returns what the slot held (EMPTY: the caller claimed it)
+__device__ __forceinline__ fq_u64 fq_gb_cas(fq_u64 *k, fq_u64 key) {
+  return atomicCAS((unsigned long long *)k, FQ_GB_EMPTY, (unsigned long long)key);
+}
+__device__ __forceinline__ fq_gb_key2 fq_gb_cas(fq_gb_key2 *k, const fq_gb_key2 &key) { return atomicCAS(k, fq_gb_empty<fq_gb_key2>(), key); }
+
 // slot of `key` in the HBM table (claimed on the spot when new); gb_cap for the key that equals the EMPTY mark; -1 = full
 // or not wanted.  Called by every lane that is active at the call site, `want` says which of them search.  The loop's exit
 // is a warp vote, so the lanes leave it together whatever their chain lengths: with an early `return slot` the compiler
 // threads each exit straight into the caller's atomics and they run once per distinct chain length (ncu: 25 instead of
 // 5 atomic instructions per 32 rows at 1000 keys).
-__device__ __forceinline__ fq_i64 fq_gb_find(const fq_launch_params &p, fq_u64 *tkeys, fq_u64 key, fq_u64 h, bool want) {
+template <class Key>
+__device__ __forceinline__ fq_i64 fq_gb_find(const fq_launch_params &p, Key *tkeys, Key key, fq_u64 h, bool want) {
   const fq_u32 warp = __activemask();
   fq_i64 slot = -1;
-  if (want && key == FQ_GB_EMPTY) {
+  if (fq_gb_is_empty(key) && want) {
     if (*(volatile fq_u32 *)(p.gb_flags + 1) == 0) p.gb_flags[1] = 1u;
     slot = (fq_i64)p.gb_cap;
     want = false;
@@ -1793,9 +1844,9 @@ __device__ __forceinline__ fq_i64 fq_gb_find(const fq_launch_params &p, fq_u64 *
   fq_u32 probe = 0;
   while (__any_sync(warp, want)) {
     if (want) {
-      fq_u64 cur = fq_ld_volatile(tkeys + i);
-      if (cur == FQ_GB_EMPTY) cur = atomicCAS((unsigned long long *)(tkeys + i), FQ_GB_EMPTY, (unsigned long long)key);
-      if (cur == FQ_GB_EMPTY || cur == key) {
+      Key cur = fq_gb_look(tkeys + i);
+      if (fq_gb_unsure(cur)) cur = fq_gb_cas(tkeys + i, key);
+      if (fq_gb_is_empty(cur) || fq_gb_eq(cur, key)) {
         slot = (fq_i64)i;
         want = false;
       } else if (++probe >= limit) {
@@ -1833,14 +1884,14 @@ __device__ __forceinline__ void fq_atom_add64_s(fq_u64 *slot, fq_u64 x) {
 // its rows find their key here, a lane stops looking (an unsuccessful search of a 3/4-full table costs more than the HBM
 // atomics it tries to avoid — 1e9 rows, 5000 keys: 53 ms with the search, 33 ms without).
 template <class Q>
-__device__ __forceinline__ void fq_gb_put(const fq_launch_params &p, fq_u64 *tkeys, fq_u64 *tslots, fq_u64 *skeys, fq_u64 *sslots, fq_u32 *s_used,
-                                          fq_u64 key, const fq_u64 *st, bool live, int &smem_try) {
+__device__ __forceinline__ void fq_gb_put(const fq_launch_params &p, typename Q::Key *tkeys, fq_u64 *tslots, typename Q::Key *skeys, fq_u64 *sslots,
+                                          fq_u32 *s_used, const typename Q::Key &key, const fq_u64 *st, bool live, int &smem_try) {
   const fq_u32 warp = __activemask();
-  const fq_u64 h = fq_gb_hash(key ^ p.gb_seed);
+  const fq_u64 h = fq_gb_seeded(key, p.gb_seed);
   const fq_u32 smask = p.gb_smem_cap - 1;
   const fq_u32 admit = p.gb_smem_cap - (p.gb_smem_cap >> FQ_GB_ADMIT_SHIFT);
   bool in_smem = false;
-  bool look = live && p.gb_smem_cap && key != FQ_GB_EMPTY && smem_try > 0;
+  bool look = live && p.gb_smem_cap && !fq_gb_is_empty(key) && smem_try > 0;
   const bool looked = look;
   // double hashing (an odd step walks the whole power-of-two table): no primary clustering, so the longest chain among the
   // warp's 32 lanes — the loop's trip count — stays short even at 3/4 load
@@ -1848,17 +1899,18 @@ __device__ __forceinline__ void fq_gb_put(const fq_launch_params &p, fq_u64 *tke
   fq_u32 i = (fq_u32)(h >> 32) & smask, probe = 0;
   while (__any_sync(warp, look)) {
     if (look) {
-      fq_u64 cur = *(volatile fq_u64 *)(skeys + i);
-      if (cur == FQ_GB_EMPTY) {
-        if (*(volatile fq_u32 *)s_used >= admit) {
+      typename Q::Key cur = fq_gb_look_s(skeys + i);
+      if (fq_gb_unsure(cur)) {
+        // an EMPTY look when admissions are closed sends the row to HBM: right whatever the slot really holds
+        if (fq_gb_is_empty(cur) && *(volatile fq_u32 *)s_used >= admit) {
           look = false;          // not admitted: this key lives in HBM
         } else {
-          cur = atomicCAS((unsigned long long *)(skeys + i), FQ_GB_EMPTY, (unsigned long long)key);
-          if (cur == FQ_GB_EMPTY) atomicAdd(s_used, 1u);
+          cur = fq_gb_cas(skeys + i, key);
+          if (fq_gb_is_empty(cur)) atomicAdd(s_used, 1u);
         }
       }
       if (look) {
-        if (cur == FQ_GB_EMPTY || cur == key) {
+        if (fq_gb_is_empty(cur) || fq_gb_eq(cur, key)) {
           in_smem = true;
           look = false;
         } else if (++probe >= p.gb_smem_cap) {
@@ -1878,9 +1930,10 @@ __device__ __forceinline__ void fq_gb_put(const fq_launch_params &p, fq_u64 *tke
 // One row per lane.  (Folding the lanes of a warp that share a key first — MATCH.ANY + REDUX over the match groups — was
 // measured on 1e9 rows, number % 7: 42 ms against 8.2 ms with plain native shared-memory atomics, and removed.)
 template <class Q>
-__device__ __forceinline__ void fq_gb_row(const fq_launch_params &p, fq_u64 *tkeys, fq_u64 *tslots, fq_u64 *skeys, fq_u64 *sslots, fq_u32 *s_used,
-                                          const typename Q::Rows &r, int v, fq_u32 &err, int &smem_try) {
-  fq_u64 key = 0, val[Q::NSLOTS > 0 ? Q::NSLOTS : 1] = {};
+__device__ __forceinline__ void fq_gb_row(const fq_launch_params &p, typename Q::Key *tkeys, fq_u64 *tslots, typename Q::Key *skeys, fq_u64 *sslots,
+                                          fq_u32 *s_used, const typename Q::Rows &r, int v, fq_u32 &err, int &smem_try) {
+  typename Q::Key key = {};
+  fq_u64 val[Q::NSLOTS > 0 ? Q::NSLOTS : 1] = {};
   fq_u32 vmask = 0;
   const bool live = Q::gb_row(p, r, v, err, key, val, vmask);
   fq_u64 st[Q::G];
@@ -1891,23 +1944,25 @@ __device__ __forceinline__ void fq_gb_row(const fq_launch_params &p, fq_u64 *tke
 template <class Q, int UNROLL>
 __device__ __forceinline__ void fq_groupby_kernel(const fq_launch_params &p) {
   constexpr int V = Q::V;
+  using Key = typename Q::Key;
   extern __shared__ __align__(128) unsigned char fq_dyn_smem[];
-  fq_u64 *skeys = (fq_u64 *)fq_dyn_smem;
-  fq_u64 *sslots = skeys + p.gb_smem_cap;
+  Key *skeys = (Key *)fq_dyn_smem;   // the keys (16-byte aligned when two words), then the states
+  fq_u64 *sslots = (fq_u64 *)(skeys + p.gb_smem_cap);
   __shared__ fq_u32 s_used;   // keys admitted to the shared-memory table
   if (threadIdx.x == 0) s_used = 0;
   for (fq_u32 i = threadIdx.x; i < p.gb_smem_cap; i += blockDim.x) {
-    skeys[i] = FQ_GB_EMPTY;
+    skeys[i] = fq_gb_empty<Key>();
     Q::gb_init(sslots + (size_t)i * Q::G);
   }
   __syncthreads();
   // this CTA's table in HBM: replica blockIdx % gb_reps.  A key that overflows the shared-memory table is hit by every CTA
   // on the same few L2 lines; with replicas only the CTAs that share one collide (1e9 rows, 5000 keys: 117 ms with one table)
-  fq_u64 *tkeys = p.gb_keys, *tslots = p.gb_slots;
+  Key *tkeys = (Key *)p.gb_keys;
+  fq_u64 *tslots = p.gb_slots;
   if (p.gb_reps > 1) {
     const fq_u32 rep = blockIdx.x % p.gb_reps;
     if (rep) {
-      tkeys = p.gb_rep_keys + (fq_u64)(rep - 1) * (p.gb_cap + 1);
+      tkeys = (Key *)p.gb_rep_keys + (fq_u64)(rep - 1) * (p.gb_cap + 1);
       tslots = p.gb_rep_slots + (fq_u64)(rep - 1) * (p.gb_cap + 1) * Q::G;
     }
   }
@@ -1942,39 +1997,42 @@ __device__ __forceinline__ void fq_groupby_kernel(const fq_launch_params &p) {
   __syncthreads();
   // flush the CTA's groups into the table in HBM
   for (fq_u32 i = threadIdx.x; i < p.gb_smem_cap; i += blockDim.x) {
-    const fq_u64 key = skeys[i];
-    const fq_i64 slot = fq_gb_find(p, tkeys, key, fq_gb_hash(key ^ p.gb_seed), key != FQ_GB_EMPTY);
+    const Key key = skeys[i];
+    const fq_i64 slot = fq_gb_find(p, tkeys, key, fq_gb_seeded(key, p.gb_seed), !fq_gb_is_empty(key));
     if (slot >= 0) Q::gb_merge(tslots + (fq_u64)slot * Q::G, sslots + (size_t)i * Q::G);
   }
   if (err) atomicOr((fq_u32 *)(p.result + 1), err);
 }
 
-// partial groups folded into the table.  With gb_entries: n_rows entries of 1 + Q::G slots (packed key, state — what
-// fq_pipe_export_partials writes).  Without: the (gb_reps - 1) replicas the aggregation kernel filled, n_rows =
-// (gb_reps - 1) * (gb_cap + 1) of their slots; every group met is folded into the table and its replica slot is reset, so
-// the replicas are empty again when the kernel ends.
+// partial groups folded into the table.  With gb_entries: n_rows entries of KW + Q::G slots (the packed key's KW words,
+// the state — what fq_pipe_export_partials writes).  Without: the (gb_reps - 1) replicas the aggregation kernel filled,
+// n_rows = (gb_reps - 1) * (gb_cap + 1) of their slots; every group met is folded into the table and its replica slot is
+// reset (every word of its key), so the replicas are empty again when the kernel ends.
 template <class Q>
 __device__ __forceinline__ void fq_groupby_merge_kernel(const fq_launch_params &p) {
+  using Key = typename Q::Key;
+  constexpr int KW = sizeof(Key) / 8;
   const fq_u64 tid = (fq_u64)blockIdx.x * blockDim.x + threadIdx.x;
   const fq_u64 nthreads = (fq_u64)gridDim.x * blockDim.x;
   if (p.gb_entries) {
     for (fq_u64 e = tid; e < p.n_rows; e += nthreads) {
-      const fq_u64 *ent = p.gb_entries + e * (1 + Q::G);
-      const fq_u64 key = ent[0];
-      const fq_i64 slot = fq_gb_find(p, p.gb_keys, key, fq_gb_hash(key ^ p.gb_seed), true);
-      if (slot >= 0) Q::gb_merge(p.gb_slots + (fq_u64)slot * Q::G, ent + 1);
+      const fq_u64 *ent = p.gb_entries + e * (KW + Q::G);
+      Key key;
+      fq_gb_from_words(key, ent);
+      const fq_i64 slot = fq_gb_find(p, (Key *)p.gb_keys, key, fq_gb_seeded(key, p.gb_seed), true);
+      if (slot >= 0) Q::gb_merge(p.gb_slots + (fq_u64)slot * Q::G, ent + KW);
     }
     return;
   }
   for (fq_u64 e = tid; e < p.n_rows; e += nthreads) {
     const bool special = e % (p.gb_cap + 1) == p.gb_cap;   // the slot of the key that equals the EMPTY mark
-    const fq_u64 key = special ? FQ_GB_EMPTY : p.gb_rep_keys[e];
+    const Key key = special ? fq_gb_empty<Key>() : ((Key *)p.gb_rep_keys)[e];
     fq_u64 *from = p.gb_rep_slots + e * Q::G;
-    const bool occupied = special ? from[0] != 0 : key != FQ_GB_EMPTY;   // from[0] = the group's row count
-    const fq_i64 slot = fq_gb_find(p, p.gb_keys, key, fq_gb_hash(key ^ p.gb_seed), occupied);
+    const bool occupied = special ? from[0] != 0 : !fq_gb_is_empty(key);   // from[0] = the group's row count
+    const fq_i64 slot = fq_gb_find(p, (Key *)p.gb_keys, key, fq_gb_seeded(key, p.gb_seed), occupied);
     if (slot >= 0) Q::gb_merge(p.gb_slots + (fq_u64)slot * Q::G, from);
     if (occupied) {
-      if (!special) p.gb_rep_keys[e] = FQ_GB_EMPTY;
+      if (!special) ((Key *)p.gb_rep_keys)[e] = fq_gb_empty<Key>();
       Q::gb_init(from);
     }
   }

@@ -333,9 +333,10 @@ fq_status fq_pipe_state_device(fq_ctx *ctx, const fq_pipe *pipe, void **dev_ptr,
  * skip NULL slots and are Type(None) for a group without a valid row, Count is the group's row count
  * (function_aggregator.rs:57-100, data_array_aggregate.rs:29); integer sums wrap.  Row order of the result is unspecified.
  *
- * A FQ_PIPE_GROUPBY pipe keeps an open-addressing hash table in HBM: 64-bit packed keys (the key expressions' value bits,
- * plus one bit per nullable key: at most 64 bits in all) and one 8-byte state per Aggregator leaf per group, updated with
- * atomics; every CTA pre-aggregates in a shared-memory table first, so low-cardinality keys never leave the SM.
+ * A FQ_PIPE_GROUPBY pipe keeps an open-addressing hash table in HBM: packed keys (the key expressions' value bits, plus
+ * one bit per nullable key: one 64-bit word for up to 64 bits in all, two words for 65..128 bits, claimed by one 16-byte
+ * compare-and-swap; wider key sets are refused) and one 8-byte state per Aggregator leaf per group, updated with atomics;
+ * every CTA pre-aggregates in a shared-memory table first, so low-cardinality keys never leave the SM.
  * fq_pipe_groupby_reserve sizes (and clears) the table; a launch that meets more groups than reserved makes
  * fq_pipe_fetch_groupby return FQ_ERR_CAPACITY (reserve more, relaunch).  Every reservation after a pipe's first also hashes
  * the keys with a new seed, so keys whose hashes clustered in one table (a probe chain too long: FQ_ERR_CAPACITY with room
@@ -353,8 +354,8 @@ fq_status fq_pipe_fetch_groupby(fq_ctx *ctx, fq_pipe *pipe, uint64_t *n_groups);
 fq_status fq_pipe_export_groups(fq_ctx *ctx, fq_pipe *pipe, fq_column *const *key_cols, fq_column *const *key_valid,
                                 fq_column *const *leaf_cols, fq_column *const *leaf_valid, uint64_t capacity, void *stream);
 /* Multi-GPU exchange of partial groups (one process per GPU).  fq_pipe_export_partials writes this rank's groups as raw
- * table entries — `entries` is a UInt64 column of n_groups x fq_pipe_group_entry_slots rows: the packed key, then the
- * state slots — ordered by owner rank = hash(key) mod world, and reports how many go to each rank (counts[world], host
+ * table entries — `entries` is a UInt64 column of n_groups x fq_pipe_group_entry_slots rows: the packed key, 1 or 2
+ * words, then the state slots — ordered by owner rank = hash(key) mod world, and reports how many go to each rank (counts[world], host
  * memory, valid after fq_stream_synchronize).  The host moves the runs to their owners (NCCL all-to-all over NVLink);
  * fq_pipe_merge_partials folds received entries into this pipe's table with the merge_state rules.  Afterwards every rank
  * owns a disjoint set of complete groups and exports them with fq_pipe_export_groups. */
